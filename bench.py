@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            this repo's CUDA engine (one process per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  the UNMODIFIED reference on the host cores
+    python bench.py ... --dump-outputs DIR                   also writes the outputs of the last timed step (dump_outputs)
 
 Workload (config.workload): BASELINE.json configs[4], the synthetic dense mpQP with 100 constraints / 30 variables /
 6 parameters = generate_mpqp(30, 6, 40, seed=0) after the reference's presolve (tests/golden/synthetic_30_6_40_s0.npz),
@@ -286,6 +287,48 @@ class ClockSampler(threading.Thread):
                 'reasons': sorted(reasons), 'samples': len(self.samples)}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, dev_sol, e2e_sol):
+    """Writes what the last timed step of each GPU path returned, as float64 .npy files, so that two builds can be compared
+    output for output: level_stats (level, candidates, feasible, optimal, regions) of the device-resident pass, and the
+    critical regions of the end-to-end solve.  A and b are stacked per region; the rows of C, d, E, f and the active sets
+    are concatenated over the regions, region_rows gives each region's (active set length, rows of E).  Above DUMP_BYTES
+    a fixed seeded sample of the regions is written; region_index lists which ones."""
+    os.makedirs(out_dir, exist_ok=True)
+    f64 = lambda x: numpy.asarray(x, dtype=numpy.float64)
+    stats = f64([[s['level'], s['candidates'], s['feasible'], s['optimal'], s['regions']] for s in dev_sol.level_stats])
+    regions = e2e_sol.critical_regions
+    size = [8 * (numpy.size(r.A) + numpy.size(r.b) + numpy.size(r.C) + numpy.size(r.d) + numpy.size(r.E) + numpy.size(r.f)
+                 + len(r.active_set) + 3) for r in regions]
+    keep = list(range(len(regions)))
+    room = DUMP_BYTES - stats.nbytes - (16 << 10)   # the .npy headers
+    if sum(size) > room:
+        keep = []
+        for i in numpy.random.default_rng(0).permutation(len(regions)).tolist():
+            if size[i] <= room:
+                keep.append(i)
+                room -= size[i]
+        keep.sort()
+    sel = [regions[i] for i in keep]
+    t = e2e_sol.program.num_t()
+    n = e2e_sol.program.num_x()
+    out = {
+        'level_stats': stats.reshape(-1, 5),
+        'region_index': f64(keep),
+        'region_rows': f64([[len(r.active_set), numpy.shape(r.E)[0]] for r in sel]).reshape(-1, 2),
+        'region_active_set': f64([i for r in sel for i in r.active_set]),
+        'region_A': f64([r.A for r in sel]).reshape(-1, n, t),
+        'region_b': f64([r.b for r in sel]).reshape(-1, n),
+    }
+    for fld, shape in (('C', (-1, t)), ('d', (-1,)), ('E', (-1, t)), ('f', (-1,))):
+        rows = [f64(getattr(r, fld)).reshape(shape) for r in sel]
+        out['region_' + fld] = numpy.concatenate(rows) if rows else numpy.zeros((0,) + shape[1:])
+    for name, a in out.items():
+        numpy.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def run_gpu(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -370,6 +413,8 @@ def run_gpu(args, rank, world, local_rank):
             h2d, d2h, n_regions = s2.h2d_bytes, s2.d2h_bytes, len(s2.critical_regions)
     if os.environ.get('PPGPU_BENCH_VERBOSE'):
         print(f'[rank {rank}] e2e ms per step ' + str([round(x, 1) for x in ms_e2e]), file=sys.stderr, flush=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sol, s2)
     # ---- parity of the sharded run: same digest as a single-GPU run of the same program (rank 0, same process)
     parity = None
     d_all = engine.solve(prog, max_levels=L, engine=eng, digest=True).digest
@@ -508,7 +553,10 @@ def main():
     ap.add_argument('--cpu-seconds', type=float, default=15.0)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-full-solves', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='GPU arm: write what the last timed step returned as DIR/<name>.npy (see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.warmup < 3:
         args.warmup = 3
     rank = int(os.environ.get('RANK', '0'))

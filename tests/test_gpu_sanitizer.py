@@ -17,8 +17,11 @@ def test_compute_sanitizer_clean(tool):
     exe = shutil.which('compute-sanitizer') or '/usr/local/cuda/bin/compute-sanitizer'
     if not os.path.exists(exe):
         pytest.skip('compute-sanitizer not installed')
-    out = subprocess.run([exe, '--tool', tool, '--error-exitcode', '9', sys.executable, os.path.join(ROOT, 'scripts', 'sanitize_target.py')],
-                         cwd=ROOT, capture_output=True, text=True, timeout=900)
+    try:
+        out = subprocess.run([exe, '--tool', tool, '--error-exitcode', '9', sys.executable, os.path.join(ROOT, 'scripts', 'sanitize_target.py')],
+                             cwd=ROOT, capture_output=True, text=True, timeout=900)
+    except PermissionError:
+        pytest.skip('compute-sanitizer is installed but this user may not run it')
     text = out.stdout + out.stderr
     assert out.returncode == 0, text[-3000:]
     assert ('ERROR SUMMARY: 0 errors' in text) or ('0 hazards displayed (0 errors, 0 warnings)' in text), text[-2000:]
