@@ -153,6 +153,21 @@ int ppgpu_locate_points(const double* d_theta, int64_t n_points, int32_t t, cons
                         const double* d_Q, const double* d_H, const double* d_c, int32_t* d_region, double* d_x,
                         ppgpu_stream stream);
 
+/* Batched fixed-parameter QP solves of an mpQP handle (MPQP_Program.solve_theta, mpqp_program.py, with the solver the
+ * reference hands it to - daqp / gurobi / ... - and sample_theta_space; Solution.verify_solution's per-point QP solves).
+ * A dual active-set iteration on the Gram data of the handle (csrc/k8_theta_qp.cu), one point per warp.
+ *   d_theta   n_points x t          parameter points (the Theta rows A_t theta <= b_t do not constrain x: not imposed)
+ *   d_status  n_points uint8        PPG_QP_* of csrc/tolerances.h: 0 optimal, 1 infeasible, 2 iteration cap, 3 numerical breakdown
+ *   d_x       n_points x n or NULL  optimal x (NaN unless optimal)
+ *   d_dual    n_points x m or NULL  multipliers of the rows: equality rows first (mu), then the inequality rows (lambda >= 0), so
+ *                                   that Q x + H theta + c + A' dual = 0 (the convention of the regions' C theta + d laws)
+ *   d_active  n_points x words or NULL  final working set, as a candidate mask (inequality rows only)
+ *   d_iters   n_points int32 or NULL    steps taken (constraint additions + drops)
+ * Asynchronous on `stream`.  Returns -2 for an mpLP handle or when use_gram is 0 (Hessian not positive definite on the space
+ * left by the equalities). */
+int ppgpu_solve_theta_batch(ppgpu_program* prog, const double* d_theta, int64_t n_points, uint8_t* d_status, double* d_x,
+                            double* d_dual, uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream);
+
 /* Batched Chebyshev balls of polytopes {theta : E theta <= f} (chebyshev_ball, utils/chebyshev_ball.py:10-63: max r subject to
  * E_i theta + |E_i| r <= f_i): CriticalRegion.is_full_dimension (critical_region.py:89-105, radius > 1e-8) and the Chebyshev /
  * feasibility checks of the program constructor's warnings() (mplp_program.py:162-215).  Stateless - no program handle.

@@ -129,6 +129,7 @@ int ppgpu_program_create(const ppgpu_dims* d, const double* A, const double* b, 
     D.dc0 = R.nfree + 2;
 #define UP(field, vecname) if ((e = upload(p, R.vecname, &D.field)) != cudaSuccess) { ppgpu_program_destroy(p); return fail("upload " #field, e); }
     UP(At, At) UP(C1, C1) UP(T0, T0) UP(Gam, Gam) UP(G, G) UP(V, V) UP(th_lo, th_lo) UP(th_hi, th_hi) UP(A, A) UP(b, b) UP(F, F) UP(A_t, At_theta) UP(b_t, bt) UP(Q, Q) UP(c, c) UP(H, H)
+    UP(Xp, Xp) UP(K, K) UP(Pm, Pm)
 #undef UP
     D.wk_ok = R.wk_ok; D.wk_nb = R.wk_nb; D.wk_ld = R.wk_ld; D.wk_D0 = nullptr; D.wk_bvar = nullptr; D.wk_nvar = nullptr;
     if (R.wk_ok) {
@@ -562,6 +563,22 @@ int ppgpu_locate_points(const double* d_theta, int64_t n_points, int32_t t, cons
     e = launch_locate(d_theta, n_points, t, d_rows, (const long long*)d_row_off, n_regions, d_laws, n_x, use_tol, tol,
                       overlap ? 1 : 0, d_Q, d_H, d_c, d_region, d_x, sms, (cudaStream_t)stream);
     if (e != cudaSuccess) return fail("K7 point location", e);
+    return 0;
+}
+
+int ppgpu_solve_theta_batch(ppgpu_program* p, const double* d_theta, int64_t n_points, uint8_t* d_status, double* d_x,
+                            double* d_dual, uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream) {
+    if (!p) return fail_msg("null argument");
+    if (!p->dev.is_qp || !p->dev.use_gram)
+        return fail_msg("solve_theta needs an mpQP whose Hessian is positive definite on the reduced space (use_gram = 0)");
+    if (n_points < 0) return fail_msg("negative size");
+    if (n_points == 0) return 0;
+    if (!d_theta || !d_status) return fail_msg("null argument");
+    cudaError_t e = cudaSetDevice(p->device);
+    if (e == cudaSuccess)
+        e = launch_theta_qp(p->dev, d_theta, n_points, d_status, d_x, d_dual, d_active, d_iters, p->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return fail("K8 fixed-theta QP", e);
+    p->launches++;
     return 0;
 }
 

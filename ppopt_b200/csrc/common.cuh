@@ -23,6 +23,10 @@ struct DevProgram {
     const double* A; const double* b; const double* F;      // originals (K5)
     const double* A_t; const double* b_t;
     const double* Q; const double* c; const double* H;
+    // K8 fixed-theta QP (use_gram only): x = Xp [1; theta] - K lambda,  mu = -Pm (Q x + H theta + c + A_in' lambda)
+    const double* Xp;   // n x (t+1)
+    const double* K;    // n x mi
+    const double* Pm;   // ne x n
     // K2a -> K2 hand-over (api.cu owns the buffers; null/0 = disabled): candidates the relaxation could not certify leave
     // the exact residuals G z* - h of their last iterate here, and the simplex starts from z* instead of the origin
     double* warm_resid;               // warm_cap x R0

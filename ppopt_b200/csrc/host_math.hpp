@@ -37,6 +37,9 @@ struct ReducedProgram {
     vec Gam;
     // K3: Gram G (mi x mi) and V (mi x (t+1)) with layout [const | theta coefficients]
     vec G, V;
+    // K8 (fixed-theta QP, only when use_gram): x = Xp [1; theta] - K lambda  and  equality multipliers
+    // mu = -Pm (Q x + H theta + c + A_in' lambda)
+    vec Xp, K, Pm;   // n x (t+1), n x mi, ne x n
     // outer bounding box of Theta from the single-variable rows of A_t theta <= b_t (+-inf where there is none);
     // used by K3 as a cheap NECESSARY test: lambda_j(theta) must be able to reach >= 0 somewhere in the box
     vec th_lo, th_hi;
@@ -214,7 +217,7 @@ inline bool reduce_program(int n, int t, int m, int q, int ne, int is_qp, const 
     if (is_qp) P.Q.assign(Q, Q + (size_t)n * n); else P.Q.assign((size_t)n * n, 0.0);
     const int np = P.np, mi = P.mi;
     // ---- eliminate the equalities: x = x0 + Xt*theta + Q2*v
-    vec Q2((size_t)n * np, 0.0), x0(n, 0.0), Xt((size_t)n * t, 0.0);
+    vec Q2((size_t)n * np, 0.0), x0(n, 0.0), Xt((size_t)n * t, 0.0), Pm((size_t)ne * n, 0.0);
     if (ne == 0) {
         for (int i = 0; i < n; ++i) Q2[(size_t)i * np + i] = 1.0;
     } else {
@@ -241,6 +244,13 @@ inline bool reduce_program(int n, int t, int m, int q, int ne, int is_qp, const 
             }
             for (int j = 0; j < np; ++j) Q2[(size_t)i * np + j] = Qf[(size_t)i * n + ne + j];
         }
+        // Pm = R^-1 Q1' (A_eq' = Q1 R): the equality multipliers of a stationary point (K8)
+        for (int col = 0; col < n; ++col)
+            for (int i = ne - 1; i >= 0; --i) {
+                double s = Qf[(size_t)col * n + i];
+                for (int k = i + 1; k < ne; ++k) s -= M[(size_t)i * ne + k] * Pm[(size_t)k * n + col];
+                Pm[(size_t)i * n + col] = s / M[(size_t)i * ne + i];
+            }
     }
     // ---- reduced inequality rows
     P.At.assign((size_t)mi * np, 0.0);
@@ -379,6 +389,34 @@ inline bool reduce_program(int n, int t, int m, int q, int ne, int is_qp, const 
                     P.V[(size_t)i * (t + 1) + col] = s;
                 }
             }
+            // K8: Qr^-1 lin = L^-T Z and Qr^-1 At' = L^-T Y, mapped back to x through Q2
+            for (int col = 0; col <= t; ++col)
+                for (int i = np - 1; i >= 0; --i) {
+                    double s = Z[(size_t)i * (t + 1) + col];
+                    for (int k = i + 1; k < np; ++k) s -= L[(size_t)k * np + i] * Z[(size_t)k * (t + 1) + col];
+                    Z[(size_t)i * (t + 1) + col] = s / L[(size_t)i * np + i];
+                }
+            for (int col = 0; col < mi; ++col)
+                for (int i = np - 1; i >= 0; --i) {
+                    double s = Y[(size_t)i * mi + col];
+                    for (int k = i + 1; k < np; ++k) s -= L[(size_t)k * np + i] * Y[(size_t)k * mi + col];
+                    Y[(size_t)i * mi + col] = s / L[(size_t)i * np + i];
+                }
+            P.Xp.assign((size_t)n * (t + 1), 0.0);
+            P.K.assign((size_t)n * mi, 0.0);
+            for (int i = 0; i < n; ++i) {
+                for (int col = 0; col <= t; ++col) {
+                    double s = col == 0 ? x0[i] : Xt[(size_t)i * t + col - 1];
+                    for (int k = 0; k < np; ++k) s -= Q2[(size_t)i * np + k] * Z[(size_t)k * (t + 1) + col];
+                    P.Xp[(size_t)i * (t + 1) + col] = s;
+                }
+                for (int col = 0; col < mi; ++col) {
+                    double s = 0.0;
+                    for (int k = 0; k < np; ++k) s += Q2[(size_t)i * np + k] * Y[(size_t)k * mi + col];
+                    P.K[(size_t)i * mi + col] = s;
+                }
+            }
+            P.Pm = Pm;
             P.use_gram = 1;
         }
     }

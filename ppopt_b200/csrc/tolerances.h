@@ -63,3 +63,20 @@
 #define PPG_LP_UNBOUNDED 2
 #define PPG_LP_INFEAS_EQ 3
 #define PPG_LP_ITERLIM 4
+
+// K8 fixed-theta QP (dual active set on  w = G lambda + V [1; theta],  csrc/k8_theta_qp.cu), shared with the CPU twin.
+// Engine-internal numerics, no reference counterpart (the reference hands the QP to daqp / gurobi / ...):
+//   PPG_QP_TOL       row j is violated when w_j < -PPG_QP_TOL * (1 + |V_j [1; theta]|) (its own scale: programs carry
+//                    big-M rows of 1e7 next to rows of 1e-3); optimal when no row outside W is violated
+//   PPG_QP_CURV      a constraint is added only when its curvature z = G_jj - |L^-1 G_Wj|^2 exceeds PPG_QP_CURV * G_jj
+//   PPG_QP_DTOL      a working-set multiplier blocks the step only when it falls at rate d_i < -PPG_QP_DTOL
+//   PPG_QP_MAX_ITER  steps (adds + drops) per point before the point is reported with status PPG_QP_ITERLIM
+#define PPG_QP_TOL 1e-10
+#define PPG_QP_CURV 1e-10
+#define PPG_QP_DTOL 1e-12
+#define PPG_QP_MAX_ITER 1000
+// status per point
+#define PPG_QP_OPTIMAL 0
+#define PPG_QP_INFEASIBLE 1
+#define PPG_QP_ITERLIM 2
+#define PPG_QP_NUMERIC 3

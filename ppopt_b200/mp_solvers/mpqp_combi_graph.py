@@ -13,9 +13,10 @@ the visited set E, the next frontier.  The visited closure does not depend on th
 the region SET equals the reference's (its list order is the arbitrary order of ``set.pop()``).
 
 Seeding.  The reference samples one theta and solves a QP for its active set (``program.sample_theta_space(1)``); the
-combinatorial path has no QP solver, so the seed is the first optimal active set the level-wise enumeration meets
-(any optimal active set will do: the graph of optimal active sets is connected - the premise of the algorithm).
-``initial_active_sets`` overrides it, as in ``combinatorial_graph_initialization`` (:10-29).
+default seed here is the first optimal active set the level-wise enumeration meets (any optimal active set will do: the
+graph of optimal active sets is connected - the premise of the algorithm).  ``initial_active_sets`` overrides it, as in
+``combinatorial_graph_initialization`` (:10-29): ``initial_active_sets=ThetaSolver(program).sample_theta_space()``
+(ppopt_b200.solve_theta, batched QP solves on the GPU) gives reference-style seeding.
 """
 from typing import Iterable, List, Optional
 

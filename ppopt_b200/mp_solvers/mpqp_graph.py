@@ -13,9 +13,10 @@ on the GPU (speculative frontier batching; grouped by cardinality):
     K5     LU-accurate rows, full-dimension test, redundancy   <- gen_cr_from_active_set + region.is_full_dimension
 A few speculatively evaluated sets are never popped by the reference (their results are simply not used).
 
-Seeding.  The reference samples theta and solves QPs (``program.sample_theta_space()``); the combinatorial path has no
-QP solver, so the default seed is the first optimal active set of the level-wise enumeration (mpqp_combi_graph._seed).
-``initial_active_sets`` overrides it, as in the reference (``graph_initialization``, :10-35).
+Seeding.  The reference samples theta and solves QPs (``program.sample_theta_space()``); the default seed here is the
+first optimal active set of the level-wise enumeration (mpqp_combi_graph._seed).  ``initial_active_sets`` overrides it,
+as in the reference (``graph_initialization``, :10-35): ``initial_active_sets=ThetaSolver(program).sample_theta_space()``
+(ppopt_b200.solve_theta, batched QP solves on the GPU) gives reference-style seeding.
 """
 from typing import Dict, Iterable, List, Optional, Tuple
 

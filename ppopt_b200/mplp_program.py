@@ -111,6 +111,23 @@ class MPQP_Program(MPLP_Program):
             + self.c_t.T @ theta_point + 0.5 * theta_point.T @ self.Q_t @ theta_point
         return float(v[0, 0])
 
+    def _theta_solver(self):
+        if getattr(self, '_theta_solver_cache', None) is None:
+            from .solve_theta import ThetaSolver
+            self._theta_solver_cache = ThetaSolver(self)
+        return self._theta_solver_cache
+
+    def solve_theta(self, theta_point, deterministic_solver=None):
+        """QP at a fixed theta (mpqp_program.py solve_theta) on the GPU (ppopt_b200.solve_theta.ThetaSolver): a
+        SolverOutput(obj, sol, slack, active_set, dual), or None when infeasible.  ``deterministic_solver`` is accepted for
+        the reference's signature and ignored.  The solver is built on first use and caches the program data: call
+        again after changing the arrays of this object only on a new object."""
+        return self._theta_solver().solve_theta(theta_point)
+
+    def sample_theta_space(self, num_samples: int = 100):
+        """distinct optimal active sets of QPs solved at points sampled in Theta (mpqp_program.py sample_theta_space)"""
+        return self._theta_solver().sample_theta_space(num_samples)
+
 
 def load_presolved(path: str):
     """Program object from a tests/golden/*.npz fixture (post-presolve arrays written by oracle/gen_golden.py)."""
