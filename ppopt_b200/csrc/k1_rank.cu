@@ -363,10 +363,8 @@ static cudaError_t launch_k1_svd(const DevProgram& P, const uint64_t* masks, lon
     const int wd = kmax * P.np;
     const size_t smem = (size_t)4 * wd * sizeof(double);
     if (smem > 200 * 1024) return cudaSuccess;
-    if (smem > 48 * 1024) {
-        cudaError_t e = allow_max_smem(k1_svd_recheck_kernel);
-        if (e != cudaSuccess) return e;
-    }
+    const cudaError_t e = fit_smem(k1_svd_recheck_kernel, smem);
+    if (e != cudaSuccess) return e;
     long long grid = (n + 127) / 128;
     if (grid > (long long)sm_count * 4) grid = (long long)sm_count * 4;
     k1_svd_recheck_kernel<<<(unsigned)grid, 128, smem, st>>>(P, masks, n, k_act, status, wd);

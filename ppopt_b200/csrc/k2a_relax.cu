@@ -226,10 +226,7 @@ static cudaError_t launch_k2a_t(const DevProgram& P, const uint64_t* masks, long
     const size_t per_warp = (size_t)k_act * k_act + 2 * (size_t)k_act + (size_t)P.nfree + (size_t)((k_act + 1) / 2 + 1);
     const size_t smem = per_warp * 4 * sizeof(double);
     cudaError_t e;
-    if (smem > 48 * 1024) {
-        e = allow_max_smem(kern);
-        if (e != cudaSuccess) return e;
-    }
+    if ((e = fit_smem(kern, smem)) != cudaSuccess) return e;
     int occ = 0;
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 128, smem);
     if (e != cudaSuccess) return e;

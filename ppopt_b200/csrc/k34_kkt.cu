@@ -358,10 +358,7 @@ static cudaError_t launch_k34_t(const DevProgram& P, const uint64_t* masks, long
     const size_t per_warp = (size_t)k_act * k_act + (size_t)k_act * (P.t + 1) + (size_t)((k_act + 1) / 2 + 1);
     const size_t smem = per_warp * WPC * sizeof(double);
     cudaError_t e;
-    if (smem > 48 * 1024) {
-        e = allow_max_smem(kern);
-        if (e != cudaSuccess) return e;
-    }
+    if ((e = fit_smem(kern, smem)) != cudaSuccess) return e;
     int occ = 0;
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 32 * WPC, smem);
     if (e != cudaSuccess) return e;

@@ -348,10 +348,7 @@ static cudaError_t launch_k5_t(const DevProgram& P, const uint64_t* masks, const
     const size_t smem = ((size_t)N * ld + (size_t)P.R0 * (P.t + 1)) * sizeof(double) + (size_t)(2 * P.R0 + k + 2) * sizeof(int);
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
     cudaError_t e;
-    if (smem > 48 * 1024) {
-        e = allow_max_smem(kern);
-        if (e != cudaSuccess) return e;
-    }
+    if ((e = fit_smem(kern, smem)) != cudaSuccess) return e;
     long long grid = n_sel;
     const long long cap = (long long)sm_count * 8;
     if (grid > cap) grid = cap;

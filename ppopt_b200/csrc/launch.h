@@ -21,6 +21,17 @@ inline cudaError_t allow_max_smem(K kern) {
     return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, lim - (int)fa.sharedSizeBytes);   // static + dynamic <= limit
 }
 
+// Opts in (allow_max_smem) when a launch with `dyn` bytes of dynamic shared memory would exceed the 48 KB a block gets without
+// it.  The kernel's static shared memory counts against the same 48 KB: a dynamic size just below 48 KB alone fails with
+// "invalid argument" on the first launch of a kernel that also has static arrays.
+template <class K>
+inline cudaError_t fit_smem(K kern, size_t dyn) {
+    cudaFuncAttributes fa;
+    const cudaError_t e = cudaFuncGetAttributes(&fa, kern);
+    if (e != cudaSuccess) return e;
+    return fa.sharedSizeBytes + dyn > 48 * 1024 ? allow_max_smem(kern) : cudaSuccess;
+}
+
 int k2_pad_columns(int ncols_with_rhs);
 
 cudaError_t launch_k1(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,

@@ -43,7 +43,7 @@ def golden_regions(g):
             nb, nd, nf = len(r['b']), len(r['d']), len(r['f'])
             t = len(r['A']) // nb if nb else (len(r['C']) // nd if nd else t)
             r['A'], r['b'] = r['A'].reshape(nb, -1), r['b'].reshape(nb, 1)
-            r['C'], r['d'] = r['C'].reshape(nd, -1), r['d'].reshape(nd, 1)
+            r['C'], r['d'] = r['C'].reshape(nd, t), r['d'].reshape(nd, 1)   # (nd = 0: the equality-only active set)
             r['E'], r['f'] = r['E'].reshape(nf, -1), r['f'].reshape(nf, 1)
             if g['pk_E_int'][i]:
                 r['E'] = r['E'].astype(numpy.int64)
