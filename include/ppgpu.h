@@ -168,6 +168,23 @@ int ppgpu_locate_points(const double* d_theta, int64_t n_points, int32_t t, cons
 int ppgpu_solve_theta_batch(ppgpu_program* prog, const double* d_theta, int64_t n_points, uint8_t* d_status, double* d_x,
                             double* d_dual, uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream);
 
+/* Batched fixed-parameter LP solves of an mpLP handle (MPLP_Program.solve_theta, mplp_program.py, with the LP backend the
+ * reference hands it to - GLPK / HiGHS / ... - and sample_theta_space; Solution.verify_solution's per-point LP solves).
+ * A dense primal dictionary simplex (Phase 1 with one auxiliary column, then Phase 2) from the theta-independent start
+ * dictionary of the handle (csrc/k9_theta_lp.cu), one point per warp.
+ *   d_theta   n_points x t          parameter points (the Theta rows A_t theta <= b_t do not constrain x: not imposed)
+ *   d_status  n_points uint8        PPG_TLP_* of csrc/tolerances.h: 0 optimal, 1 infeasible, 2 iteration cap, 3 numerical
+ *                                   breakdown, 4 unbounded
+ *   d_x       n_points x n or NULL  optimal vertex x (NaN unless optimal)
+ *   d_dual    n_points x m or NULL  multipliers of the rows: equality rows first (mu), then the inequality rows (lambda >= 0,
+ *                                   zero on basic rows), so that c + H theta + A' dual = 0 (NaN unless optimal)
+ *   d_active  n_points x words or NULL  final basis: the n - n_eq nonbasic inequality slacks, as a candidate mask
+ *   d_iters   n_points x 2 int32 or NULL  pivots of both phases, pivots of Phase 1
+ * Asynchronous on `stream`.  Returns -2 for an mpQP handle and for an mpLP whose reduced inequality rows have rank below
+ * n - n_eq (no vertex). */
+int ppgpu_solve_theta_lp_batch(ppgpu_program* prog, const double* d_theta, int64_t n_points, uint8_t* d_status, double* d_x,
+                               double* d_dual, uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream);
+
 /* Batched Chebyshev balls of polytopes {theta : E theta <= f} (chebyshev_ball, utils/chebyshev_ball.py:10-63: max r subject to
  * E_i theta + |E_i| r <= f_i): CriticalRegion.is_full_dimension (critical_region.py:89-105, radius > 1e-8) and the Chebyshev /
  * feasibility checks of the program constructor's warnings() (mplp_program.py:162-215).  Stateless - no program handle.

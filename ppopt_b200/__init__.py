@@ -3,14 +3,15 @@
     from ppopt_b200 import solve_mpqp, mpqp_algorithm
     solution = solve_mpqp(program, mpqp_algorithm.combinatorial)     # program: ppopt or ppopt_b200 program object
 
-    ThetaSolver(program).solve_batch(thetas)    # fixed-theta QPs, one batch;  verify_solution(solution): explicit vs implicit
+    ThetaSolver(program).solve_batch(thetas)    # fixed-theta QPs, one batch (ThetaLPSolver: mpLPs)
+    verify_solution(solution)                   # explicit vs implicit
 
     import ppopt_b200; ppopt_b200.install()      # or: make ppopt.solve_mpqp(..., combinatorial) run on the GPU
 """
 from .mp_solvers.solve_mpqp import mpqp_algorithm, solve_mpqp  # noqa: F401
 from .mplp_program import MPLP_Program, MPQP_Program  # noqa: F401
 from .point_location import PointLocation  # noqa: F401
-from .solve_theta import ThetaSolver, verify_solution  # noqa: F401
+from .solve_theta import ThetaLPSolver, ThetaSolver, verify_solution  # noqa: F401
 
 
 def install(ppopt_package=None):

@@ -55,6 +55,7 @@ SYMBOLS = {
     'ppgpu_locate_points': (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp, _i64, _vp, _i32, _i32, ctypes.c_double, _i32, _vp, _vp, _vp,
                                            _vp, _vp, _vp]),
     'ppgpu_solve_theta_batch': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'ppgpu_solve_theta_lp_batch': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'ppgpu_chebyshev_batch': (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
     'ppgpu_measure_fp64_peak': (ctypes.c_int, [_i32, ctypes.POINTER(ctypes.c_double), _vp]),
 }

@@ -136,6 +136,16 @@ int ppgpu_program_create(const ppgpu_dims* d, const double* A, const double* b, 
         if ((e = upload(p, R.wk_D0, &D.wk_D0)) != cudaSuccess || (e = upload(p, R.wk_bvar, &D.wk_bvar)) != cudaSuccess ||
             (e = upload(p, R.wk_nvar, &D.wk_nvar)) != cudaSuccess) { ppgpu_program_destroy(p); return fail("upload walk dictionary", e); }
     }
+    D.lp_ok = R.lp_ok; D.lp_ld = R.lp_ld; D.lp_D0 = nullptr; D.lp_bvar = nullptr; D.lp_nvar = nullptr; D.lp_obj = nullptr;
+    D.X0t = nullptr; D.Q2 = nullptr;
+    if (R.lp_ok) {
+        if ((e = upload(p, R.lp_D0, &D.lp_D0)) != cudaSuccess || (e = upload(p, R.lp_bvar, &D.lp_bvar)) != cudaSuccess ||
+            (e = upload(p, R.lp_nvar, &D.lp_nvar)) != cudaSuccess || (e = upload(p, R.lp_obj, &D.lp_obj)) != cudaSuccess ||
+            (e = upload(p, R.X0t, &D.X0t)) != cudaSuccess || (e = upload(p, R.Q2, &D.Q2)) != cudaSuccess) {
+            ppgpu_program_destroy(p);
+            return fail("upload LP start dictionary", e);
+        }
+    }
     void* dc = nullptr;
     if ((e = cudaMalloc(&dc, (CNT_COUNT + QUEUE_SLOTS) * sizeof(unsigned long long))) != cudaSuccess) {
         ppgpu_program_destroy(p);
@@ -578,6 +588,22 @@ int ppgpu_solve_theta_batch(ppgpu_program* p, const double* d_theta, int64_t n_p
     if (e == cudaSuccess)
         e = launch_theta_qp(p->dev, d_theta, n_points, d_status, d_x, d_dual, d_active, d_iters, p->sm_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return fail("K8 fixed-theta QP", e);
+    p->launches++;
+    return 0;
+}
+
+int ppgpu_solve_theta_lp_batch(ppgpu_program* p, const double* d_theta, int64_t n_points, uint8_t* d_status, double* d_x,
+                               double* d_dual, uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream) {
+    if (!p) return fail_msg("null argument");
+    if (p->dev.is_qp) return fail_msg("solve_theta_lp needs an mpLP handle (this one is an mpQP: ppgpu_solve_theta_batch)");
+    if (!p->dev.lp_ok) return fail_msg("solve_theta_lp: the reduced inequality rows have rank below n - n_eq, the LP has no vertex");
+    if (n_points < 0) return fail_msg("negative size");
+    if (n_points == 0) return 0;
+    if (!d_theta || !d_status) return fail_msg("null argument");
+    cudaError_t e = cudaSetDevice(p->device);
+    if (e == cudaSuccess)
+        e = launch_theta_lp(p->dev, d_theta, n_points, d_status, d_x, d_dual, d_active, d_iters, p->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return fail("K9 fixed-theta LP", e);
     p->launches++;
     return 0;
 }

@@ -38,6 +38,14 @@ struct DevProgram {
     const double* wk_D0;   // wk_nb x wk_ld  [beta | D]
     const int* wk_bvar;    // wk_nb  row (slack) basic in every dictionary row
     const int* wk_nvar;    // nfree  row (slack) nonbasic in every column
+    // K9 fixed-theta LP (mpLPs with a vertex only, host_math.hpp::build_lp_dictionary; Pm above is set for mpLPs too)
+    int lp_ok, lp_ld;      // lp_ld = 1 + np + t
+    const double* lp_D0;   // mi x lp_ld  [beta0 | D | Dth]: row = beta0 - D s_N - Dth theta
+    const int* lp_bvar;    // mi          slack basic in the row, or -1 - c for the free direction v_c
+    const int* lp_nvar;    // np          slack nonbasic in each column
+    const double* lp_obj;  // np x (t+1)  [d0 | dth]: z = zeta - d(theta)' s_N
+    const double* X0t;     // n x (t+1)   x = X0t [1; theta] + Q2 v
+    const double* Q2;      // n x np
 };
 
 // indices into the device counter array (uint64 each)

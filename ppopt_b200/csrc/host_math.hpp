@@ -51,6 +51,15 @@ struct ReducedProgram {
     int wk_ok = 0, wk_nb = 0, wk_ld = 0;
     vec wk_D0;
     std::vector<int> wk_bvar, wk_nvar;
+    // K9 (fixed-theta LP, mpLPs only): the free directions v exchanged against np inequality slacks, a dictionary whose
+    // entries are constant and whose right-hand side and objective row are affine in theta.  Row i of lp_D0 (mi x lp_ld,
+    // lp_ld = 1 + np + t) reads  y_i = beta0_i - D_i s_N - Dth_i theta  with layout [beta0 | D (np) | Dth (t)]; y_i is the
+    // slack lp_bvar[i] >= 0, or the free variable v_c when lp_bvar[i] = -1 - c.  Column c of D is the slack lp_nvar[c].
+    // Objective (the v part of (c + H theta)' x):  z = zeta - d(theta)' s_N  with lp_obj (np x (t + 1)) = [d0 | dth].
+    // lp_ok = 0 when the reduced rows At have rank below np (the LP has no vertex).  x = X0t [1; theta] + Q2 v.
+    int lp_ok = 0, lp_ld = 0;
+    vec lp_D0, lp_obj, X0t, Q2;   // mi x lp_ld, np x (t + 1), n x (t + 1), n x np
+    std::vector<int> lp_bvar, lp_nvar;
     std::string error;
 };
 
@@ -123,8 +132,28 @@ inline void dict_pivot(vec& D, int nb, int ld, int l, int j) {
     for (int c = 0; c < ld; ++c) D[(size_t)l * ld + c] = q[c];
 }
 
+// Exchanges the free variables held in columns 0..nx-1 of a slack dictionary  s = beta - D [x; rest]  (nr x ld rows, every
+// row a slack, rowvar[i] = i) against slacks, one Gauss-Jordan pivot per column on the largest remaining entry (partial
+// pivoting).  Afterwards row rowvar[i] < 0 holds the free variable -1 - rowvar[i], column c < nx the slack colvar[c]; columns
+// nx.. are carried along by the pivots as further right-hand sides.  Returns false when the columns have no full rank.
+inline bool exchange_free_columns(vec& D, int nr, int ld, int nx, std::vector<int>& rowvar, std::vector<int>& colvar) {
+    rowvar.resize(nr);
+    colvar.assign(nx, -1);
+    for (int i = 0; i < nr; ++i) rowvar[i] = i;
+    for (int c = 0; c < nx; ++c) {
+        int best = -1; double bv = 0.0;
+        for (int i = 0; i < nr; ++i)
+            if (rowvar[i] >= 0 && std::fabs(D[(size_t)i * ld + 1 + c]) > bv) { bv = std::fabs(D[(size_t)i * ld + 1 + c]); best = i; }
+        if (best < 0 || bv < 1e-9) return false;
+        dict_pivot(D, nr, ld, best, c);
+        colvar[c] = rowvar[best];
+        rowvar[best] = -1 - c;
+    }
+    return true;
+}
+
 // K2w set-up: a feasible vertex of F = {z : Gf z <= h} (Gf = T0[:, 1..nfree], h = T0[:, 0]) as a slack dictionary.
-// (1) the free variables z are exchanged against slacks with partial pivoting (the rows that take a z are dropped: z is
+// (1) the free variables z are exchanged against slacks (exchange_free_columns; the rows that take a z are dropped: z is
 // never needed again), (2) a composite phase 1 (maximise the sum of the negative slacks, Dantzig, Bland after stalling)
 // makes the vertex feasible.  Runs once per program; every feasibility certificate of K2w is a vertex reached from this
 // one by primal simplex pivots (k2w_walk.cu).
@@ -138,17 +167,8 @@ inline void build_walk_dictionary(ReducedProgram& P) {
         D[(size_t)i * ld] = P.T0[(size_t)i * dc];
         for (int c = 0; c < nf; ++c) D[(size_t)i * ld + 1 + c] = P.T0[(size_t)i * dc + 1 + c];
     }
-    std::vector<int> rowvar(R0), colvar(nf, -1);   // rowvar: slack id, or -1 once the row holds a z
-    for (int i = 0; i < R0; ++i) rowvar[i] = i;
-    for (int c = 0; c < nf; ++c) {
-        int best = -1; double bv = 0.0;
-        for (int i = 0; i < R0; ++i)
-            if (rowvar[i] >= 0 && std::fabs(D[(size_t)i * ld + 1 + c]) > bv) { bv = std::fabs(D[(size_t)i * ld + 1 + c]); best = i; }
-        if (best < 0 || bv < 1e-9) return;   // Gf has no full column rank: F has no vertex
-        dict_pivot(D, R0, ld, best, c);
-        colvar[c] = rowvar[best];
-        rowvar[best] = -1;
-    }
+    std::vector<int> rowvar, colvar;   // rowvar: slack id, or < 0 once the row holds a z
+    if (!exchange_free_columns(D, R0, ld, nf, rowvar, colvar)) return;   // Gf has no full column rank: F has no vertex
     const int nb = R0 - nf;
     vec E((size_t)nb * ld);
     std::vector<int> bvar(nb);
@@ -199,6 +219,40 @@ inline void build_walk_dictionary(ReducedProgram& P) {
     for (int i = 0; i < nb; ++i) if (E[(size_t)i * ld] < 0.0) E[(size_t)i * ld] = 0.0;
     for (size_t k = 0; k < E.size(); ++k) if (!std::isfinite(E[k])) { P.wk_ok = 0; return; }
     P.wk_nb = nb; P.wk_ld = ld; P.wk_D0 = E; P.wk_bvar = bvar; P.wk_nvar = colvar;
+}
+
+// K9 set-up (mpLPs): the reduced rows  s = bti + Ft theta - At v  (rows 0..mi-1 of T0, whose theta columns hold -Ft) with
+// the np free directions v exchanged against slacks (exchange_free_columns, as K2w's start), and the objective row of
+// (c + H theta)' x = const + g(theta)' v,  g = Q2' (c + H theta), in the nonbasic slacks.  Entries are constant, right-hand
+// side and objective row affine in theta: the kernel evaluates them per point and runs the simplex from there.
+inline void build_lp_dictionary(ReducedProgram& P) {
+    P.lp_ok = 0;
+    const int mi = P.mi, np = P.np, t = P.t, n = P.n, dc = P.nfree + 2, ld = 1 + np + t;
+    vec D((size_t)mi * ld);
+    for (int i = 0; i < mi; ++i)
+        for (int c = 0; c < ld; ++c) D[(size_t)i * ld + c] = P.T0[(size_t)i * dc + c];
+    std::vector<int> rowvar, colvar;
+    if (!exchange_free_columns(D, mi, ld, np, rowvar, colvar)) return;   // At has rank below np: no vertex
+    std::vector<int> vrow(np);
+    for (int i = 0; i < mi; ++i) if (rowvar[i] < 0) vrow[-1 - rowvar[i]] = i;
+    vec obj((size_t)np * (t + 1), 0.0);
+    for (int col = 0; col <= t; ++col) {
+        vec g(np);
+        for (int c = 0; c < np; ++c) {
+            double s = 0.0;
+            for (int k = 0; k < n; ++k) s += P.Q2[(size_t)k * np + c] * (col == 0 ? P.c[k] : P.H[(size_t)k * t + col - 1]);
+            g[c] = s;
+        }
+        for (int j = 0; j < np; ++j) {
+            double s = 0.0;
+            for (int c = 0; c < np; ++c) s += g[c] * D[(size_t)vrow[c] * ld + 1 + j];
+            obj[(size_t)j * (t + 1) + col] = s;
+        }
+    }
+    for (size_t k = 0; k < D.size(); ++k) if (!std::isfinite(D[k])) return;
+    for (size_t k = 0; k < obj.size(); ++k) if (!std::isfinite(obj[k])) return;
+    P.lp_ld = ld; P.lp_D0 = D; P.lp_obj = obj; P.lp_bvar = rowvar; P.lp_nvar = colvar;
+    P.lp_ok = 1;
 }
 
 // Builds the reduced program. Inputs are row-major, equalities are rows 0..ne-1 of A/b/F.
@@ -421,6 +475,16 @@ inline bool reduce_program(int n, int t, int m, int q, int ne, int is_qp, const 
         }
     }
     build_walk_dictionary(P);
+    if (!is_qp) {
+        P.X0t.assign((size_t)n * (t + 1), 0.0);
+        for (int i = 0; i < n; ++i) {
+            P.X0t[(size_t)i * (t + 1)] = x0[i];
+            for (int j = 0; j < t; ++j) P.X0t[(size_t)i * (t + 1) + 1 + j] = Xt[(size_t)i * t + j];
+        }
+        P.Q2 = Q2;
+        P.Pm = Pm;
+        build_lp_dictionary(P);
+    }
     return true;
 }
 

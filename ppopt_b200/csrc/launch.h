@@ -93,6 +93,10 @@ cudaError_t launch_cheb_batch(const double* rows, const long long* row_off, long
 // K8: one fixed-theta QP per point (dual active set on the Gram data, csrc/k8_theta_qp.cu); x / dual / mask / iters may be null
 cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
                             double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);
+// K9: one fixed-theta LP per point (dictionary simplex from the handle's start dictionary, csrc/k9_theta_lp.cu);
+// iters (n x 2: pivots, Phase 1 pivots), x / dual / mask / iters may be null
+cudaError_t launch_theta_lp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
+                            double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);
 cudaError_t launch_clear_bits(uint8_t* status, long long n, uint8_t bits, cudaStream_t st);
 
 cudaError_t measure_fp64_peak(int iters, double* tflops, cudaStream_t st);

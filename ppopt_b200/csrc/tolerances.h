@@ -80,3 +80,30 @@
 #define PPG_QP_INFEASIBLE 1
 #define PPG_QP_ITERLIM 2
 #define PPG_QP_NUMERIC 3
+
+// K9 fixed-theta LP (dense primal dictionary simplex from the theta-independent start of host_math.hpp::build_lp_dictionary,
+// csrc/k9_theta_lp.cu).  Engine-internal numerics, no reference counterpart (the reference hands the LP to GLPK / HiGHS / ...):
+//   PPG_TLP_TOL       feasibility tolerance of slack i: delta_i = PPG_TLP_TOL * (1 + |bti_i + Ft_i theta|), the scale of the
+//                     row's own right-hand side (as K8's PPG_QP_TOL): the synthetic programs carry box rows of 1e7 next to
+//                     rows near 1, and one absolute tolerance is either meaningless on the first or too loose on the second
+//                     (the start dictionary's beta is no scale: the start vertex can lie far outside the feasible set).
+//                     delta_i is the Harris relaxation of the row in the ratio test and the margin below which Phase 1
+//                     starts at all; x0 > delta of the slack x0 entered on ends Phase 1 as infeasible
+//   PPG_TLP_OPT       reduced-cost threshold: Phase 2 is optimal when every d_j <= PPG_TLP_OPT * (1 + max_i |c_i + H_i theta|)
+//                     (the cost vector's own scale); Phase 1 uses it unscaled (the auxiliary row starts with coefficients -1)
+//   PPG_TLP_TINY      column entries at or below this do not block the ratio test (structural zeros left by elimination)
+//   PPG_TLP_PIV       a basic auxiliary variable at zero is pivoted out on its largest entry only when that exceeds this
+//   PPG_TLP_MAX_ITER  pivots per point (both phases) before the point is reported with PPG_TLP_ITERLIM; Bland's rule
+//                     (after PPG_BLAND_AFTER degenerate pivots) excludes cycling, so the cap is a guard against numerical
+//                     stalling only: a vertex path of a 256-row dictionary is far shorter
+#define PPG_TLP_TOL 1e-10
+#define PPG_TLP_OPT 1e-12
+#define PPG_TLP_TINY 1e-12
+#define PPG_TLP_PIV 1e-9
+#define PPG_TLP_MAX_ITER 4000
+// status per point: 0-3 mean what PPG_QP_* means
+#define PPG_TLP_OPTIMAL 0
+#define PPG_TLP_INFEASIBLE 1
+#define PPG_TLP_ITERLIM 2
+#define PPG_TLP_NUMERIC 3
+#define PPG_TLP_UNBOUNDED 4

@@ -94,6 +94,24 @@ class MPLP_Program:
             + 0.5 * theta_point.T @ self.Q_t @ theta_point
         return float(v[0, 0])
 
+    def _theta_solver(self):
+        if getattr(self, '_theta_solver_cache', None) is None:
+            from .solve_theta import ThetaLPSolver
+            self._theta_solver_cache = ThetaLPSolver(self)
+        return self._theta_solver_cache
+
+    def solve_theta(self, theta_point, deterministic_solver=None):
+        """LP at a fixed theta (mplp_program.py solve_theta) on the GPU (ppopt_b200.solve_theta.ThetaLPSolver): a
+        SolverOutput(obj, sol, slack, active_set, dual), or None when infeasible or unbounded.  ``deterministic_solver`` is
+        accepted for the reference's signature and ignored.  The solver is built on first use and caches the program data:
+        call again after changing the arrays of this object only on a new object."""
+        return self._theta_solver().solve_theta(theta_point)
+
+    def sample_theta_space(self, num_samples: int = 100):
+        """distinct optimal bases (equality rows first) of LPs solved at points sampled in Theta (mplp_program.py
+        sample_theta_space)"""
+        return self._theta_solver().sample_theta_space(num_samples)
+
 
 class MPQP_Program(MPLP_Program):
     r"""min 1/2 x'Qx + theta'H'x + c'x  with the constraints of MPLP_Program."""
