@@ -90,7 +90,7 @@ int ppgpu_level_eval(ppgpu_program* prog, const uint64_t* d_masks, int64_t n, in
  *                  vertex (slot 0) and at a later vertex of the walk that holds the candidate too (slot 1, may stay 0);
  *   d_parent_*     (or NULL / 0) describe the level the candidates were generated from: the feasible masks and the
  *                  workspace exactly as ppgpu_children_count / ppgpu_children_prepare left them (the workspace holds the
- *                  hash set of those masks), and the witnesses of those parents in the same order.  A candidate one of
+ *                  prefix-group index of those masks), and the witnesses of those parents in the same order.  A candidate one of
  *                  whose parents has a witness that also holds the added row is certified by that same vertex before any
  *                  LP work is spent on it (and passes the witness on).
  * Decisions are identical with and without witnesses; only which kernel exhibits the feasible point changes. */
@@ -99,9 +99,14 @@ int ppgpu_level_eval_w(ppgpu_program* prog, const uint64_t* d_masks, int64_t n, 
                        int32_t stages, uint64_t* d_witness, const uint64_t* d_parent_feas, int64_t parent_nf,
                        const void* d_parent_ws, const uint64_t* d_parent_wit, ppgpu_stream stream);
 
-/* Ordered compaction: ascending indices i with (d_status[i] & bits) == value.  Synchronises the stream to return the
- * count.  d_ws must hold ppgpu_scan_workspace_bytes(n) bytes. */
+/* Workspaces.  K6 (ppgpu_children_*, n = nf): the scan scratch and the prefix-group index of the feasible parents
+ * (~56 bytes per parent: a table, and per group the index of its first member and the bitmap of its members' highest
+ * rows).  Ordered compaction (ppgpu_level_select): ~8 bytes per candidate; any workspace of
+ * ppgpu_scan_workspace_bytes(n) bytes serves it as well. */
 size_t ppgpu_scan_workspace_bytes(int64_t n);
+size_t ppgpu_select_workspace_bytes(int64_t n);
+/* Ordered compaction: ascending indices i with (d_status[i] & bits) == value.  Synchronises the stream to return the
+ * count.  d_ws must hold ppgpu_select_workspace_bytes(n) bytes. */
 int ppgpu_level_select(ppgpu_program* prog, const uint8_t* d_status, int64_t n, uint8_t bits, uint8_t value,
                        int64_t* d_idx_out, int64_t* h_count, void* d_ws, size_t ws_bytes, ppgpu_stream stream);
 
@@ -117,12 +122,16 @@ int ppgpu_regions_emit(ppgpu_program* prog, const uint64_t* d_masks, const int64
 
 /* generate_children_sets + CombinationTester.check for all feasible parents (solver_utils.py:29-55,154-166):
  * pass 1 gathers the parents (d_feas_masks, nf x words), finds the surviving children of each (d_survive, nf x words)
- * and the exclusive scan of their counts (d_offsets, nf + 1); returns the total.  Pass 2 writes them, in order. */
+ * and the exclusive scan of their counts (d_offsets, nf + 1); returns the total.  Pass 2 writes them, in order.
+ * d_feas_idx selects the parents in the level's order, which is lexicographic (ppgpu_root_level, then this pass); a
+ * selection that is not strictly increasing in that order, or mixes cardinalities, is an error (reported by this call
+ * and by ppgpu_children_scan).  d_ws (ppgpu_scan_workspace_bytes(nf) bytes) keeps their prefix-group index for the
+ * next level's ppgpu_level_eval_w. */
 int ppgpu_children_count(ppgpu_program* prog, const uint64_t* d_masks, const int64_t* d_feas_idx, int64_t nf,
                          int32_t k_act, uint64_t* d_feas_masks, uint64_t* d_survive, int64_t* d_offsets,
                          int64_t* h_total, void* d_ws, size_t ws_bytes, ppgpu_stream stream);
 /* The same pass 1 in three steps, for callers that split the parents between GPUs (SURVEY.md 8e): prepare gathers the
- * parents and builds their hash set; count_range fills d_survive / d_counts for the parents [p_lo, p_hi) only (the
+ * parents and builds their prefix-group index; count_range fills d_survive / d_counts for the parents [p_lo, p_hi) only (the
  * caller zero-fills both and sums them across ranks); scan turns the counts (nf + 1 entries) into offsets. */
 int ppgpu_children_prepare(ppgpu_program* prog, const uint64_t* d_masks, const int64_t* d_feas_idx, int64_t nf,
                            uint64_t* d_feas_masks, void* d_ws, size_t ws_bytes, ppgpu_stream stream);

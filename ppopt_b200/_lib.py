@@ -41,6 +41,7 @@ SYMBOLS = {
     'ppgpu_level_eval': (ctypes.c_int, [_vp, _vp, _i64, _i32, _vp, _i32, _vp]),
     'ppgpu_level_eval_w': (ctypes.c_int, [_vp, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _i64, _vp, _vp, _vp]),
     'ppgpu_scan_workspace_bytes': (_sz, [_i64]),
+    'ppgpu_select_workspace_bytes': (_sz, [_i64]),
     'ppgpu_level_select': (ctypes.c_int, [_vp, _vp, _i64, _u8, _u8, _vp, ctypes.POINTER(_i64), _vp, _sz, _vp]),
     'ppgpu_regions_emit': (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     'ppgpu_children_count': (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, ctypes.POINTER(_i64), _vp, _sz, _vp]),

@@ -266,7 +266,7 @@ static_assert(PPGPU_WITNESS_SLOTS == PPG_WITNESS_SLOTS, "witness slots: include/
 // what ppgpu_level_eval_w adds to a level evaluation (all optional)
 struct WitnessIo {
     uint64_t* out = nullptr;                 // n x slots x W: witnesses of the candidates the walk certifies / that inherit one
-    const uint64_t* parent_feas = nullptr;   // parent level: feasible masks (nf x W), K6 workspace with their hash set,
+    const uint64_t* parent_feas = nullptr;   // parent level: feasible masks (nf x W), K6 workspace with their group index,
     long long parent_nf = 0;                 // and the witnesses of those parents in the same order
     const void* parent_ws = nullptr;
     const uint64_t* parent_wit = nullptr;
@@ -388,6 +388,7 @@ int ppgpu_level_eval_w(ppgpu_program* p, const uint64_t* d_masks, int64_t n, int
 }
 
 size_t ppgpu_scan_workspace_bytes(int64_t n) { return scan_workspace_bytes(n); }
+size_t ppgpu_select_workspace_bytes(int64_t n) { return select_workspace_bytes(n); }
 
 int ppgpu_level_select(ppgpu_program* p, const uint8_t* d_status, int64_t n, uint8_t bits, uint8_t value,
                        int64_t* d_idx_out, int64_t* h_count, void* d_ws, size_t ws_bytes, ppgpu_stream stream) {
@@ -396,8 +397,8 @@ int ppgpu_level_select(ppgpu_program* p, const uint8_t* d_status, int64_t n, uin
     if (n <= 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     // the count lands in the last workspace word, then comes back to the host
-    if (ws_bytes < scan_workspace_bytes(n)) return fail_msg("workspace too small");
-    long long* d_count = (long long*)d_ws + (scan_workspace_bytes(n) / sizeof(long long) - 1);
+    if (ws_bytes < select_workspace_bytes(n)) return fail_msg("workspace too small");
+    long long* d_count = (long long*)d_ws + (select_workspace_bytes(n) / sizeof(long long) - 1);
     cudaError_t e;
     {
         ProfScope ps(p, st, 6);
@@ -443,11 +444,13 @@ int ppgpu_children_count(ppgpu_program* p, const uint64_t* d_masks, const int64_
                            (long long*)d_offsets, d_ws, ws_bytes, p->d_counters, st);
     }
     if (e != cudaSuccess) return fail("K6 count", e);
-    p->launches += 5;
-    long long tot = 0;
+    p->launches += 12;   // prepare 8, count 1, scan 3
+    long long tot = 0, disorder = 0;
     e = cudaMemcpyAsync(&tot, (long long*)d_offsets + nf, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&disorder, children_order_flag(d_ws, nf), sizeof(long long), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail("K6 total", e);
+    if (disorder) return fail_msg("K6: the feasible parents are not one level's sets in lexicographic order");
     *h_total = tot;
     return 0;
 }
@@ -462,7 +465,7 @@ int ppgpu_children_prepare(ppgpu_program* p, const uint64_t* d_masks, const int6
         e = children_prepare(p->dev, d_masks, (const long long*)d_feas_idx, nf, d_feas_masks, d_ws, ws_bytes, (cudaStream_t)stream);
     }
     if (e != cudaSuccess) return fail("K6 prepare", e);
-    p->launches += 3;
+    p->launches += 8;    // gather, run flags, scan 3, groups, table clear, table insert (+ a memset)
     return 0;
 }
 
@@ -498,10 +501,12 @@ int ppgpu_children_scan(ppgpu_program* p, int64_t* d_counts_to_offsets, int64_t 
     }
     if (e != cudaSuccess) return fail("K6 scan", e);
     p->launches += 2;
-    long long tot = 0;
+    long long tot = 0, disorder = 0;
     e = cudaMemcpyAsync(&tot, (long long*)d_counts_to_offsets + nf, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&disorder, children_order_flag(d_ws, nf), sizeof(long long), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail("K6 total", e);
+    if (disorder) return fail_msg("K6: the feasible parents are not one level's sets in lexicographic order");
     *h_total = tot;
     return 0;
 }

@@ -54,12 +54,12 @@ enum Counter {
     CNT_K2_LPS, CNT_K2_PIVOTS, CNT_K2_WORK,
     CNT_K4_LPS, CNT_K4_PIVOTS, CNT_K4_WORK,
     CNT_K5_LPS, CNT_K5_PIVOTS, CNT_K5_WORK,
-    CNT_NUMERIC, CNT_BORDER, CNT_K6_LOOKUPS,
+    CNT_NUMERIC, CNT_BORDER, CNT_K6_LOOKUPS,          // 10, 11, 12: K6 prefix-group probes (<= k per parent)
     CNT_K2A_TRIED, CNT_K2A_CERTIFIED, CNT_K2A_STEPS,  // 13, 14, 15
     CNT_K2A_WORK,                                     // 16: steps x R0 x (1 + k') useful FMAs
     CNT_K2W_CERTIFIED, CNT_K2W_PIVOTS, CNT_K2W_WORK,  // 17, 18, 19: vertex walk (pivots x basic rows x columns FMAs)
     CNT_K2W_GIVEUP,                                   // 20: drives abandoned (iteration cap, empty face, dependent row)
-    CNT_INHERITED, CNT_INHERIT_LOOKUPS,               // 21, 22: certificates inherited from parent witnesses / hash look-ups
+    CNT_INHERITED, CNT_INHERIT_LOOKUPS,               // 21, 22: certificates inherited from parent witnesses / parents looked up
     CNT_COUNT = 24
 };
 

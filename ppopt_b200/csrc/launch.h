@@ -51,7 +51,7 @@ cudaError_t launch_k2w(const DevProgram& P, const uint64_t* masks, long long n, 
 // ints of scratch launch_k2w wants for ordering the work items of an n-candidate launch (may be passed as null: natural order)
 size_t k2w_order_scratch_ints(long long n);
 // certificates INHERITED from the previous level: a candidate is feasible when the witness vertex of one of its parents
-// (candidate minus one row, looked up in the hash set K6 built for that level) has the dropped row active as well
+// (candidate minus one row, looked up in the prefix-group index K6 built for that level) has the dropped row active as well
 cudaError_t launch_inherit(const DevProgram& P, const uint64_t* masks, long long n, uint8_t* status, uint64_t* witness_out,
                            const uint64_t* parent_feas, long long parent_nf, const void* parent_ws, const uint64_t* parent_wit,
                            unsigned long long* counters, cudaStream_t st);
@@ -68,6 +68,8 @@ cudaError_t launch_k5(const DevProgram& P, const uint64_t* masks, const long lon
                       unsigned long long* counters, int sm_count, cudaStream_t st);
 
 size_t scan_workspace_bytes(long long n);
+size_t select_workspace_bytes(long long n);
+const long long* children_order_flag(const void* ws, long long nf);
 cudaError_t select_indices(const uint8_t* status, long long n, uint8_t bits, uint8_t value, long long* idx_out,
                            long long* d_count, void* ws, size_t ws_bytes, cudaStream_t st);
 cudaError_t root_level(const DevProgram& P, uint64_t* masks, long long* d_count, cudaStream_t st);

@@ -129,7 +129,7 @@ class Engine:
         n = status.shape[0]
         if n == 0:
             return self.empty((0,), torch.int64)
-        ws_bytes = self.lib.ppgpu_scan_workspace_bytes(n)
+        ws_bytes = self.lib.ppgpu_select_workspace_bytes(n)
         ws = self.empty(((ws_bytes + 7) // 8,), torch.int64)
         idx = self.empty((n,), torch.int64)
         cnt = ctypes.c_int64(0)
@@ -152,7 +152,7 @@ class Engine:
     def children(self, masks: torch.Tensor, feas_idx: torch.Tensor, k_act: int, dist=None, keep: Optional[dict] = None) -> torch.Tensor:
         """next level's candidates; with dist (torch.distributed, world > 1) the pruning look-ups of the parents are split
         between the ranks and the per-parent results summed (every rank ends up with the identical child array).
-        ``keep`` (dict) receives the gathered feasible masks and the workspace holding their hash set: what the next
+        ``keep`` (dict) receives the gathered feasible masks and the workspace holding their prefix-group index: what the next
         level needs to look its candidates' parents up (witness inheritance)"""
         nf = feas_idx.shape[0]
         if nf == 0:
@@ -401,7 +401,7 @@ def build_regions(eng: Engine, cr_cls, active_sets, k_act, laws, rows, flags, in
 
 class ParentLevel:
     """What a level leaves behind for the next one (witness inheritance): its feasible masks in K6's order, the K6 workspace
-    holding their hash set, and the witnesses (active-row masks of the certifying vertices) in the same order."""
+    holding their prefix-group index, and the witnesses (active-row masks of the certifying vertices) in the same order."""
     __slots__ = ('feas_masks', 'ws', 'nf', 'wit')
 
     def __init__(self, feas_masks, ws, nf, wit):
