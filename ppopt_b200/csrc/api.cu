@@ -423,10 +423,10 @@ int ppgpu_regions_emit(ppgpu_program* p, const uint64_t* d_masks, const int64_t*
     {
         ProfScope ps(p, (cudaStream_t)stream, 3);
         e = launch_k5(p->dev, d_masks, (const long long*)d_sel, n_sel, k_act, d_laws, d_rows, d_flags, d_info, d_status,
-                      p->d_counters, p->sm_count, (cudaStream_t)stream);
+                      next_queue(p, (cudaStream_t)stream), p->d_counters, p->sm_count, (cudaStream_t)stream);
     }
     if (e != cudaSuccess) return fail("K5 emit", e);
-    p->launches++;
+    p->launches += k5_launches(p->dev.t);
     return 0;
 }
 

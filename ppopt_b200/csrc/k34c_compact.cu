@@ -19,6 +19,7 @@
 #include "launch.h"
 #include "lp_core.cuh"
 
+#include <algorithm>
 #include <cstdlib>
 
 namespace ppgpu {
@@ -168,7 +169,7 @@ __device__ __noinline__ K4cOut k4c_solve(double* __restrict__ Tab, unsigned char
 __global__ void __launch_bounds__(128)
 k34c_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, int k_act, uint8_t* __restrict__ status,
             unsigned long long* __restrict__ queue, unsigned long long* __restrict__ counters, int use_pre, int warp_bytes,
-            int lds) {
+            int lds, int per_item) {
     extern __shared__ unsigned char k34c_smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int t = P.t, t1 = P.t + 1, mi = P.mi, W = P.W, k = k_act, m = P.R0;
@@ -184,19 +185,19 @@ k34c_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, int k
     int* nbv = reinterpret_cast<int*>(base); base += (size_t)((lds + 1) & ~1) * 4;
     unsigned char* flag = base;
     unsigned long long n_lp = 0, n_piv = 0, n_work = 0, n_num = 0;
-    const long long nblocks = (n + 31) / 32;
+    const long long nblocks = (n + per_item - 1) / per_item;
     for (;;) {
         unsigned long long v = 0;
         if (lane == 0) v = atomicAdd(queue, 1ull);
         const long long item = (long long)__shfl_sync(PPG_FULL, v, 0);
         if (item >= nblocks) break;
-        const long long c0 = item * 32 + lane;
-        const uint8_t sb = c0 < n ? status[c0] : 0;
+        const long long c0 = item * per_item + lane;
+        const uint8_t sb = (lane < per_item && c0 < n) ? status[c0] : 0;
         unsigned todo = __ballot_sync(PPG_FULL, (sb & PPG_ST_FEAS) && (!use_pre || (sb & PPG_ST_PRE)));
         while (todo) {
             const int src = __ffs((int)todo) - 1;
             todo &= todo - 1u;
-            const long long idx = item * 32 + src;
+            const long long idx = item * per_item + src;
             uint8_t st = (uint8_t)__shfl_sync(PPG_FULL, (int)sb, src);
             if (use_pre) st &= (uint8_t)~PPG_ST_PRE;
             const uint64_t* mk = masks + idx * W;
@@ -375,11 +376,17 @@ cudaError_t launch_k34_compact(const DevProgram& P, const uint64_t* masks, long 
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k34c_kernel, 32 * WPC, smem);
     if (e != cudaSuccess) return e;
     if (occ < 1) occ = 1;
+    // a warp decides the candidates of a queue item one after another: 32 per item, fewer when the level would leave
+    // warps of the resident grid without an item (level 1: 100 candidates were 4 items, 25 candidates in a row per warp)
+    const long long warps = (long long)sm_count * occ * WPC;
+    const int per_item = (int)std::min<long long>(32, std::max<long long>(1, (n + warps - 1) / warps));
+    const long long items = (n + per_item - 1) / per_item;
     long long grid = (long long)sm_count * occ;
-    const long long need = (n + 32 * WPC - 1) / (32 * WPC);
+    const long long need = (items + WPC - 1) / WPC;
     if (grid > need) grid = need;
     if (grid < 1) grid = 1;
-    k34c_kernel<<<(unsigned)grid, 32 * WPC, smem, st>>>(P, masks, n, k_act, status, queue, counters, use_pre, (int)wb, lds);
+    k34c_kernel<<<(unsigned)grid, 32 * WPC, smem, st>>>(P, masks, n, k_act, status, queue, counters, use_pre, (int)wb, lds,
+                                                        per_item);
     *handled = true;
     return cudaGetLastError();
 }

@@ -11,6 +11,18 @@
 //   5. exact-duplicate removal keeping the first occurrence         (constraint_utilities.py:125-134)
 // Output per region: laws (n+k) x (t+1) [const | theta], rows R0 x (t+1) [f | a] normalised, int flags per row
 // (bit0 nonzero, bit1 non-redundant, bit2 duplicate of an earlier kept row) and info[4] = {region?, radius, lo, hi}.
+//
+// Three launches (t > 1):
+//   K5a k5_emit_kernel<.., false>  one CTA per region: steps 1-3 (t == 1: all five, the redundancy test is interval arithmetic)
+//   K5b k5_redund_kernel           step 4 as ONE batch of (region, row) LPs, one warp per LP, from the rows K5a wrote
+//   K5c k5_dedupe_kernel           step 5, one warp per region
+// A region's redundancy LPs are independent of each other, but inside one CTA four warps solve the ~110 LPs of a region
+// one after another, at the 222 registers of the LU + Chebyshev kernel (2 CTAs per SM).  K5b holds only the LP, runs 4x
+// more warps per SM and spreads the LPs of all regions over the whole device.  Every LP is the same routine on the same
+// registers as before, so laws, rows, flags, info, status and counters are bit-identical to the fused kernel
+// (k5_emit_kernel<.., true>, selected with PPGPU_K5_FUSED=1).
+#include <cstdlib>
+
 #include "common.cuh"
 #include "launch.h"
 #include "lp_core.cuh"
@@ -20,7 +32,7 @@ namespace ppgpu {
 constexpr int K5_WARPS = 4;
 constexpr int K5_THREADS = K5_WARPS * 32;
 
-template <int RPT, int DC>
+template <int RPT, int DC, bool FUSED>
 __global__ void __launch_bounds__(K5_THREADS)
 k5_emit_kernel(DevProgram P, const uint64_t* __restrict__ masks, const long long* __restrict__ sel, long long n_sel,
                int k_act, double* __restrict__ laws_out, double* __restrict__ rows_out, int32_t* __restrict__ flags_out,
@@ -274,7 +286,7 @@ k5_emit_kernel(DevProgram P, const uint64_t* __restrict__ masks, const long long
                         const double q = rows[(size_t)r * 2] / rows[(size_t)r * 2 + 1];
                         if (lo <= q && q <= hi) keptf[r] = 1;
                     }
-            } else {
+            } else if constexpr (FUSED) {
                 for (int a = warp; a < R0; a += K5_WARPS) {
                     if (!(flags[a] & 1)) continue;
                     double T[RPT][DC];
@@ -298,7 +310,7 @@ k5_emit_kernel(DevProgram P, const uint64_t* __restrict__ masks, const long long
             __syncthreads();
             for (int r = tid; r < R0; r += K5_THREADS) if (keptf[r]) flags[r] |= 2;
             __syncthreads();
-            if (t != 1) {
+            if (FUSED && t != 1) {
                 // duplicates among kept rows (value equality, first occurrence survives); verdicts land after a barrier
                 for (int i = tid; i < R0; i += K5_THREADS) {
                     bool dup = false;
@@ -339,11 +351,117 @@ k5_emit_kernel(DevProgram P, const uint64_t* __restrict__ masks, const long long
     }
 }
 
+// K5b: the redundancy LPs of every region of the launch as one flat list of (region, row) pairs, pair = si * R0 + row.
+// Warps take K5B_CHUNK consecutive pairs at a time from an atomic queue (consecutive warps work on the same region, whose
+// rows then come from L1 / L2); pairs of a non-region or of a zero row are dropped without an LP.  The LP, its tableau and
+// the verdict rule are those of the fused kernel.  The verdict lands in bit 1 of the row's flag word, which no other warp
+// of the launch writes (bit 0, the only bit read here, never changes).
+constexpr int K5B_WARPS = 4;
+constexpr int K5B_CHUNK = 4;
+
+// CTAs per SM the register budget is planned for, by tableau doubles a lane: <= 16: 4 (16 warps, <= 128 registers a thread);
+// 32: 3 (<= 168; at 128 the bench instance <4, 8> spills); 64: 2; 128 (<8, 16>): 1, where the tableau alone needs 256
+template <int RPT, int DC>
+constexpr int k5b_min_ctas() { return RPT * DC <= 16 ? 4 : (RPT * DC <= 32 ? 3 : (RPT * DC <= 64 ? 2 : 1)); }
+
+template <int RPT, int DC>
+__global__ void __launch_bounds__(K5B_WARPS * 32, k5b_min_ctas<RPT, DC>())
+k5_redund_kernel(int R0, int t1, long long n_sel, const double* __restrict__ rows_out, int32_t* flags_out,
+                 const double* __restrict__ info_out, unsigned long long* __restrict__ queue,
+                 unsigned long long* __restrict__ counters) {
+    typedef LpCore<1, RPT, DC> Core;
+    __shared__ typename Core::Shared sh_all[K5B_WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long n_pairs = n_sel * R0;
+    unsigned long long n_lp = 0, n_piv = 0, n_work = 0;
+    for (;;) {
+        unsigned long long v = 0;
+        if (lane == 0) v = atomicAdd(queue, (unsigned long long)K5B_CHUNK);
+        const long long base = (long long)__shfl_sync(PPG_FULL, v, 0);
+        if (base >= n_pairs) break;
+        bool live = false;
+        if (lane < K5B_CHUNK && base + lane < n_pairs) {
+            const long long pr = base + lane;
+            live = __ldg(info_out + (pr / R0) * 4) == 1.0 && (flags_out[pr] & 1);
+        }
+        unsigned todo = __ballot_sync(PPG_FULL, live);
+        while (todo) {
+            const int src = __ffs((int)todo) - 1;
+            todo &= todo - 1u;
+            const long long pr = base + src, si = pr / R0;
+            const int a = (int)(pr - si * R0);
+            const double* rows = rows_out + (size_t)si * R0 * t1;
+            const int32_t* flags = flags_out + (size_t)si * R0;
+            double T[RPT][DC];
+            int rflag[RPT];
+            static_for<RPT>([&](auto RR) {
+                constexpr int rr = decltype(RR)::value;
+                const int row = rr * 32 + lane;
+                const bool on = row < R0 && (flags[row] & 1);
+#pragma unroll
+                for (int c = 0; c < DC; ++c)
+                    T[rr][c] = (on && c < t1) ? __ldg(rows + (size_t)row * t1 + c) : ((on && c == t1 && row != a) ? 1.0 : 0.0);
+                rflag[rr] = on ? (row == a ? 2 : 1) : 0;
+            });
+            LpOut res = Core::solve(sh_all[warp], T, rflag, R0, t1, -PPG_REDUND_TOL, false, lane);
+            n_lp++; n_piv += res.pivots; n_work += (unsigned long long)res.work;
+            const bool feas = res.code == PPG_LP_EARLY || res.code == PPG_LP_UNBOUNDED ||
+                              (res.code == PPG_LP_OPTIMAL && res.beta >= -PPG_REDUND_TOL);
+            if (lane == 0 && feas) atomicOr(flags_out + pr, 2);
+        }
+    }
+    if (lane == 0 && n_lp) {
+        atomicAdd(&counters[CNT_K5_LPS], n_lp);
+        atomicAdd(&counters[CNT_K5_PIVOTS], n_piv);
+        atomicAdd(&counters[CNT_K5_WORK], n_work);
+    }
+}
+
+// K5c: exact duplicates among the kept rows of a region (value equality, the first occurrence survives), one warp per region.
+// A row's verdict is taken before any bit 2 of the region is written.
+constexpr int K5C_WARPS = 4;
+
+__global__ void __launch_bounds__(K5C_WARPS * 32)
+k5_dedupe_kernel(int R0, int t1, long long n_sel, const double* __restrict__ rows_out, int32_t* __restrict__ flags_out,
+                 const double* __restrict__ info_out) {
+    const int lane = threadIdx.x & 31;
+    const long long nw = (long long)gridDim.x * K5C_WARPS;
+    for (long long si = (long long)blockIdx.x * K5C_WARPS + (threadIdx.x >> 5); si < n_sel; si += nw) {
+        if (__ldg(info_out + si * 4) != 1.0) continue;
+        const double* rows = rows_out + (size_t)si * R0 * t1;
+        int32_t* flags = flags_out + (size_t)si * R0;
+        unsigned dup = 0;   // bit q: row lane + 32 q
+        for (int i = lane, q = 0; i < R0; i += 32, ++q) {
+            if ((flags[i] & 3) != 3) continue;
+            bool d = false;
+            for (int j = 0; j < i && !d; ++j) {
+                if ((flags[j] & 3) != 3) continue;
+                bool same = true;
+                for (int c = 0; c < t1 && same; ++c) same = __ldg(rows + (size_t)i * t1 + c) == __ldg(rows + (size_t)j * t1 + c);
+                d = same;
+            }
+            if (d) dup |= 1u << q;
+        }
+        __syncwarp();
+        for (int i = lane, q = 0; i < R0; i += 32, ++q)
+            if ((dup >> q) & 1u) flags[i] |= 4;
+    }
+}
+
+// PPGPU_K5_FUSED=1: the fused one-CTA-per-region kernel (the A/B reference of the three launches)
+static bool k5_fused() {
+    static const bool on = getenv("PPGPU_K5_FUSED") && atoi(getenv("PPGPU_K5_FUSED")) != 0;
+    return on;
+}
+
+int k5_launches(int t) { return k5_fused() || t == 1 ? 1 : 3; }
+
 template <int RPT, int DC>
 static cudaError_t launch_k5_t(const DevProgram& P, const uint64_t* masks, const long long* idx, long long n_sel, int k_act,
                                double* laws, double* rows, int32_t* flags, double* info, uint8_t* status,
-                               unsigned long long* counters, int sm_count, cudaStream_t st) {
-    auto kern = k5_emit_kernel<RPT, DC>;
+                               unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st) {
+    const bool fused = k5_fused();
+    auto kern = fused ? k5_emit_kernel<RPT, DC, true> : k5_emit_kernel<RPT, DC, false>;
     const int k = P.ne + k_act, N = P.n + k, ld = N + P.t + 1;
     const size_t smem = ((size_t)N * ld + (size_t)P.R0 * (P.t + 1)) * sizeof(double) + (size_t)(2 * P.R0 + k + 2) * sizeof(int);
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
@@ -354,19 +472,36 @@ static cudaError_t launch_k5_t(const DevProgram& P, const uint64_t* masks, const
     if (grid > cap) grid = cap;
     if (grid < 1) return cudaSuccess;
     kern<<<(unsigned)grid, K5_THREADS, smem, st>>>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, counters);
+    if ((e = cudaGetLastError()) != cudaSuccess || fused || P.t == 1) return e;
+
+    auto kb = k5_redund_kernel<RPT, DC>;
+    if ((e = fit_smem(kb, 0)) != cudaSuccess) return e;
+    int occ = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kb, K5B_WARPS * 32, 0)) != cudaSuccess) return e;
+    if (occ < 1) occ = 1;
+    const long long items = (n_sel * P.R0 + K5B_CHUNK - 1) / K5B_CHUNK;
+    grid = (items + K5B_WARPS - 1) / K5B_WARPS;
+    if (grid > (long long)sm_count * occ) grid = (long long)sm_count * occ;
+    kb<<<(unsigned)grid, K5B_WARPS * 32, 0, st>>>(P.R0, P.t + 1, n_sel, rows, flags, info, queue, counters);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+
+    if ((e = fit_smem(k5_dedupe_kernel, 0)) != cudaSuccess) return e;
+    grid = (n_sel + K5C_WARPS - 1) / K5C_WARPS;
+    if (grid > (long long)sm_count * 16) grid = (long long)sm_count * 16;
+    k5_dedupe_kernel<<<(unsigned)grid, K5C_WARPS * 32, 0, st>>>(P.R0, P.t + 1, n_sel, rows, flags, info);
     return cudaGetLastError();
 }
 
-#define K5_RPT_SWITCH(DCV)                                                                                                            \
-    if (P.R0 <= 32) return launch_k5_t<1, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, counters, sm_count, st);  \
-    if (P.R0 <= 64) return launch_k5_t<2, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, counters, sm_count, st);  \
-    if (P.R0 <= 128) return launch_k5_t<4, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, counters, sm_count, st); \
-    if (P.R0 <= 256) return launch_k5_t<8, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, counters, sm_count, st); \
+#define K5_RPT_SWITCH(DCV)                                                                                                                   \
+    if (P.R0 <= 32) return launch_k5_t<1, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, queue, counters, sm_count, st);  \
+    if (P.R0 <= 64) return launch_k5_t<2, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, queue, counters, sm_count, st);  \
+    if (P.R0 <= 128) return launch_k5_t<4, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, queue, counters, sm_count, st); \
+    if (P.R0 <= 256) return launch_k5_t<8, DCV>(P, masks, idx, n_sel, k_act, laws, rows, flags, info, status, queue, counters, sm_count, st); \
     return cudaErrorInvalidValue;
 
 cudaError_t launch_k5(const DevProgram& P, const uint64_t* masks, const long long* idx, long long n_sel, int k_act,
                       double* laws, double* rows, int32_t* flags, double* info, uint8_t* status,
-                      unsigned long long* counters, int sm_count, cudaStream_t st) {
+                      unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st) {
     if (P.t + 2 <= 8) { K5_RPT_SWITCH(8) }
     if (P.t + 2 <= 16) { K5_RPT_SWITCH(16) }
     return cudaErrorInvalidValue;

@@ -63,9 +63,12 @@ cudaError_t launch_k34_compact(const DevProgram& P, const uint64_t* masks, long 
 // general (LU) path: marks every feasible candidate that the reference would hand to check_optimality
 cudaError_t launch_mark_general(const DevProgram& P, long long n, int k_act, uint8_t* status, cudaStream_t st);
 
+// region emission: K5a (KKT, rows, full-dimension test), K5b (redundancy LPs, one warp per LP), K5c (duplicates);
+// k5_launches(t) kernels per call
 cudaError_t launch_k5(const DevProgram& P, const uint64_t* masks, const long long* idx, long long n_sel, int k_act,
                       double* laws, double* rows, int32_t* flags, double* info, uint8_t* status,
-                      unsigned long long* counters, int sm_count, cudaStream_t st);
+                      unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st);
+int k5_launches(int t);
 
 size_t scan_workspace_bytes(long long n);
 size_t select_workspace_bytes(long long n);
