@@ -204,6 +204,44 @@ int ppgpu_solve_theta_lp_batch(ppgpu_program* prog, const double* d_theta, int64
 int ppgpu_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_t n_polytopes, int32_t t, int32_t max_rows,
                           double* d_radius, int32_t* d_code, ppgpu_stream stream);
 
+/* The relaxation tree of a mixed-integer program (mpMILP / mpMIQP): which assignments of the binaries have a feasible
+ * relaxation.  Replaces the reference's MITree.__init__ / get_full_leafs (mitree.py) and, at the leaves, its
+ * check_bin_feasibility (mpmilp_program.py); the reference runs a MILP per node with Gurobi, here an inner node answers
+ * the LP RELAXATION of its partial assignment (sound pruning: an infeasible relaxation has no feasible leaf below it) and a
+ * leaf, where every binary is fixed, answers exactly the LP the MILP reduces to.  A handle of its own (csrc/k11_mitree.cu):
+ * none of ppgpu_program_create's limits apply.
+ *
+ * The lifted LP: variables z = (x, theta) (n + t, x in program order), rows A x - F theta <= b (= b on the equality rows
+ * 0..n_eq-1 of dims), A_t theta <= b_t, and y_k <= u_k, -y_k <= -l_k for every binary y_k = x[binary_indices[k]].  The
+ * root relaxes every binary to [0, 1]; a node at depth d fixes y_k (k < d) to bit k of its uint64.  A node is feasible iff
+ * its relaxation has a point within PPG_FEAS_TOL (1 + |rhs|) on every row (csrc/tolerances.h, PPG_TREE_*).
+ *   create   dims (n, t, m, q, n_eq; is_qp ignored: the objective plays no part), binary_indices (nb <= 63 column indices of
+ *            A), the arrays of ppgpu_program_create.  Returns -2 (ppgpu_last_error says why) when the equalities are rank
+ *            deficient, when the lifted rows have rank below the n + t - n_eq free variables (no vertex), or when the
+ *            lifted system exceeds the kernel's envelope: (m - n_eq) + q + 2 nb <= 256 rows, n + t - n_eq <= 64 columns.
+ *   eval     d_nodes (n uint64) at `depth`: d_status (n uint8: 0 feasible, 1 infeasible, 2 iteration cap, 3 numerical
+ *            breakdown), d_point (n x (n + t) or NULL: the feasible point, NaN elsewhere), d_iters (n int32 or NULL:
+ *            pivots of the node's LP, -1 when the node inherited its parent's point).  d_parent_point / d_parent_of (or
+ *            NULL): the points of the previous depth's eval and, per node, the index of its parent there
+ *            (ppgpu_tree_children writes it); when given and inheritance is on, a node whose parent's point, with y_{depth-1}
+ *            snapped to the node's value, satisfies every row is feasible without an LP.  Statuses do not depend on it.
+ *   children the nodes with status 0 in order (d_idx, n int64 scratch), each followed by its two children at depth + 1:
+ *            d_children[2j] fixes y_depth = 0, d_children[2j + 1] fixes it to 1 (2n uint64), d_parent_of the index of the
+ *            parent (2n int64); h_count = number of feasible parents.  d_ws: ppgpu_select_workspace_bytes(n) bytes.
+ *            Synchronises the stream. */
+typedef struct ppgpu_tree ppgpu_tree;
+int ppgpu_tree_create(const ppgpu_dims* dims, const int32_t* h_binary_indices, int32_t nb, const double* h_A, const double* h_b,
+                      const double* h_F, const double* h_A_t, const double* h_b_t, int device, ppgpu_tree** out);
+int ppgpu_tree_destroy(ppgpu_tree* tree);
+/*   PPGPU_TREE_OPT_INHERIT  1 / 0 (default; the environment's PPGPU_TREE_INHERIT at create): point inheritance on / off */
+#define PPGPU_TREE_OPT_INHERIT 0
+int ppgpu_tree_set_option(ppgpu_tree* tree, int32_t option, int64_t value);
+int ppgpu_tree_eval(ppgpu_tree* tree, const uint64_t* d_nodes, int64_t n, int32_t depth, uint8_t* d_status, double* d_point,
+                    const double* d_parent_point, const int64_t* d_parent_of, int32_t* d_iters, ppgpu_stream stream);
+int ppgpu_tree_children(ppgpu_tree* tree, const uint64_t* d_nodes, const uint8_t* d_status, int64_t n, int32_t depth,
+                        int64_t* d_idx, uint64_t* d_children, int64_t* d_parent_of, int64_t* h_count, void* d_ws,
+                        size_t ws_bytes, ppgpu_stream stream);
+
 /* cumulative device counters (LPs, pivots, useful FMAs per kernel family, borderline/numeric flags) */
 int ppgpu_counters(ppgpu_program* prog, uint64_t* h_out, int32_t reset, ppgpu_stream stream);
 

@@ -16,6 +16,7 @@ COUNTER_NAMES = ('k1_candidates', 'k2_lps', 'k2_pivots', 'k2_work', 'k4_lps', 'k
 # status bits (csrc/tolerances.h)
 ST_RANK, ST_FEAS, ST_OPT, ST_REGION, ST_BORDER, ST_NUMERIC, ST_THIN = 1, 2, 4, 8, 16, 32, 64
 OPT_K2W_MIN = 0   # ppgpu_set_option (include/ppgpu.h)
+TREE_OPT_INHERIT = 0   # ppgpu_tree_set_option
 WITNESS_SLOTS = 2  # PPGPU_WITNESS_SLOTS
 
 
@@ -58,6 +59,11 @@ SYMBOLS = {
     'ppgpu_solve_theta_batch': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'ppgpu_solve_theta_lp_batch': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'ppgpu_chebyshev_batch': (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
+    'ppgpu_tree_create': (ctypes.c_int, [ctypes.POINTER(Dims), _vp, _i32] + [_vp] * 5 + [ctypes.c_int, ctypes.POINTER(_vp)]),
+    'ppgpu_tree_destroy': (ctypes.c_int, [_vp]),
+    'ppgpu_tree_set_option': (ctypes.c_int, [_vp, _i32, _i64]),
+    'ppgpu_tree_eval': (ctypes.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'ppgpu_tree_children': (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, ctypes.POINTER(_i64), _vp, _sz, _vp]),
     'ppgpu_measure_fp64_peak': (ctypes.c_int, [_i32, ctypes.POINTER(ctypes.c_double), _vp]),
 }
 

@@ -629,6 +629,134 @@ int ppgpu_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_
     return 0;
 }
 
+}  // extern "C"
+
+// ---- K11: the relaxation tree of a mixed-integer program (a handle of its own: none of the path's limits apply)
+struct ppgpu_tree {
+    TreeProgram host;
+    DevTree dev;
+    int device = 0;
+    int sm_count = 0;
+    bool inherit = false;
+    std::vector<void*> allocs;
+};
+
+template <class T>
+static cudaError_t tree_upload(ppgpu_tree* h, const std::vector<T>& v, const T** out) {
+    void* d = nullptr;
+    const size_t bytes = (v.size() ? v.size() : 1) * sizeof(T);
+    cudaError_t e = cudaMalloc(&d, bytes);
+    if (e != cudaSuccess) return e;
+    h->allocs.push_back(d);
+    if (v.size()) e = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
+    *out = (const T*)d;
+    return e;
+}
+
+extern "C" {
+
+int ppgpu_tree_create(const ppgpu_dims* d, const int32_t* binary_indices, int32_t nb, const double* A, const double* b,
+                      const double* F, const double* A_t, const double* b_t, int device, ppgpu_tree** out) {
+    if (!d || !out || (nb > 0 && !binary_indices)) return fail_msg("null argument");
+    if (nb < 0 || nb > 63) return fail_msg("the tree supports 0 <= nb <= 63 binaries (a node is one uint64 of fixed bits)");
+    ppgpu_tree* h = new ppgpu_tree();
+    std::vector<int> bin(binary_indices, binary_indices + nb);
+    if (!build_tree_dictionary(d->n, d->t, d->m, d->q, d->n_eq, nb, bin.data(), A, b, F, A_t, b_t, h->host)) {
+        std::string m = "tree: " + h->host.error;
+        delete h;
+        return fail_msg(m);
+    }
+    const TreeProgram& R = h->host;
+    // K11 keeps a node's dictionary in the shared memory of one warp: K9's envelope
+    if (R.rows > 256) {
+        std::string m = "tree: the lifted system has " + std::to_string(R.rows) +
+                        " inequality rows ((m - n_eq) + q + 2 nb); at most 256 are supported";
+        delete h;
+        return fail_msg(m);
+    }
+    if (R.cols > 64) {
+        std::string m = "tree: the lifted system has " + std::to_string(R.cols) +
+                        " free variables (n + t - n_eq); at most 64 are supported";
+        delete h;
+        return fail_msg(m);
+    }
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) { delete h; return fail("cudaSetDevice", e); }
+    h->device = device;
+    cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
+    const char* env = getenv("PPGPU_TREE_INHERIT");
+    h->inherit = env && atoi(env) != 0;
+    DevTree& D = h->dev;
+    D.nv = R.nv; D.rows = R.rows; D.cols = R.cols; D.rb0 = R.rb0; D.tp = R.tp; D.ld = R.ld; D.ne = R.ne; D.nb = R.nb;
+#define UP(field, vecname) if ((e = tree_upload(h, R.vecname, &D.field)) != cudaSuccess) { ppgpu_tree_destroy(h); return fail("tree upload " #field, e); }
+    UP(D0, D0) UP(bvar, bvar) UP(nvar, nvar) UP(hs, hs) UP(z0, z0) UP(Q2, Q2) UP(Arows, Arows) UP(brows, brows) UP(bin, bin)
+#undef UP
+    *out = h;
+    return 0;
+}
+
+int ppgpu_tree_destroy(ppgpu_tree* h) {
+    if (!h) return 0;
+    for (void* d : h->allocs) cudaFree(d);
+    delete h;
+    return 0;
+}
+
+int ppgpu_tree_set_option(ppgpu_tree* h, int32_t option, int64_t value) {
+    if (!h) return fail_msg("null argument");
+    switch (option) {
+        case PPGPU_TREE_OPT_INHERIT: h->inherit = value != 0; return 0;
+        default: return fail_msg("unknown option");
+    }
+}
+
+int ppgpu_tree_eval(ppgpu_tree* h, const uint64_t* d_nodes, int64_t n, int32_t depth, uint8_t* d_status, double* d_point,
+                    const double* d_parent_point, const int64_t* d_parent_of, int32_t* d_iters, ppgpu_stream stream) {
+    if (!h) return fail_msg("null argument");
+    if (n < 0) return fail_msg("negative size");
+    if (depth < 0 || depth > h->host.nb) return fail_msg("depth outside [0, nb]");
+    if (n == 0) return 0;
+    if (!d_nodes || !d_status) return fail_msg("null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaSetDevice(h->device);
+    if (e != cudaSuccess) return fail("cudaSetDevice", e);
+    const bool inherit = h->inherit && depth >= 1 && d_parent_point && d_parent_of;
+    if (inherit) {
+        e = launch_tree_inherit(h->dev, d_nodes, n, depth, d_parent_point, (const long long*)d_parent_of, d_status, d_point,
+                                d_iters, st);
+        if (e != cudaSuccess) return fail("K11 inheritance", e);
+    }
+    e = launch_tree_node(h->dev, d_nodes, n, depth, d_status, d_point, d_iters, inherit ? 1 : 0, h->sm_count, st);
+    if (e != cudaSuccess) return fail("K11 tree node LP", e);
+    return 0;
+}
+
+int ppgpu_tree_children(ppgpu_tree* h, const uint64_t* d_nodes, const uint8_t* d_status, int64_t n, int32_t depth,
+                        int64_t* d_idx, uint64_t* d_children, int64_t* d_parent_of, int64_t* h_count, void* d_ws,
+                        size_t ws_bytes, ppgpu_stream stream) {
+    if (!h || !h_count) return fail_msg("null argument");
+    *h_count = 0;
+    if (n < 0) return fail_msg("negative size");
+    if (depth < 0 || depth >= h->host.nb) return fail_msg("children need a depth in [0, nb)");
+    if (n == 0) return 0;
+    if (!d_nodes || !d_status || !d_idx || !d_children || !d_parent_of || !d_ws) return fail_msg("null argument");
+    if (ws_bytes < select_workspace_bytes(n)) return fail_msg("workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaSetDevice(h->device);
+    if (e != cudaSuccess) return fail("cudaSetDevice", e);
+    long long* d_count = (long long*)d_ws + (select_workspace_bytes(n) / sizeof(long long) - 1);
+    e = select_indices(d_status, n, 0xff, PPG_TREE_FEASIBLE, (long long*)d_idx, d_count, d_ws, ws_bytes - sizeof(long long), st);
+    if (e != cudaSuccess) return fail("K11 select", e);
+    e = launch_tree_children(d_nodes, (const long long*)d_idx, d_count, n, depth, d_children, (long long*)d_parent_of, st);
+    if (e != cudaSuccess) return fail("K11 children", e);
+    long long cnt = 0;
+    e = cudaMemcpyAsync(&cnt, d_count, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail("K11 children count", e);
+    *h_count = cnt;
+    return 0;
+}
+
 int ppgpu_measure_fp64_peak(int32_t iters, double* h_tflops, ppgpu_stream stream) {
     if (!h_tflops) return fail_msg("null argument");
     cudaError_t e = measure_fp64_peak(iters, h_tflops, (cudaStream_t)stream);

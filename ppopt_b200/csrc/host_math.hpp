@@ -488,4 +488,81 @@ inline bool reduce_program(int n, int t, int m, int q, int ne, int is_qp, const 
     return true;
 }
 
+// K11 (mixed-integer programs: which binary assignments have a feasible relaxation).  The LIFTED LP of a program
+//   variables  z = (x, theta)  (x in program order, the binaries y = x[bin] relaxed to [l, u]),
+//   rows       A x - F theta <= b (= b on the equality rows),  A_t theta <= b_t,  y_k <= u_k,  -y_k <= -l_k
+// is an LP whose right-hand side is affine in the 2 nb bound values: it is reduced exactly as an mpLP whose parameters are
+// p = (u_0 - 1, -l_0, u_1 - 1, -l_1, ...) (reduce_program: the equalities eliminated by QR, then build_lp_dictionary: the free
+// directions v exchanged against slacks with exchange_free_columns, the bound columns carried along as right-hand sides).
+// A tree node at depth d fixes y_k = v_k for k < d, i.e. p_{2k + v_k} = -1 and every other p = 0, so the right-hand side of
+// dictionary row r is  beta0_r + sum_{k<d} Dbnd[r][2k + v_k]  (d loads per row), and the entries never change.
+struct TreeProgram {
+    int n = 0, t = 0, m = 0, q = 0, ne = 0, nb = 0;
+    int nv = 0;     // n + t lifted variables
+    int rows = 0;   // inequality rows of the lifted system: (m - ne) + q + 2 nb; dictionary rows (v rows included)
+    int cols = 0;   // free directions v after the equalities: nv - ne
+    int rb0 = 0;    // first bound row (inequality numbering): rb0 + 2k is y_k <= u_k, rb0 + 2k + 1 is -y_k <= -l_k
+    int tp = 0;     // bound parameters: 2 nb (1 when nb = 0)
+    int ld = 0;     // row stride of D0: 1 + cols + tp
+    vec D0;         // rows x ld  [beta0 | D (cols) | Dbnd (tp)]: y_r = beta0_r - D_r s_N - Dbnd_r p
+    std::vector<int> bvar, nvar;   // row r holds slack bvar[r] >= 0 or v_c for bvar[r] = -1 - c; column c is slack nvar[c]
+    vec hs;         // per inequality row: 1 + |h_i| at the root bounds (u = 1, l = 0), the scale of its tolerance
+    vec z0, Q2;     // z = z0 + Q2 v  (nv, nv x cols; the equality rows carry no bound parameter, so z0 is node independent)
+    vec Arows, brows;  // the lifted rows, equalities first ((ne + rows) x nv) and their right-hand sides at the root bounds
+    std::vector<int> bin;
+    std::string error;
+};
+
+// Builds the lifted system of a program whose equality rows are rows 0..ne-1 of A / b / F.  Returns false (error set) on
+// malformed input, rank-deficient equalities, or a lifted system without a vertex (rows of rank below the free variables).
+inline bool build_tree_dictionary(int n, int t, int m, int q, int ne, int nb, const int* bin, const double* A,
+                                  const double* b, const double* F, const double* A_t, const double* b_t, TreeProgram& T) {
+    T.n = n; T.t = t; T.m = m; T.q = q; T.ne = ne; T.nb = nb;
+    if (n < 1 || t < 0 || m < 0 || q < 0 || ne < 0 || ne > m || nb < 0 || nb > 63) { T.error = "bad dimensions"; return false; }
+    T.bin.assign(bin, bin + nb);
+    for (int k = 0; k < nb; ++k) {
+        if (bin[k] < 0 || bin[k] >= n) { T.error = "binary index out of range"; return false; }
+        for (int j = 0; j < k; ++j) if (bin[j] == bin[k]) { T.error = "repeated binary index"; return false; }
+    }
+    const int nv = n + t, tp = nb > 0 ? 2 * nb : 1, mL = m + q + 2 * nb;
+    T.nv = nv; T.tp = tp;
+    if (ne > nv) { T.error = "more equality rows than variables"; return false; }
+    vec AL((size_t)mL * nv, 0.0), bL(mL, 0.0), FL((size_t)mL * tp, 0.0);
+    for (int i = 0; i < m; ++i) {
+        for (int j = 0; j < n; ++j) AL[(size_t)i * nv + j] = A[(size_t)i * n + j];
+        for (int j = 0; j < t; ++j) AL[(size_t)i * nv + n + j] = -F[(size_t)i * t + j];
+        bL[i] = b[i];
+    }
+    for (int i = 0; i < q; ++i) {
+        for (int j = 0; j < t; ++j) AL[(size_t)(m + i) * nv + n + j] = A_t[(size_t)i * t + j];
+        bL[m + i] = b_t[i];
+    }
+    for (int k = 0; k < nb; ++k) {
+        const int ru = m + q + 2 * k, rl = ru + 1;
+        AL[(size_t)ru * nv + bin[k]] = 1.0;  bL[ru] = 1.0; FL[(size_t)ru * tp + 2 * k] = 1.0;       // y_k <= 1 + p_2k
+        AL[(size_t)rl * nv + bin[k]] = -1.0; bL[rl] = 0.0; FL[(size_t)rl * tp + 2 * k + 1] = 1.0;   // -y_k <= 0 + p_2k+1
+    }
+    vec c(nv, 0.0), H((size_t)nv * tp, 0.0);
+    ReducedProgram R;
+    if (!reduce_program(nv, tp, mL, 0, ne, 0, AL.data(), bL.data(), FL.data(), nullptr, nullptr, nullptr, c.data(), H.data(), R)) {
+        T.error = R.error;
+        return false;
+    }
+    if (!R.lp_ok) {
+        T.error = "the lifted rows (program rows, Theta rows and binary bounds) have rank below the " + std::to_string(R.np) +
+                  " free variables left by the equalities: the relaxation has no vertex (a continuous variable or parameter is "
+                  "unbounded in some direction)";
+        return false;
+    }
+    T.rows = R.mi; T.cols = R.np; T.rb0 = m - ne + q; T.ld = R.lp_ld;
+    T.D0 = R.lp_D0; T.bvar = R.lp_bvar; T.nvar = R.lp_nvar;
+    T.hs.resize(T.rows);
+    for (int i = 0; i < T.rows; ++i) T.hs[i] = 1.0 + std::fabs(bL[ne + i]);
+    T.z0.resize(nv);
+    for (int i = 0; i < nv; ++i) T.z0[i] = R.X0t[(size_t)i * (tp + 1)];
+    T.Q2 = R.Q2;
+    T.Arows = AL; T.brows = bL;
+    return true;
+}
+
 }  // namespace ppgpu

@@ -102,6 +102,31 @@ cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long 
 // iters (n x 2: pivots, Phase 1 pivots), x / dual / mask / iters may be null
 cudaError_t launch_theta_lp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
                             double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);
+// K11: the relaxation tree of a mixed-integer program (csrc/k11_mitree.cu, lifted system of host_math.hpp::TreeProgram).
+// Nodes are uint64 with bit k = y_k for k < depth.
+struct DevTree {
+    int nv, rows, cols, rb0, tp, ld, ne, nb;
+    const double* D0;      // rows x ld  [beta0 | D | Dbnd]
+    const int* bvar;       // rows
+    const int* nvar;       // cols
+    const double* hs;      // rows
+    const double* z0;      // nv
+    const double* Q2;      // nv x cols
+    const double* Arows;   // (ne + rows) x nv
+    const double* brows;   // ne + rows
+    const int* bin;        // nb
+};
+// status (PPG_TREE_*), point (n x nv, NaN unless feasible) and iters (pivots) may be null except status; skip_done: nodes
+// whose status is already PPG_TREE_FEASIBLE (certified by inheritance) are left as they are
+cudaError_t launch_tree_node(const DevTree& P, const uint64_t* nodes, long long n, int depth, uint8_t* status, double* point,
+                             int* iters, int skip_done, int sm_count, cudaStream_t st);
+// one thread per node at `depth` >= 1: the parent's point with y_{depth-1} snapped to the node's value; certified ->
+// status PPG_TREE_FEASIBLE, the snapped point and iters = -1; otherwise status PPG_TREE_UNDECIDED
+cudaError_t launch_tree_inherit(const DevTree& P, const uint64_t* nodes, long long n, int depth, const double* parent_point,
+                                const long long* parent_of, uint8_t* status, double* point, int* iters, cudaStream_t st);
+// children of the selected nodes idx[0..*d_count) (n_max bounds the count): 2j fixes y_depth = 0, 2j + 1 fixes it to 1
+cudaError_t launch_tree_children(const uint64_t* nodes, const long long* idx, const long long* d_count, long long n_max, int depth,
+                                 uint64_t* children, long long* parent_of, cudaStream_t st);
 cudaError_t launch_clear_bits(uint8_t* status, long long n, uint8_t bits, cudaStream_t st);
 
 cudaError_t measure_fp64_peak(int iters, double* tflops, cudaStream_t st);

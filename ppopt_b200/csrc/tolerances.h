@@ -107,3 +107,16 @@
 #define PPG_TLP_ITERLIM 2
 #define PPG_TLP_NUMERIC 3
 #define PPG_TLP_UNBOUNDED 4
+
+// K11 relaxation tree of an mpMIQP / mpMILP (Phase 1 of the lifted LP per node, csrc/k11_mitree.cu).  A node is feasible iff
+// its relaxation has a point z with  a_i z - h_i <= PPG_FEAS_TOL (1 + |h_i|)  on every row (|.| on the equality rows), h_i the
+// row's right-hand side at the node's bounds.  Phase 1 splits that budget: the Harris relaxation of a slack row is half of it
+// and x0 (Chvatal's auxiliary column) must end at or below PPG_TREE_AUX = half of PPG_FEAS_TOL, so the point read off a
+// feasible node's final dictionary violates row i by at most PPG_FEAS_TOL (1 + |h_i|).  An inherited point is certified
+// against the full PPG_FEAS_TOL (1 + |h_i|) of every row.  Pivoting rules and the other thresholds are K9's (PPG_TLP_*).
+#define PPG_TREE_HARRIS 0.5e-7
+#define PPG_TREE_AUX 0.5e-7
+// status per node: 0-3 mean what PPG_TLP_* means (feasible / infeasible / iteration cap / numerical breakdown)
+#define PPG_TREE_FEASIBLE 0
+#define PPG_TREE_INFEASIBLE 1
+#define PPG_TREE_UNDECIDED 255   // transient: the inheritance check did not certify the node, the LP decides it

@@ -4,10 +4,14 @@ combination, merged into one overlapping Solution.
 
 What runs where
   * the binary tree (``MITree`` / ``check_bin_feasibility``, mitree.py, mpmilp_program.py:206-246) needs a MILP solver
-    (the reference only has a Gurobi binding, solver.py:278-281) and stays on the host: pass ``feasible_combinations`` (what
-    the reference's tree returns), or let this module enumerate all 2^nb combinations and keep the ones whose substituted
-    problem is feasible - for a LEAF of the tree the MILP feasibility question is an LP (every binary is fixed), and that LP
-    is the base-set feasibility test of the engine (K2 on the empty active set);
+    (the reference only has a Gurobi binding, solver.py:278-281).  Here the feasible combinations come from one of
+      - ``feasible_combinations`` passed by the caller (what the reference's tree returns), which wins over ``screen``;
+      - ``screen='tree'``: the relaxation tree on the GPU (K11, mitree.py): breadth first, one batch per depth, an inner
+        node answers the LP relaxation of its partial assignment, a leaf the LP the MILP reduces to;
+      - ``screen='enumerate'``: all 2^nb combinations on the host, keeping the ones whose substituted problem is feasible -
+        for a LEAF the MILP feasibility question is an LP (every binary is fixed), and that LP is the base-set feasibility
+        test of the engine (K2 on the empty active set); at most 20 binaries;
+      - ``screen='auto'`` (default): 'enumerate' up to 20 binaries, 'tree' beyond;
   * the sub-problems are built by the program's own ``generate_substituted_problem`` (mpmilp_program.py:150-195,
     mpmiqp_program.py:71-116: numpy + the constructor's presolve);
   * every sub-problem is solved by the GPU engine.  A sub-problem is small (the binaries are gone), so one solve cannot fill
@@ -24,6 +28,7 @@ import numpy
 import torch
 
 from .. import engine as _engine
+from . import mitree
 from .._lib import ST_FEAS
 from .solve_mpqp import mpqp_algorithm, solve_mpqp
 
@@ -54,15 +59,29 @@ def leaf_is_feasible(sub_problem) -> bool:
 
 
 def solve_mpmiqp_enumeration(program, num_cores: int = -1, cont_algorithm: mpqp_algorithm = mpqp_algorithm.combinatorial,
-                             feasible_combinations: Optional[Iterable[List[int]]] = None, streams: int = 4):
+                             feasible_combinations: Optional[Iterable[List[int]]] = None, streams: int = 4,
+                             screen: str = 'auto'):
     """Same arguments and result as the reference's solve_mpmiqp_enumeration (``num_cores`` is accepted for signature
     parity; the GPU replaces the process pool).  ``feasible_combinations``: the leaves of the reference's MITree, when the
-    caller has them; otherwise all 2^nb assignments are screened on the GPU.  ``streams``: sub-problems in flight."""
+    caller has them; otherwise ``screen`` selects how they are found: 'tree' (the relaxation tree on the GPU), 'enumerate'
+    (all 2^nb assignments, at most 20 binaries) or 'auto' ('enumerate' up to 20 binaries, 'tree' beyond).
+    ``streams``: sub-problems in flight."""
+    if screen not in ('auto', 'tree', 'enumerate'):
+        raise ValueError(f"screen must be 'auto', 'tree' or 'enumerate', not {screen!r}")
     nb = len(program.binary_indices)
     subs = {}
-    if feasible_combinations is None:
+    if feasible_combinations is None and (screen == 'tree' or (screen == 'auto' and nb > 20)):
+        combos = []
+        for y in mitree.feasible_combinations(program).leaves:
+            try:
+                sub = program.generate_substituted_problem(list(y))
+            except Exception:   # the constructor's presolve found the substituted constraint set infeasible (tolerance band)
+                continue
+            combos.append(list(y))
+            subs[tuple(y)] = sub
+    elif feasible_combinations is None:
         if nb > 20:
-            raise ValueError('more than 20 binaries: pass feasible_combinations (the reference enumerates them with MITree)')
+            raise ValueError("more than 20 binaries: use screen='tree' or pass feasible_combinations")
         combos = []
         for y in itertools.product((0, 1), repeat=nb):
             if not binary_rows_hold(program, y):
