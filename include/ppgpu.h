@@ -48,7 +48,7 @@ typedef struct {
 } ppgpu_info;
 
 /* number of uint64 counters returned by ppgpu_counters */
-#define PPGPU_NUM_COUNTERS 24
+#define PPGPU_NUM_COUNTERS 26
 
 const char* ppgpu_last_error(void);
 int ppgpu_version(void);
@@ -67,6 +67,9 @@ int ppgpu_program_info(const ppgpu_program* prog, ppgpu_info* out);
  *                      produced by the vertex walk (csrc/k2w_walk.cu) before the relaxation (default 100000; 0: always;
  *                      negative: never).  Decisions do not depend on it - only which kernel exhibits the feasible point. */
 #define PPGPU_OPT_K2W_MIN 0
+/*   PPGPU_OPT_K2W_REF  1: the vertex walk applies every pivot to its whole dictionary (the reference of the deferred
+ *                      updates it uses by default where the dictionary's shape allows; results are identical); 0: default */
+#define PPGPU_OPT_K2W_REF 1
 int ppgpu_set_option(ppgpu_program* prog, int32_t option, int64_t value);
 
 /* Level-1 candidates = generate_children_sets(equality_indices, m, murder_list) (solver_utils.py:154-166) plus the mpLP

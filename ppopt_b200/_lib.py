@@ -6,16 +6,18 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'libppgpu.so')
 
-NUM_COUNTERS = 24
+NUM_COUNTERS = 26
 NUM_FAMILIES = 10
 FAMILY_NAMES = ('k1_rank', 'k2_feas_lp', 'k34_kkt_cheb', 'k5_emit', 'k6_count', 'k6_write', 'select', 'k2a_relax', 'k2w_walk', 'inherit')
 COUNTER_NAMES = ('k1_candidates', 'k2_lps', 'k2_pivots', 'k2_work', 'k4_lps', 'k4_pivots', 'k4_work', 'k5_lps',
                  'k5_pivots', 'k5_work', 'numeric', 'border', 'k6_lookups', 'k2a_tried', 'k2a_certified', 'k2a_steps', 'k2a_work',
-                 'k2w_certified', 'k2w_pivots', 'k2w_work', 'k2w_giveup', 'inherited', 'inherit_lookups')
+                 'k2w_certified', 'k2w_pivots', 'k2w_work', 'k2w_giveup', 'inherited', 'inherit_lookups',
+                 'k2w_drop_reset', 'k2w_drop_giveup')
 
 # status bits (csrc/tolerances.h)
 ST_RANK, ST_FEAS, ST_OPT, ST_REGION, ST_BORDER, ST_NUMERIC, ST_THIN = 1, 2, 4, 8, 16, 32, 64
 OPT_K2W_MIN = 0   # ppgpu_set_option (include/ppgpu.h)
+OPT_K2W_REF = 1
 TREE_OPT_INHERIT = 0   # ppgpu_tree_set_option
 WITNESS_SLOTS = 2  # PPGPU_WITNESS_SLOTS
 

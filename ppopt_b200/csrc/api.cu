@@ -38,6 +38,7 @@ struct ppgpu_program {
     int* d_k2w_order = nullptr;   // scratch for the cost order of the walk's work items (grown on demand)
     size_t k2w_order_cap = 0;
     long long k2w_min = 100000;   // smallest launch the vertex walk (K2w) is used for (ppgpu_set_option)
+    bool k2w_ref = false;         // K2w with the reference dictionary updates (PPGPU_OPT_K2W_REF)
     double prof_ms[PPGPU_NUM_FAMILIES] = {0};
     long long prof_launches[PPGPU_NUM_FAMILIES] = {0};
 };
@@ -174,6 +175,7 @@ int ppgpu_set_option(ppgpu_program* p, int32_t option, int64_t value) {
     if (!p) return fail_msg("null argument");
     switch (option) {
         case PPGPU_OPT_K2W_MIN: p->k2w_min = value; return 0;
+        case PPGPU_OPT_K2W_REF: p->k2w_ref = value != 0; return 0;
         default: return fail_msg("unknown option");
     }
 }
@@ -314,7 +316,8 @@ static int level_eval_chunk(ppgpu_program* p, const uint64_t* d_masks, int64_t n
             if ((e = cudaMalloc((void**)&p->d_k2w_order, want * sizeof(int))) != cudaSuccess) return fail("K2w order scratch", e);
             p->k2w_order_cap = want;
         }
-        e = launch_k2w(p->dev, d_masks, n, k_act, d_status, next_queue(p, st), p->d_counters, p->sm_count, st, &handled, wio.out, p->d_k2w_order);
+        e = launch_k2w(p->dev, d_masks, n, k_act, d_status, next_queue(p, st), p->d_counters, p->sm_count, st, &handled, wio.out, p->d_k2w_order,
+                       p->k2w_ref);
         if (e != cudaSuccess) return fail("K2w vertex walk", e);
         if (handled) p->launches += (n > 128ll * 8 * p->sm_count) ? 4 : 1;   // + the three kernels that order the work items
     }

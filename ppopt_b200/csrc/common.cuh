@@ -60,7 +60,9 @@ enum Counter {
     CNT_K2W_CERTIFIED, CNT_K2W_PIVOTS, CNT_K2W_WORK,  // 17, 18, 19: vertex walk (pivots x basic rows x columns FMAs)
     CNT_K2W_GIVEUP,                                   // 20: drives abandoned (iteration cap, empty face, dependent row)
     CNT_INHERITED, CNT_INHERIT_LOOKUPS,               // 21, 22: certificates inherited from parent witnesses / parents looked up
-    CNT_COUNT = 24
+    CNT_K2W_DROP_RESET, CNT_K2W_DROP_GIVEUP,          // 23, 24: K2w reloads (K2W_RESET / vertex out of the band) that discarded
+                                                      //         deferred pivots (K2wDeferDict)
+    CNT_COUNT = 26
 };
 
 __device__ __forceinline__ bool mask_test(const uint64_t* m, int i) { return (m[i >> 6] >> (i & 63)) & 1ull; }

@@ -37,10 +37,14 @@ constexpr int K2W_DRIVE_CAP = 400;  // pivots per drive before giving up
 constexpr int K2W_RESET = 3000;     // pivots after which the dictionary is reloaded (bounds the accumulated rounding)
 constexpr double K2W_PIV_MIN = 1e-7;   // smallest entering coefficient worth pivoting on
 constexpr double K2W_NEG_OK = 1e-8;    // a vertex certifies only while every basic slack is >= -K2W_NEG_OK
+// pivots K2wDeferDict keeps pending before it updates the whole dictionary (measured on the bench step, K2w 130.6 ms with
+// every pivot applied to the whole dictionary: 117.3 at K = 2, 123.6 at 3, 138.2 at 4 - a longer pending chain on the
+// entries a pivot reads costs more latency than the flushes it saves)
+constexpr int K2W_DEFER = 2;
 
 struct K2wCtx {
     double* D;        // nb x lds   [beta | coefficients], lds odd: rows over lanes are bank-conflict free
-    double* prow;     // lds        scaled pivot row
+    double* prow;     // PROWS x lds scaled pivot row(s) of the storage policy
     int* bvar;        // nb         row id basic in dictionary row i
     int* nvar;        // nf         row id nonbasic in column j
     int* where;       // R0         >= 0: dictionary row, < 0: ~column
@@ -120,6 +124,7 @@ struct K2wSmemDict {
     static constexpr int RPL = RPL_;
     static constexpr bool IN_SMEM = true;
     static constexpr int SMEM_ROW0 = 0;
+    static constexpr int PROWS = 1;   // scaled pivot rows in shared memory (c.prow)
     __device__ __forceinline__ void reload(const DevProgram& P, const K2wCtx& c, int lane) {
         for (int e = lane; e < c.nb * c.ld; e += 32) {
             const int r = e / c.ld, k = e - r * c.ld;
@@ -243,6 +248,204 @@ struct K2wSmemDict {
     }
 };
 
+// ---- storage policy D: the dictionary in SHARED memory with DEFERRED updates - policy A's arithmetic, bit for bit, but
+// the rank-1 updates reach the bulk of D only once every K pivots.  Per pending step m the walker keeps the scaled pivot
+// row p_m (c.prow + m * LD: policy A's prow, 0 in the entering column cj_m) and, in registers, u_m[r] = policy A's colr
+// (the entering-column entry of row r, 0 for the pivot row and rows >= nb).  The current value of entry (i, k) is
+//         D[i][k], then x = fma(-u_m[i], p_m[k], x) for every pending m in order
+// - the FMAs policy A performs, in the same order.  The two overwrites of a Gauss-Jordan step are stored at once and
+// cancel the pending steps on what they overwrite: the new pivot row goes straight into D and its owner zeroes u_m'[l],
+// the exchanged column -u_m[r] / pivot goes into D for every other row and p_m'[cj] = 0 (m' < m).  Only signs of zeros
+// can differ from policy A, which no comparison observes.  The right-hand side (column 0) lives in registers and is
+// updated at every pivot like policy A's column 0, so the certification band is still checked after every pivot;
+// column 0 of D is only read by reload.  Per pivot (76 x 37) this reads / writes ~3.2 k dictionary entries at K = 2
+// (~1.8 k at K = 4) instead of ~5.6 k: the target row, the entering column and the pivot row through the pending chain,
+// plus 1 / K of a flush.
+template <int RPL_, int LD, int K>
+struct K2wDeferDict {
+    static constexpr int RPL = RPL_;
+    static constexpr bool IN_SMEM = true;
+    static constexpr int SMEM_ROW0 = 0;
+    static constexpr int PROWS = K;
+    double u[K][RPL];   // u_m of my rows (lane + 32 rr)
+    double beta[RPL];   // right-hand side of my rows, always current
+    int np;             // pending steps (uniform); np == pivots since reload mod K
+    // current values the next pivot may reuse: row trow_i at columns 1 + lane + 32 h (target_scan), the entering column
+    // 1 + ccol_j of my rows (column)
+    static constexpr int TH = (LD - 1 + 31) / 32;
+    double trow[TH], ccol[RPL];
+    int trow_i, ccol_j;
+    // value of basic row `slot * 32 + owner`, uniform over the warp
+    template <int N>
+    __device__ __forceinline__ double from_row(const double (&v)[N], int slot, int owner) const {
+        double x = 0.0;
+#pragma unroll
+        for (int rr = 0; rr < N; ++rr) if (rr == slot) x = v[rr];
+        return shfl_d(x, owner);
+    }
+    // u_m of basic row l (uniform), m < np
+    __device__ __forceinline__ void row_u(int l, double (&ul)[K]) const {
+#pragma unroll
+        for (int m = 0; m < K; ++m) ul[m] = m < np ? from_row(u[m], l >> 5, l & 31) : 0.0;
+    }
+    // current value of an entry from its stored value: the pending chain with row factors um, column k of the p_m
+    __device__ __forceinline__ double chain(const K2wCtx& c, double x, const double (&um)[K], int k) const {
+#pragma unroll
+        for (int m = 0; m < K; ++m)
+            if (m < np) x = fma(-um[m], c.prow[m * LD + k], x);
+        return x;
+    }
+    __device__ __forceinline__ void reload(const DevProgram& P, const K2wCtx& c, int lane) {
+        for (int e = lane; e < c.nb * LD; e += 32) c.D[e] = __ldg(P.wk_D0 + e);
+#pragma unroll
+        for (int rr = 0; rr < RPL; ++rr) {
+            const int r = lane + 32 * rr;
+            beta[rr] = r < c.nb ? __ldg(P.wk_D0 + (size_t)r * LD) : 0.0;
+        }
+        np = 0;   // whatever was pending is discarded with the old dictionary
+        trow_i = -1; ccol_j = -1;
+        k2w_reload_labels(P, c, lane);
+    }
+    __device__ __forceinline__ void target_scan(const K2wCtx& c, int wi, uint64_t fm, int lane, double& bi, double& wbest, int& j) {
+        double uw[K];
+        row_u(wi, uw);
+        bi = from_row(beta, wi >> 5, wi & 31);
+        const double* Di = c.D + (size_t)wi * LD;
+        const bool degen = bi <= 1e-11;
+        double best = 0.0; int bj = 0x7fffffff;
+#pragma unroll
+        for (int h = 0; h < TH; ++h) {
+            const int jj = lane + 32 * h;
+            if (1 + jj >= LD) continue;
+            trow[h] = chain(c, Di[1 + jj], uw, 1 + jj);
+            if (jj >= c.nf || ((fm >> jj) & 1ull)) continue;
+            const double x = degen ? fabs(trow[h]) : trow[h];
+            if (x > best) { best = x; bj = jj; }
+        }
+        trow_i = wi;
+        wbest = warp_max_nonneg(best);
+        j = __reduce_min_sync(PPG_FULL, best == wbest ? bj : 0x7fffffff);
+    }
+    // entering column of my rows (lanes over rows, broadcast loads of p_m[cj])
+    __device__ __forceinline__ void cur_column(const K2wCtx& c, int cj, int lane, double (&col)[RPL]) const {
+#pragma unroll
+        for (int rr = 0; rr < RPL; ++rr) {
+            const int r = lane + 32 * rr;
+            double um[K];
+#pragma unroll
+            for (int m = 0; m < K; ++m) um[m] = u[m][rr];
+            col[rr] = r < c.nb ? chain(c, c.D[(size_t)r * LD + cj], um, cj) : 0.0;
+        }
+    }
+    __device__ __forceinline__ void column(const K2wCtx& c, int j, int lane, double (&col)[RPL], double (&beta_out)[RPL]) {
+        cur_column(c, 1 + j, lane, col);
+#pragma unroll
+        for (int rr = 0; rr < RPL; ++rr) { ccol[rr] = col[rr]; beta_out[rr] = beta[rr]; }
+        ccol_j = j;
+    }
+    __device__ __forceinline__ bool pivot(const K2wCtx& c, int l, int j, int lane) {
+        const int cj = 1 + j, nb = c.nb, slot = l >> 5, owner = l & 31;
+        double col[RPL];
+        if (ccol_j == j) {
+#pragma unroll
+            for (int rr = 0; rr < RPL; ++rr) col[rr] = ccol[rr];
+        } else {
+            cur_column(c, cj, lane, col);
+        }
+        const double inv = k2w_rcp(from_row(col, slot, owner));
+        double ul[K];
+        row_u(l, ul);
+        const double q0 = from_row(beta, slot, owner) * inv;
+        __syncwarp();
+        // the pivot row: p_np = current row l x inv (0 in the entering column), and the new row l stored in D
+        double* Dl = c.D + (size_t)l * LD;
+        double* pn = c.prow + np * LD;
+        if (lane == 0) pn[0] = q0;
+#pragma unroll
+        for (int h = 0; h < TH; ++h) {
+            const int k = 1 + lane + 32 * h;
+            if (k >= LD) continue;
+            const double x = trow_i == l ? trow[h] : chain(c, Dl[k], ul, k);
+            const double q = (k == cj) ? 0.0 : x * inv;
+            pn[k] = q;
+            Dl[k] = (k == cj) ? inv : q;
+        }
+        trow_i = -1; ccol_j = -1;
+        bool ok = true;
+#pragma unroll
+        for (int rr = 0; rr < RPL; ++rr) {
+            const int r = lane + 32 * rr;
+            if (r == l) {
+                // the new row l carries none of the earlier pending steps
+#pragma unroll
+                for (int m = 0; m < K; ++m) if (m < np) u[m][rr] = 0.0;
+            }
+            const double ur = (r < nb && r != l) ? col[rr] : 0.0;
+#pragma unroll
+            for (int m = 0; m < K; ++m) if (m == np) u[m][rr] = ur;
+            // right-hand side: policy A's column 0, checked on the value just computed
+            const double x = fma(-ur, q0, beta[rr]);
+            beta[rr] = r == l ? q0 : x;
+            ok = ok && (r >= nb || r == l || x >= -K2W_NEG_OK);
+            // the exchanged column, stored for every other row (zeros included: the earlier steps are cancelled on it)
+            if (r < nb && r != l) c.D[(size_t)r * LD + cj] = -ur * inv;
+        }
+        __syncwarp();
+        if (lane < np) c.prow[lane * LD + cj] = 0.0;
+        if (lane == 0) k2w_swap_labels(c, l, j);
+        if (++np == K) {
+            __syncwarp();
+            flush(c, lane);
+        }
+        ok = __all_sync(PPG_FULL, ok);
+        __syncwarp();
+        return ok;
+    }
+    // the K pending steps applied to columns 1.. of every row: one load, K FMAs and one store per entry, in groups of G
+    // columns whose loads are all issued before their first FMA (as policy A's update).  A row whose pending u are all zero
+    // is not stored (policy A skips the store of a row whose column entry is zero).
+    __device__ __forceinline__ void flush(const K2wCtx& c, int lane) {
+        constexpr int G = 6;
+        double* Dr[RPL];
+        bool st[RPL];
+#pragma unroll
+        for (int rr = 0; rr < RPL; ++rr) {
+            const int r = lane + 32 * rr;
+            Dr[rr] = c.D + (size_t)(r < c.nb ? r : 0) * LD;
+            st[rr] = false;
+#pragma unroll
+            for (int m = 0; m < K; ++m) st[rr] = st[rr] || u[m][rr] != 0.0;
+        }
+        const double* __restrict__ p = c.prow;
+        static_for<(LD - 1 + G - 1) / G>([&](auto KK) {
+            constexpr int k0 = 1 + decltype(KK)::value * G;
+            constexpr int GN = (LD - k0) < G ? (LD - k0) : G;
+            double x[RPL][GN];
+#pragma unroll
+            for (int rr = 0; rr < RPL; ++rr)
+#pragma unroll
+                for (int g = 0; g < GN; ++g) x[rr][g] = Dr[rr][k0 + g];
+#pragma unroll
+            for (int m = 0; m < K; ++m) {
+                double pk[GN];
+#pragma unroll
+                for (int g = 0; g < GN; ++g) pk[g] = p[m * LD + k0 + g];
+#pragma unroll
+                for (int rr = 0; rr < RPL; ++rr)
+#pragma unroll
+                    for (int g = 0; g < GN; ++g) x[rr][g] = fma(-u[m][rr], pk[g], x[rr][g]);
+            }
+#pragma unroll
+            for (int rr = 0; rr < RPL; ++rr)
+                if (st[rr]) {
+#pragma unroll
+                    for (int g = 0; g < GN; ++g) Dr[rr][k0 + g] = x[rr][g];
+                }
+        });
+        np = 0;
+    }
+};
+
 // ---- storage policy C: HYBRID - the first 32 basic rows (row slot 0: one row per lane) in REGISTERS, the other slots in
 // shared memory.  The walk is bound by shared-memory bandwidth (a pivot reads and writes every dictionary entry: ncu 69 %
 // of the wavefront peak with everything in shared memory); one slot in registers removes 4 of the 11 wavefronts per column
@@ -254,6 +457,7 @@ struct K2wHybridDict {
     static constexpr int RPL = RPL_;
     static constexpr bool IN_SMEM = true;
     static constexpr int SMEM_ROW0 = 32;   // shared memory holds rows 32.. (row r at (r - 32) * LD)
+    static constexpr int PROWS = 1;
     double T0[LD];                          // row `lane` of the dictionary
     __device__ __forceinline__ void reload(const DevProgram& P, const K2wCtx& c, int lane) {
 #pragma unroll
@@ -394,6 +598,7 @@ struct K2wRegDict {
     static constexpr int RPL = RPL_;
     static constexpr bool IN_SMEM = false;
     static constexpr int SMEM_ROW0 = 0;
+    static constexpr int PROWS = 1;
     double T[RPL][DC];
     __device__ __forceinline__ void reload(const DevProgram& P, const K2wCtx& c, int lane) {
         static_for<RPL>([&](auto RR) {
@@ -641,7 +846,7 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
     {
         unsigned char* base = k2w_smem + (size_t)warp * walker_bytes;
         c.D = reinterpret_cast<double*>(base); base += k2w_dict_smem_bytes<Dict>(c.nb, lds);
-        c.prow = reinterpret_cast<double*>(base); base += (size_t)lds * 8;
+        c.prow = reinterpret_cast<double*>(base); base += (size_t)Dict::PROWS * lds * 8;
         c.orig = reinterpret_cast<uint64_t*>(base); base += (size_t)c.R0 * W4 * 8;
         c.todo = reinterpret_cast<uint64_t*>(base); base += (size_t)c.R0 * W4 * 8;
         c.nbm = reinterpret_cast<uint64_t*>(base); base += (size_t)W4 * 8;
@@ -653,7 +858,7 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
     }
     const int W = P.W, R0 = P.R0, nb = c.nb, nf = c.nf;
     const int p = k_act >= 2 ? k_act - 2 : 0;
-    unsigned long long n_piv = 0, n_give = 0;
+    unsigned long long n_piv = 0, n_give = 0, n_drop_reset = 0, n_drop_give = 0;
     int n_cert = 0;
     // prefix words / last two rows of candidate q
     auto split = [&](long long q, uint64_t (&pf)[4], int& a, int& b) {
@@ -758,6 +963,8 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
             bool restart = (npiv > K2W_RESET) || !vertex_ok;
             for (;;) {
                 if (restart) {
+                    // (a deferring policy holds npiv mod PROWS pivots that never reached the bulk of its dictionary)
+                    if (npiv % Dict::PROWS) ++(vertex_ok ? n_drop_reset : n_drop_give);
                     dict.reload(P, c, lane);
                     n_piv += npiv; npiv = 0; nfixed = 0; vertex_ok = true; restart = false;
                     stage = 0; f = 0; a = -1;
@@ -893,6 +1100,8 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
         atomicAdd(&counters[CNT_K2W_PIVOTS], n_piv);
         atomicAdd(&counters[CNT_K2W_WORK], n_piv * (unsigned long long)(c.nb * c.ld));
         atomicAdd(&counters[CNT_K2W_GIVEUP], n_give);
+        if (n_drop_reset) atomicAdd(&counters[CNT_K2W_DROP_RESET], n_drop_reset);
+        if (n_drop_give) atomicAdd(&counters[CNT_K2W_DROP_GIVEUP], n_drop_give);
     }
 }
 
@@ -960,7 +1169,7 @@ static cudaError_t launch_k2w_t(const DevProgram& P, const uint64_t* masks, long
                                 unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st,
                                 bool* handled, uint64_t* witness, int* order_scratch) {
     const int nb = P.wk_nb, ld = P.wk_ld, lds = ld | 1, W4 = (P.R0 + 63) / 64;
-    size_t wb = k2w_dict_smem_bytes<Dict>(nb, lds) + (size_t)lds * 8 + (size_t)2 * P.R0 * W4 * 8 + (size_t)W4 * 8 +
+    size_t wb = k2w_dict_smem_bytes<Dict>(nb, lds) + (size_t)Dict::PROWS * lds * 8 + (size_t)2 * P.R0 * W4 * 8 + (size_t)W4 * 8 +
                 (size_t)(nb + P.nfree + 2 * P.R0 + K2W_MAXFIX + 2) * 4;
     wb = (wb + 15) & ~(size_t)15;
     auto kern = k2w_walk_kernel<Dict>;
@@ -1009,7 +1218,7 @@ static cudaError_t launch_k2w_t(const DevProgram& P, const uint64_t* masks, long
 // *handled == false: the walk is off for this program / level (no vertex dictionary, prefix too long, dictionary too large)
 cudaError_t launch_k2w(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,
                        unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st, bool* handled,
-                       uint64_t* witness, int* order_scratch) {
+                       uint64_t* witness, int* order_scratch, bool reference) {
     *handled = false;
     static const int on = getenv("PPGPU_K2W") ? atoi(getenv("PPGPU_K2W")) : 1;
     static const int regs_on = getenv("PPGPU_K2W_REG") ? atoi(getenv("PPGPU_K2W_REG")) : 0;
@@ -1026,7 +1235,10 @@ cudaError_t launch_k2w(const DevProgram& P, const uint64_t* masks, long long n, 
     // pivot row's owner, a serial scan of the target row): an EXPERIMENT, off by default like policy B)
     static const int hybrid_on = getenv("PPGPU_K2W_HYBRID") ? atoi(getenv("PPGPU_K2W_HYBRID")) : 0;
     if (hybrid_on && rpl == 3 && P.wk_ld == 37) K2W_GO(K2wHybridDict<3 K2W_COMMA 37>);   // the bench shape: row slot 0 in registers
-    if (rpl == 3 && P.wk_ld == 37) K2W_GO(K2wSmemDict<3 K2W_COMMA 37>);   // ... everything in shared memory, columns known at compile time
+    // ... everything in shared memory, columns known at compile time: updates deferred over K2W_DEFER pivots, or (the
+    // reference, PPGPU_OPT_K2W_REF) every pivot applied to the whole dictionary
+    if (rpl == 3 && P.wk_ld == 37 && reference) K2W_GO(K2wSmemDict<3 K2W_COMMA 37>);
+    if (rpl == 3 && P.wk_ld == 37) K2W_GO(K2wDeferDict<3 K2W_COMMA 37 K2W_COMMA K2W_DEFER>);
     switch (rpl) {
         case 1: K2W_GO(K2wSmemDict<1>);
         case 2: K2W_GO(K2wSmemDict<2>);

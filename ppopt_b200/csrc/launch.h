@@ -47,7 +47,7 @@ cudaError_t launch_k2a_prefix(const DevProgram& P, const uint64_t* masks, long l
 // witness (n x W, may be null): receives the active-row mask of the vertex that certified a candidate
 cudaError_t launch_k2w(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,
                        unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st, bool* handled,
-                       uint64_t* witness, int* order_scratch);
+                       uint64_t* witness, int* order_scratch, bool reference);
 // ints of scratch launch_k2w wants for ordering the work items of an n-candidate launch (may be passed as null: natural order)
 size_t k2w_order_scratch_ints(long long n);
 // certificates INHERITED from the previous level: a candidate is feasible when the witness vertex of one of its parents
