@@ -67,13 +67,13 @@ static int fail(const char* where, cudaError_t e) {
 static int fail_msg(const std::string& m) { g_err = m; return -2; }
 
 template <class T>
-static cudaError_t upload(ppgpu_program* p, const std::vector<T>& v, const T** out) {
+static cudaError_t upload(std::vector<void*>& allocs, const std::vector<T>& v, const T** out) {
     void* d = nullptr;
     // 1 KiB zero tail: K2a reads 32-wide row segments of Gam without clamping the last one (k2a_relax.cu)
     const size_t bytes = v.size() * sizeof(T) + 1024;
     cudaError_t e = cudaMalloc(&d, bytes);
     if (e != cudaSuccess) return e;
-    p->allocs.push_back(d);
+    allocs.push_back(d);
     if ((e = cudaMemset(d, 0, bytes)) != cudaSuccess) return e;
     if (v.size()) e = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
     *out = (const T*)d;
@@ -128,21 +128,21 @@ int ppgpu_program_create(const ppgpu_dims* d, const double* A, const double* b, 
     D.n = R.n; D.t = R.t; D.m = R.m; D.q = R.q; D.ne = R.ne; D.is_qp = R.is_qp;
     D.mi = R.mi; D.np = R.np; D.W = R.W; D.R0 = R.R0; D.nfree = R.nfree; D.use_gram = R.use_gram;
     D.dc0 = R.nfree + 2;
-#define UP(field, vecname) if ((e = upload(p, R.vecname, &D.field)) != cudaSuccess) { ppgpu_program_destroy(p); return fail("upload " #field, e); }
+#define UP(field, vecname) if ((e = upload(p->allocs, R.vecname, &D.field)) != cudaSuccess) { ppgpu_program_destroy(p); return fail("upload " #field, e); }
     UP(At, At) UP(C1, C1) UP(T0, T0) UP(Gam, Gam) UP(G, G) UP(V, V) UP(th_lo, th_lo) UP(th_hi, th_hi) UP(A, A) UP(b, b) UP(F, F) UP(A_t, At_theta) UP(b_t, bt) UP(Q, Q) UP(c, c) UP(H, H)
     UP(Xp, Xp) UP(K, K) UP(Pm, Pm)
 #undef UP
     D.wk_ok = R.wk_ok; D.wk_nb = R.wk_nb; D.wk_ld = R.wk_ld; D.wk_D0 = nullptr; D.wk_bvar = nullptr; D.wk_nvar = nullptr;
     if (R.wk_ok) {
-        if ((e = upload(p, R.wk_D0, &D.wk_D0)) != cudaSuccess || (e = upload(p, R.wk_bvar, &D.wk_bvar)) != cudaSuccess ||
-            (e = upload(p, R.wk_nvar, &D.wk_nvar)) != cudaSuccess) { ppgpu_program_destroy(p); return fail("upload walk dictionary", e); }
+        if ((e = upload(p->allocs, R.wk_D0, &D.wk_D0)) != cudaSuccess || (e = upload(p->allocs, R.wk_bvar, &D.wk_bvar)) != cudaSuccess ||
+            (e = upload(p->allocs, R.wk_nvar, &D.wk_nvar)) != cudaSuccess) { ppgpu_program_destroy(p); return fail("upload walk dictionary", e); }
     }
     D.lp_ok = R.lp_ok; D.lp_ld = R.lp_ld; D.lp_D0 = nullptr; D.lp_bvar = nullptr; D.lp_nvar = nullptr; D.lp_obj = nullptr;
     D.X0t = nullptr; D.Q2 = nullptr;
     if (R.lp_ok) {
-        if ((e = upload(p, R.lp_D0, &D.lp_D0)) != cudaSuccess || (e = upload(p, R.lp_bvar, &D.lp_bvar)) != cudaSuccess ||
-            (e = upload(p, R.lp_nvar, &D.lp_nvar)) != cudaSuccess || (e = upload(p, R.lp_obj, &D.lp_obj)) != cudaSuccess ||
-            (e = upload(p, R.X0t, &D.X0t)) != cudaSuccess || (e = upload(p, R.Q2, &D.Q2)) != cudaSuccess) {
+        if ((e = upload(p->allocs, R.lp_D0, &D.lp_D0)) != cudaSuccess || (e = upload(p->allocs, R.lp_bvar, &D.lp_bvar)) != cudaSuccess ||
+            (e = upload(p->allocs, R.lp_nvar, &D.lp_nvar)) != cudaSuccess || (e = upload(p->allocs, R.lp_obj, &D.lp_obj)) != cudaSuccess ||
+            (e = upload(p->allocs, R.X0t, &D.X0t)) != cudaSuccess || (e = upload(p->allocs, R.Q2, &D.Q2)) != cudaSuccess) {
             ppgpu_program_destroy(p);
             return fail("upload LP start dictionary", e);
         }
@@ -644,18 +644,6 @@ struct ppgpu_tree {
     std::vector<void*> allocs;
 };
 
-template <class T>
-static cudaError_t tree_upload(ppgpu_tree* h, const std::vector<T>& v, const T** out) {
-    void* d = nullptr;
-    const size_t bytes = (v.size() ? v.size() : 1) * sizeof(T);
-    cudaError_t e = cudaMalloc(&d, bytes);
-    if (e != cudaSuccess) return e;
-    h->allocs.push_back(d);
-    if (v.size()) e = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
-    *out = (const T*)d;
-    return e;
-}
-
 extern "C" {
 
 int ppgpu_tree_create(const ppgpu_dims* d, const int32_t* binary_indices, int32_t nb, const double* A, const double* b,
@@ -691,7 +679,7 @@ int ppgpu_tree_create(const ppgpu_dims* d, const int32_t* binary_indices, int32_
     h->inherit = env && atoi(env) != 0;
     DevTree& D = h->dev;
     D.nv = R.nv; D.rows = R.rows; D.cols = R.cols; D.rb0 = R.rb0; D.tp = R.tp; D.ld = R.ld; D.ne = R.ne; D.nb = R.nb;
-#define UP(field, vecname) if ((e = tree_upload(h, R.vecname, &D.field)) != cudaSuccess) { ppgpu_tree_destroy(h); return fail("tree upload " #field, e); }
+#define UP(field, vecname) if ((e = upload(h->allocs, R.vecname, &D.field)) != cudaSuccess) { ppgpu_tree_destroy(h); return fail("tree upload " #field, e); }
     UP(D0, D0) UP(bvar, bvar) UP(nvar, nvar) UP(hs, hs) UP(z0, z0) UP(Q2, Q2) UP(Arows, Arows) UP(brows, brows) UP(bin, bin)
 #undef UP
     *out = h;

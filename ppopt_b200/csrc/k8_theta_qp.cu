@@ -287,19 +287,10 @@ cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long 
     const size_t warp_bytes = (size_t)k8_layout(P.mi, P.np, P.t, P.n, P.W).stride * sizeof(double);
     const size_t g_bytes = (((size_t)P.mi * P.mi + 1) & ~(size_t)1) * sizeof(double);
     const int stage_g = g_bytes + 4 * warp_bytes <= (size_t)lim;
-    const size_t avail = (size_t)lim - (stage_g ? g_bytes : 0);
-    int wpb = (int)(avail / warp_bytes);
-    if (wpb > K8_MAX_WARPS) wpb = K8_MAX_WARPS;
-    if (wpb < 1) return cudaErrorInvalidValue;
-    const size_t smem = (stage_g ? g_bytes : 0) + (size_t)wpb * warp_bytes;
-    if ((e = allow_max_smem(k8_theta_qp_kernel)) != cudaSuccess) return e;
-    int per_sm = 0;
-    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k8_theta_qp_kernel, wpb * 32, smem)) != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    long long grid = (n_points + wpb - 1) / wpb;
-    const long long cap = (long long)sm_count * per_sm;
-    if (grid > cap) grid = cap;
-    k8_theta_qp_kernel<<<(unsigned)grid, wpb * 32, smem, st>>>(P, theta, n_points, stage_g, status, x, dual, mask, iters);
+    WarpGrid g;
+    if ((e = warp_grid(k8_theta_qp_kernel, warp_bytes, stage_g ? g_bytes : 0, K8_MAX_WARPS, n_points, sm_count, &g)) != cudaSuccess)
+        return e;
+    k8_theta_qp_kernel<<<g.grid, g.warps * 32, g.smem, st>>>(P, theta, n_points, stage_g, status, x, dual, mask, iters);
     return cudaGetLastError();
 }
 

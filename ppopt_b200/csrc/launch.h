@@ -32,6 +32,40 @@ inline cudaError_t fit_smem(K kern, size_t dyn) {
     return fa.sharedSizeBytes + dyn > 48 * 1024 ? allow_max_smem(kern) : cudaSuccess;
 }
 
+// Launch shape of a kernel that runs one warp per item over n items with a grid-stride loop: as many warps per CTA as the
+// device's opt-in shared memory holds next to the kernel's static shared memory and `fixed_bytes` of dynamic shared memory
+// ahead of the warps' blocks (at most max_warps), the dynamic shared memory that takes, and a grid capped at the CTAs that
+// are resident at once.  Opts the kernel in (fit_smem) when the size needs it; cudaErrorInvalidValue when no warp fits.
+struct WarpGrid {
+    int warps;
+    size_t smem;
+    unsigned grid;
+};
+template <class K>
+inline cudaError_t warp_grid(K kern, size_t warp_bytes, size_t fixed_bytes, int max_warps, long long n, int sm_count,
+                             WarpGrid* out) {
+    int dev = 0, lim = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&lim, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e != cudaSuccess) return e;
+    cudaFuncAttributes fa;
+    if ((e = cudaFuncGetAttributes(&fa, kern)) != cudaSuccess) return e;
+    const size_t used = fa.sharedSizeBytes + fixed_bytes;
+    int wpb = used < (size_t)lim ? (int)(((size_t)lim - used) / warp_bytes) : 0;
+    if (wpb > max_warps) wpb = max_warps;
+    if (wpb < 1) return cudaErrorInvalidValue;
+    const size_t smem = fixed_bytes + (size_t)wpb * warp_bytes;
+    if ((e = fit_smem(kern, smem)) != cudaSuccess) return e;
+    int per_sm = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, wpb * 32, smem)) != cudaSuccess) return e;
+    if (per_sm < 1) per_sm = 1;
+    long long grid = (n + wpb - 1) / wpb;
+    const long long cap = (long long)sm_count * per_sm;
+    if (grid > cap) grid = cap;
+    *out = {wpb, smem, (unsigned)grid};
+    return cudaSuccess;
+}
+
 int k2_pad_columns(int ncols_with_rhs);
 
 cudaError_t launch_k1(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,
