@@ -48,7 +48,7 @@ typedef struct {
 } ppgpu_info;
 
 /* number of uint64 counters returned by ppgpu_counters */
-#define PPGPU_NUM_COUNTERS 26
+#define PPGPU_NUM_COUNTERS 27
 
 const char* ppgpu_last_error(void);
 int ppgpu_version(void);
@@ -70,6 +70,11 @@ int ppgpu_program_info(const ppgpu_program* prog, ppgpu_info* out);
 /*   PPGPU_OPT_K2W_REF  1: the vertex walk applies every pivot to its whole dictionary (the reference of the deferred
  *                      updates it uses by default where the dictionary's shape allows; results are identical); 0: default */
 #define PPGPU_OPT_K2W_REF 1
+/*   PPGPU_OPT_K2W_INFEAS  1 (default): a drive of the vertex walk that ends at the optimum of a candidate's last row proves
+ *                      the candidate infeasible when its bound clears the feasibility tolerance by PPG_WALK_INF_MARGIN, and
+ *                      the relaxation and the simplex skip it; 0: the walk only ever certifies feasibility (the reference
+ *                      the tests compare against; results are identical) */
+#define PPGPU_OPT_K2W_INFEAS 2
 int ppgpu_set_option(ppgpu_program* prog, int32_t option, int64_t value);
 
 /* Level-1 candidates = generate_children_sets(equality_indices, m, murder_list) (solver_utils.py:154-166) plus the mpLP

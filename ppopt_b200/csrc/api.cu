@@ -39,6 +39,7 @@ struct ppgpu_program {
     size_t k2w_order_cap = 0;
     long long k2w_min = 100000;   // smallest launch the vertex walk (K2w) is used for (ppgpu_set_option)
     bool k2w_ref = false;         // K2w with the reference dictionary updates (PPGPU_OPT_K2W_REF)
+    bool k2w_infeas = true;       // K2w proves infeasibility where a drive ends at its optimum (PPGPU_OPT_K2W_INFEAS)
     double prof_ms[PPGPU_NUM_FAMILIES] = {0};
     long long prof_launches[PPGPU_NUM_FAMILIES] = {0};
 };
@@ -176,6 +177,7 @@ int ppgpu_set_option(ppgpu_program* p, int32_t option, int64_t value) {
     switch (option) {
         case PPGPU_OPT_K2W_MIN: p->k2w_min = value; return 0;
         case PPGPU_OPT_K2W_REF: p->k2w_ref = value != 0; return 0;
+        case PPGPU_OPT_K2W_INFEAS: p->k2w_infeas = value != 0; return 0;
         default: return fail_msg("unknown option");
     }
 }
@@ -301,6 +303,7 @@ static int level_eval_chunk(ppgpu_program* p, const uint64_t* d_masks, int64_t n
     }
     static const int warm_on = getenv("PPGPU_WARM") ? atoi(getenv("PPGPU_WARM")) : 1;
     p->dev.warm_count = nullptr; p->dev.warm_resid = nullptr; p->dev.warm_idx = nullptr; p->dev.warm_cap = 0;
+    bool walked = false;   // the walk ran and may have marked candidates it proved infeasible with PPG_ST_PRE
     // (measured: leaving what inheritance does not cover at the last level to the relaxation instead of the walk is slower -
     // the 14 % of level 5 of the bench program that no parent covers cost K2a + K2 134 ms against the walk's 111)
     if ((stages & 2) && !(stages & 8) && k_act >= 1 && p->k2w_min >= 0 && n >= p->k2w_min) {
@@ -317,9 +320,10 @@ static int level_eval_chunk(ppgpu_program* p, const uint64_t* d_masks, int64_t n
             p->k2w_order_cap = want;
         }
         e = launch_k2w(p->dev, d_masks, n, k_act, d_status, next_queue(p, st), p->d_counters, p->sm_count, st, &handled, wio.out, p->d_k2w_order,
-                       p->k2w_ref);
+                       p->k2w_ref, p->k2w_infeas);
         if (e != cudaSuccess) return fail("K2w vertex walk", e);
         if (handled) p->launches += (n > 128ll * 8 * p->sm_count) ? 4 : 1;   // + the three kernels that order the work items
+        walked = handled;
     }
     if ((stages & 2) && !(stages & 8)) {
         // feasibility certificates first (cheap); the simplex only sees what is left, and starts from K2a's last iterate
@@ -345,9 +349,10 @@ static int level_eval_chunk(ppgpu_program* p, const uint64_t* d_masks, int64_t n
         e = launch_k2(p->dev, d_masks, n, d_status, next_queue(p, st), p->d_counters, p->sm_count, st);
         if (e != cudaSuccess) return fail("K2 feasibility", e);
         p->launches++;
-        if (p->dev.warm_count) {
+        if (p->dev.warm_count || walked) {
             // candidates the warm solve found infeasible keep their hand-over mark until here, so that the cold scan of
-            // the same launch does not solve them a second time
+            // the same launch does not solve them a second time; so do the candidates the walk proved infeasible, which
+            // neither K2a nor K2 looks at
             if ((e = launch_clear_bits(d_status, n, PPG_ST_PRE, st)) != cudaSuccess) return fail("status clean-up", e);
             p->launches++;
         }

@@ -62,7 +62,9 @@ enum Counter {
     CNT_INHERITED, CNT_INHERIT_LOOKUPS,               // 21, 22: certificates inherited from parent witnesses / parents looked up
     CNT_K2W_DROP_RESET, CNT_K2W_DROP_GIVEUP,          // 23, 24: K2w reloads (K2W_RESET / vertex out of the band) that discarded
                                                       //         deferred pivots (K2wDeferDict)
-    CNT_COUNT = 26
+    CNT_K2W_INFEASIBLE = 25,                          // 25: candidates the walk proved infeasible (drive of the last row ended at its optimum)
+    CNT_K2W_INF_BAND,                                 // 26: ... drives that ended so, but whose bound fell inside PPG_WALK_INF_MARGIN's band
+    CNT_COUNT = 27
 };
 
 __device__ __forceinline__ bool mask_test(const uint64_t* m, int i) { return (m[i >> 6] >> (i & 63)) & 1ull; }

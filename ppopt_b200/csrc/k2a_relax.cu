@@ -14,7 +14,8 @@
 // equality residuals included) and only then is PPG_ST_FEAS set - the same acceptance rule as the LP (s* >= -1e-7).
 // Candidates that do not converge within the step budget (all infeasible ones, and sets on which the projections
 // zig-zag) are left for K2 - the register-resident kernel hands K2 the exact residuals of its last iterate, so the
-// simplex starts from there (DevProgram::warm_*).  The relaxation never decides infeasibility.
+// simplex starts from there (DevProgram::warm_*).  The relaxation never decides infeasibility; candidates the vertex walk
+// has proved infeasible (PPG_ST_PRE without PPG_ST_FEAS, k2w_walk.cu) are skipped.
 // Two kernels: k2a_relax_reg_kernel (k' <= 8, R0 <= 128: the production path) and the generic k2a_relax_kernel.
 #include "common.cuh"
 #include "launch.h"
@@ -51,7 +52,7 @@ k2a_relax_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, 
         const long long idx = (long long)__shfl_sync(PPG_FULL, q, 0);
         if (idx >= n) break;
         const uint8_t st = status[idx];
-        if (!(st & PPG_ST_RANK) || (st & PPG_ST_FEAS)) continue;
+        if (!(st & PPG_ST_RANK) || (st & (PPG_ST_FEAS | PPG_ST_PRE))) continue;   // (PRE: the walk proved it infeasible)
         const uint64_t* mk = masks + idx * W;
         ++n_try;
         __syncwarp();
@@ -321,7 +322,7 @@ k2a_relax_reg_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long
             for (int w = 0; w < W; ++w) mk_s[warp][lane * 4 + w] = masks[(base + lane) * W + w];
         }
         __syncwarp();
-        unsigned todo = __ballot_sync(PPG_FULL, (st_l & PPG_ST_RANK) && !(st_l & PPG_ST_FEAS));
+        unsigned todo = __ballot_sync(PPG_FULL, (st_l & PPG_ST_RANK) && !(st_l & (PPG_ST_FEAS | PPG_ST_PRE)));
         while (todo) {
         const int bj = __ffs((int)todo) - 1;
         todo &= todo - 1;

@@ -144,9 +144,20 @@ k2p_relax_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, 
         const long long base = ctl.base;
         if (base >= n) break;
         const int cn = (int)((n - base) < (long long)chunk ? (n - base) : (long long)chunk);
+        // whether a candidate needs work; PPG_ST_PRE: the vertex walk proved it infeasible (k2w_walk.cu).  A chunk with
+        // nothing to do is left before its masks are read and its prefixes projected - after a walked level that is
+        // nearly every chunk.  (No candidate's result depends on the chunk around it: a prefix cut by a chunk boundary is
+        // simply projected twice, and chunk sizes already vary with n.)
+        int any_chunk = 0;
         for (int i = tid; i < cn; i += THREADS) {
-            // stage the candidate: mask words, its two highest rows (the suffix), whether it needs work
             const uint8_t sb = status[base + i];
+            const bool todo = (sb & PPG_ST_RANK) && !(sb & (PPG_ST_FEAS | PPG_ST_PRE));
+            cab[i] = (todo ? K2P_TODO : 0u) | ((unsigned)sb << 24);
+            any_chunk |= todo;
+        }
+        if (!__syncthreads_or(any_chunk)) continue;
+        for (int i = tid; i < cn; i += THREADS) {
+            // stage the candidate: mask words, its two highest rows (the suffix)
             int hi1 = 0, hi2 = 0;
             for (int w = 0; w < W; ++w) {
                 const uint64_t x = masks[(base + i) * W + w];
@@ -159,8 +170,7 @@ k2p_relax_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, 
                 }
             }
             const unsigned a = has_b ? (unsigned)hi2 : (unsigned)hi1, b = (unsigned)hi1;
-            const bool todo = (sb & PPG_ST_RANK) && !(sb & PPG_ST_FEAS);
-            cab[i] = a | (b << 8) | (todo ? K2P_TODO : 0u) | ((unsigned)sb << 24);
+            cab[i] |= a | (b << 8);
         }
         __syncthreads();
         int s0 = 0;

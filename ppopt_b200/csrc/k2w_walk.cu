@@ -22,8 +22,12 @@
 // A certificate is therefore an exact statement: "the rows of A are nonbasic at a vertex whose basic slacks are >= -1e-8"
 // (nonbasic slacks are zero by construction; beta carries the rounding of the pivots only: the dictionary is reloaded from
 // the host-built vertex (host_math.hpp::build_walk_dictionary) at every work item and after K2W_RESET pivots).
-// K2w never decides infeasibility and gives up freely (empty face, dependent row, iteration cap): whatever it leaves
-// open goes to the relaxation (K2a) and then to the simplex (K2) exactly as before.
+// The walk gives up freely (empty face, dependent row, iteration cap): whatever it leaves open goes to the relaxation (K2a)
+// and then to the simplex (K2) exactly as before.  One kind of give-up is a proof instead: a drive of the last row b of a
+// candidate that stops because no free column has a positive coefficient in row b ends at the optimum of min s_b over the
+// face of the candidate's other rows, and the final row s_b = beta_b - sum_j D_bj s_j bounds the LP that K2 would solve
+// (k2w_infeasible_verdict).  Where that bound clears K2's threshold by PPG_WALK_INF_MARGIN the candidate is marked
+// PPG_ST_PRE without PPG_ST_FEAS: proved infeasible, skipped by K2a and K2 (api.cu clears the mark after K2).
 #include "common.cuh"
 #include "launch.h"
 #include "lp_core.cuh"
@@ -87,6 +91,13 @@ __device__ __forceinline__ int k2w_nth(const uint64_t (&m)[4], int j) {
     return -1;
 }
 
+// sum over the warp (butterfly: every lane gets the same bits)
+__device__ __forceinline__ double k2w_warp_sum(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(PPG_FULL, v, o);
+    return v;
+}
+
 // 1 / x to full double precision without the IEEE division sequence (x is a pivot / ratio denominator: normal, non-zero)
 __device__ __forceinline__ double k2w_rcp(double x) {
     double r;
@@ -147,6 +158,19 @@ struct K2wSmemDict {
         }
         wbest = warp_max_nonneg(best);
         j = __reduce_min_sync(PPG_FULL, best == wbest ? bj : 0x7fffffff);
+    }
+    // sum of -D_wi,j over the free columns j (not in fm) of basic row wi, and whether one of them is positive (uniform)
+    __device__ __forceinline__ double free_neg_sum(const K2wCtx& c, int wi, uint64_t fm, int lane, bool& pos) const {
+        const int lds = LD_ > 0 ? LD_ : c.lds;
+        const double* Di = c.D + (size_t)wi * lds;
+        double s = 0.0; bool p = false;
+        for (int jj = lane; jj < c.nf; jj += 32) {
+            if ((fm >> jj) & 1ull) continue;
+            const double x = Di[1 + jj];
+            if (x > 0.0) p = true; else s -= x;
+        }
+        pos = __any_sync(PPG_FULL, p);
+        return k2w_warp_sum(s);
     }
     __device__ __forceinline__ void column(const K2wCtx& c, int j, int lane, double (&col)[RPL], double (&beta)[RPL]) {
 #pragma unroll
@@ -326,6 +350,19 @@ struct K2wDeferDict {
         wbest = warp_max_nonneg(best);
         j = __reduce_min_sync(PPG_FULL, best == wbest ? bj : 0x7fffffff);
     }
+    // policy A's free_neg_sum on the current row values target_scan left in trow (the caller has just scanned row wi)
+    __device__ __forceinline__ double free_neg_sum(const K2wCtx& c, int wi, uint64_t fm, int lane, bool& pos) const {
+        double s = 0.0; bool p = false;
+#pragma unroll
+        for (int h = 0; h < TH; ++h) {
+            const int jj = lane + 32 * h;
+            if (jj >= c.nf || 1 + jj >= LD || ((fm >> jj) & 1ull)) continue;
+            const double x = trow[h];
+            if (x > 0.0) p = true; else s -= x;
+        }
+        pos = __any_sync(PPG_FULL, p);
+        return k2w_warp_sum(s);
+    }
     // entering column of my rows (lanes over rows, broadcast loads of p_m[cj])
     __device__ __forceinline__ void cur_column(const K2wCtx& c, int cj, int lane, double (&col)[RPL]) const {
 #pragma unroll
@@ -495,6 +532,26 @@ struct K2wHybridDict {
             j = __reduce_min_sync(PPG_FULL, best == wbest ? bj : 0x7fffffff);
         }
     }
+    __device__ __forceinline__ double free_neg_sum(const K2wCtx& c, int wi, uint64_t fm, int lane, bool& pos) const {
+        double s = 0.0; bool p = false;
+        if (wi < 32) {
+            if (lane == wi) {
+#pragma unroll
+                for (int k = 1; k < LD; ++k) {
+                    if (k - 1 >= c.nf || ((fm >> (k - 1)) & 1ull)) continue;
+                    if (T0[k] > 0.0) p = true; else s -= T0[k];
+                }
+            }
+        } else {
+            const double* Di = c.D + (size_t)(wi - 32) * LD;
+            for (int jj = lane; jj < c.nf; jj += 32) {
+                if ((fm >> jj) & 1ull) continue;
+                if (Di[1 + jj] > 0.0) p = true; else s -= Di[1 + jj];
+            }
+        }
+        pos = __any_sync(PPG_FULL, p);
+        return k2w_warp_sum(s);
+    }
     __device__ __forceinline__ void column(const K2wCtx& c, int j, int lane, double (&col)[RPL], double (&beta)[RPL]) {
         col[0] = lane < c.nb ? reg_pick<LD>(T0, 1 + j) : 0.0;
         beta[0] = T0[0];
@@ -630,6 +687,22 @@ struct K2wRegDict {
         wbest = shfl_d(best, owner);
         j = __shfl_sync(PPG_FULL, bj, owner);
     }
+    __device__ __forceinline__ double free_neg_sum(const K2wCtx& c, int wi, uint64_t fm, int lane, bool& pos) const {
+        const int slot = wi >> 5, owner = wi & 31;
+        double s = 0.0; bool p = false;
+        static_for<RPL>([&](auto RR) {
+            constexpr int rr = decltype(RR)::value;
+            if (rr == slot && lane == owner) {
+#pragma unroll
+                for (int k = 1; k < DC; ++k) {
+                    if (k - 1 >= c.nf || ((fm >> (k - 1)) & 1ull)) continue;
+                    if (T[rr][k] > 0.0) p = true; else s -= T[rr][k];
+                }
+            }
+        });
+        pos = __any_sync(PPG_FULL, p);
+        return k2w_warp_sum(s);
+    }
     __device__ __forceinline__ void column(const K2wCtx& c, int j, int lane, double (&col)[RPL], double (&beta)[RPL]) {
         static_for<RPL>([&](auto RR) {
             constexpr int rr = decltype(RR)::value;
@@ -701,16 +774,26 @@ __device__ __forceinline__ uint64_t k2w_ge_mask(int a, int w) {
     return w < aw ? 0ull : (w == aw ? (~0ull << (a & 63)) : ~0ull);
 }
 
-// certify candidate (a, b) of the segment (the caller has cleared its todo bit)
-__device__ __forceinline__ void k2w_certify(const K2wCtx& c, uint8_t* __restrict__ status, long long seg_base, int a, int b) {
+// level index of candidate (a, b), a <= b, of the segment that starts at seg_base
+__device__ __forceinline__ long long k2w_index(const K2wCtx& c, long long seg_base, int a, int b) {
     int rank = 0;
     const int w = b >> 6;
     for (int w2 = 0; w2 < w; ++w2) rank += __popcll(c.orig[(size_t)a * c.W4 + w2] & k2w_ge_mask(a, w2));
     rank += __popcll(c.orig[(size_t)a * c.W4 + w] & k2w_ge_mask(a, w) & ((1ull << (b & 63)) - 1ull));
-    const long long idx = seg_base + c.rowstart[a] + rank;
-    // fire-and-forget OR on the aligned word that holds the byte (a load + store would stall the walker for an L2 round trip)
+    return seg_base + c.rowstart[a] + rank;
+}
+
+// fire-and-forget OR of status bits into the aligned word that holds the byte (a load + store would stall the walker for
+// an L2 round trip)
+__device__ __forceinline__ void k2w_status_or(uint8_t* __restrict__ status, long long idx, unsigned bits) {
     const uintptr_t addr = reinterpret_cast<uintptr_t>(status + idx);
-    atomicOr(reinterpret_cast<unsigned*>(addr & ~(uintptr_t)3), (unsigned)PPG_ST_FEAS << (8u * (unsigned)(addr & 3)));
+    atomicOr(reinterpret_cast<unsigned*>(addr & ~(uintptr_t)3), bits << (8u * (unsigned)(addr & 3)));
+}
+
+// certify candidate (a, b) of the segment (the caller has cleared its todo bit)
+__device__ __forceinline__ void k2w_certify(const K2wCtx& c, uint8_t* __restrict__ status, long long seg_base, int a, int b) {
+    const long long idx = k2w_index(c, seg_base, a, b);
+    k2w_status_or(status, idx, PPG_ST_FEAS);
     // the WITNESS: the rows active at the certifying vertex.  Every superset of the candidate inside this mask is certified
     // by the same vertex - the next level inherits it (k6_children.cu::inherit_kernel) instead of walking again
     if (c.witness)
@@ -721,11 +804,7 @@ __device__ __forceinline__ void k2w_certify(const K2wCtx& c, uint8_t* __restrict
 // Two different vertices per parent cover more children than one (CPU model, level 4 -> 5 of the 100x30x6 program: 76 % of
 // the children inherit from first witnesses alone, 88 % with a later vertex next to them)
 __device__ __forceinline__ void k2w_second_witness(const K2wCtx& c, uint8_t* __restrict__ status, long long seg_base, int a, int b, int turn) {
-    int rank = 0;
-    const int w = b >> 6;
-    for (int w2 = 0; w2 < w; ++w2) rank += __popcll(c.orig[(size_t)a * c.W4 + w2] & k2w_ge_mask(a, w2));
-    rank += __popcll(c.orig[(size_t)a * c.W4 + w] & k2w_ge_mask(a, w) & ((1ull << (b & 63)) - 1ull));
-    const long long idx = seg_base + c.rowstart[a] + rank;
+    const long long idx = k2w_index(c, seg_base, a, b);
     const int slot = 1 + (turn % (PPG_WITNESS_SLOTS - 1));
     for (int x = 0; x < c.Wm; ++x) c.witness[idx * (PPG_WITNESS_SLOTS * c.Wm) + slot * c.Wm + x] = c.nbm[x];
     // (a candidate the walk gave up on earlier is closed too; its feasible bit is left to the relaxation / the simplex, and
@@ -762,6 +841,18 @@ __device__ __forceinline__ void k2w_revisit_all(const K2wCtx& c, uint8_t* __rest
             }
         }
     }
+}
+
+// A drive of row b with the candidate's other rows F fixed has stopped because no free column (nonbasic, not in F) has a
+// coefficient > K2W_PIV_MIN in row b; bi = beta_b, neg = sum over the free columns of -D_bj, pos = one of them is > 0.
+// Row b reads s_b = beta_b - sum_j D_bj s_j with s_j = 0 for j in F.  K2 solves max s subject to every slack >= s and the
+// candidate's slacks = 0, and calls the candidate infeasible iff s* < -PPG_FEAS_TOL.  With every free D_bj <= 0 and every
+// free s_j >= s, s_b = 0 forces beta_b <= -s * neg: s* <= -beta_b / neg (no feasible s at all when neg = 0).
+// Returns 1: proved infeasible with PPG_WALK_INF_MARGIN to spare (tolerances.h); 2: that bound, but inside the band;
+// 0: no bound (a degenerate target, or a free coefficient in (0, K2W_PIV_MIN]).
+__device__ __forceinline__ int k2w_infeasible_verdict(double bi, double neg, bool pos) {
+    if (pos || !(bi > 1e-11)) return 0;
+    return bi - PPG_WALK_INF_REL * (1.0 + fabs(bi)) > PPG_WALK_INF_MARGIN * neg ? 1 : 2;
 }
 
 // Open candidates live in a SYMMETRIC bit matrix: bit y of row x is set while the candidate with last rows {x, y} is open
@@ -835,7 +926,7 @@ __global__ void __launch_bounds__(256, 1)
 k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, int k_act, uint8_t* __restrict__ status,
                 unsigned long long* __restrict__ queue, unsigned long long* __restrict__ counters, int chunk,
                 int walker_bytes, int lds, int W4, int group_items, int split_len, uint64_t* __restrict__ witness,
-                const int* __restrict__ order, long long items) {
+                const int* __restrict__ order, long long items, bool prove_infeasible) {
     extern __shared__ unsigned char k2w_smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int RPL = Dict::RPL;
@@ -858,7 +949,7 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
     }
     const int W = P.W, R0 = P.R0, nb = c.nb, nf = c.nf;
     const int p = k_act >= 2 ? k_act - 2 : 0;
-    unsigned long long n_piv = 0, n_give = 0, n_drop_reset = 0, n_drop_give = 0;
+    unsigned long long n_piv = 0, n_give = 0, n_drop_reset = 0, n_drop_give = 0, n_inf = 0, n_band = 0;
     int n_cert = 0;
     // prefix words / last two rows of candidate q
     auto split = [&](long long q, uint64_t (&pf)[4], int& a, int& b) {
@@ -1009,6 +1100,7 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
                 }
                 // -- drive row t into the nonbasic set while the columns in fm stay put
                 bool reached = false;
+                int verdict = 0;   // stage 2: k2w_infeasible_verdict of the row where the drive stopped
                 for (int it = 0; it < K2W_DRIVE_CAP; ++it) {
                     const int wi = c.where[t];
                     if (wi < 0) { reached = true; break; }
@@ -1017,7 +1109,16 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
                     double bi, wbest; int j;
                     dict.target_scan(c, wi, fm, lane, bi, wbest, j);
                     const bool degen = bi <= 1e-11;
-                    if (!(wbest > K2W_PIV_MIN)) break;   // s_t cannot decrease on this face (empty face / dependent row)
+                    if (!(wbest > K2W_PIV_MIN)) {
+                        // s_t cannot decrease on this face (empty face / dependent row); for the last row of a candidate
+                        // that may prove the candidate infeasible
+                        if (stage == 2 && prove_infeasible && !degen) {
+                            bool pos;
+                            const double neg = dict.free_neg_sum(c, wi, fm, lane, pos);
+                            verdict = k2w_infeasible_verdict(bi, neg, pos);
+                        }
+                        break;
+                    }
                     int l = wi;
                     if (!degen) {
                         // Harris ratio test over the basic rows (lanes over rows); the target row wins when it is eligible
@@ -1086,8 +1187,17 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
                 } else {
                     // certified by the marking or not: this candidate is not tried again
                     if (lane == 0) c.todo[(size_t)a * W4 + (t >> 6)] &= ~(1ull << (t & 63));
+                    if (!reached) {
+                        ++n_give;
+                        if (verdict == 1) {
+                            // proved infeasible: decided, without the feasible bit (PPG_ST_PRE keeps K2a and K2 off it)
+                            if (lane == 0) k2w_status_or(status, k2w_index(c, i, a, t), PPG_ST_PRE);
+                            ++n_inf;
+                        } else if (verdict == 2) {
+                            ++n_band;
+                        }
+                    }
                     __syncwarp();
-                    if (!reached) ++n_give;
                 }
             }
             i = s1;
@@ -1103,6 +1213,8 @@ k2w_walk_kernel(DevProgram P, const uint64_t* __restrict__ masks, long long n, i
         if (n_drop_reset) atomicAdd(&counters[CNT_K2W_DROP_RESET], n_drop_reset);
         if (n_drop_give) atomicAdd(&counters[CNT_K2W_DROP_GIVEUP], n_drop_give);
     }
+    if (lane == 0 && n_inf) atomicAdd(&counters[CNT_K2W_INFEASIBLE], n_inf);
+    if (lane == 0 && n_band) atomicAdd(&counters[CNT_K2W_INF_BAND], n_band);
 }
 
 // ---- longest-processing-time-first order of the work items: cost = open candidates (rank OK, not yet certified) in the item's
@@ -1167,7 +1279,7 @@ static cudaError_t k2w_order_items(const uint8_t* status, long long n, int chunk
 template <class Dict>
 static cudaError_t launch_k2w_t(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,
                                 unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st,
-                                bool* handled, uint64_t* witness, int* order_scratch) {
+                                bool* handled, uint64_t* witness, int* order_scratch, bool prove_infeasible) {
     const int nb = P.wk_nb, ld = P.wk_ld, lds = ld | 1, W4 = (P.R0 + 63) / 64;
     size_t wb = k2w_dict_smem_bytes<Dict>(nb, lds) + (size_t)Dict::PROWS * lds * 8 + (size_t)2 * P.R0 * W4 * 8 + (size_t)W4 * 8 +
                 (size_t)(nb + P.nfree + 2 * P.R0 + K2W_MAXFIX + 2) * 4;
@@ -1210,7 +1322,7 @@ static cudaError_t launch_k2w_t(const DevProgram& P, const uint64_t* masks, long
         if ((e = k2w_order_items(status, n, (int)chunk, items, order_scratch, st, &order)) != cudaSuccess) return e;
     }
     kern<<<(unsigned)grid, 32 * wpc, smem, st>>>(P, masks, n, k_act, status, queue, counters, (int)chunk, (int)wb, lds, W4,
-                                                 group_items, split_len, witness, order, items);
+                                                 group_items, split_len, witness, order, items, prove_infeasible);
     *handled = true;
     return cudaGetLastError();
 }
@@ -1218,13 +1330,13 @@ static cudaError_t launch_k2w_t(const DevProgram& P, const uint64_t* masks, long
 // *handled == false: the walk is off for this program / level (no vertex dictionary, prefix too long, dictionary too large)
 cudaError_t launch_k2w(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,
                        unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st, bool* handled,
-                       uint64_t* witness, int* order_scratch, bool reference) {
+                       uint64_t* witness, int* order_scratch, bool reference, bool prove_infeasible) {
     *handled = false;
     static const int on = getenv("PPGPU_K2W") ? atoi(getenv("PPGPU_K2W")) : 1;
     static const int regs_on = getenv("PPGPU_K2W_REG") ? atoi(getenv("PPGPU_K2W_REG")) : 0;
     if (!on || !P.wk_ok || k_act < 1 || k_act - 2 > K2W_MAXFIX || P.W > 4 || P.nfree > 64) return cudaSuccess;
     const int rpl = (P.wk_nb + 31) / 32;
-#define K2W_GO(D) return launch_k2w_t<D>(P, masks, n, k_act, status, queue, counters, sm_count, st, handled, witness, order_scratch)
+#define K2W_GO(D) return launch_k2w_t<D>(P, masks, n, k_act, status, queue, counters, sm_count, st, handled, witness, order_scratch, prove_infeasible)
     // The register-resident dictionary (instantiated for the 100 x 30 x 6 bench program: 76 basic rows x 37 columns) is
     // an EXPERIMENT, off by default (PPGPU_K2W_REG=1): 255 registers + 2 KB of spills, measured 2.6x slower per pivot than
     // the shared-memory dictionary (1395 vs 535 ms on levels 4-5); kept because it decides identically and is the

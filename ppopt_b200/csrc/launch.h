@@ -79,9 +79,11 @@ cudaError_t launch_k2a_prefix(const DevProgram& P, const uint64_t* masks, long l
                               cudaStream_t st, bool* handled);
 // K2w: feasibility certificates shared between the candidates of a prefix by a primal-simplex walk over vertices
 // witness (n x W, may be null): receives the active-row mask of the vertex that certified a candidate
+// prove_infeasible: candidates whose last drive ends at an optimum that proves them infeasible get PPG_ST_PRE (and no
+// PPG_ST_FEAS); the caller clears that mark after K2
 cudaError_t launch_k2w(const DevProgram& P, const uint64_t* masks, long long n, int k_act, uint8_t* status,
                        unsigned long long* queue, unsigned long long* counters, int sm_count, cudaStream_t st, bool* handled,
-                       uint64_t* witness, int* order_scratch, bool reference);
+                       uint64_t* witness, int* order_scratch, bool reference, bool prove_infeasible);
 // ints of scratch launch_k2w wants for ordering the work items of an n-candidate launch (may be passed as null: natural order)
 size_t k2w_order_scratch_ints(long long n);
 // certificates INHERITED from the previous level: a candidate is feasible when the witness vertex of one of its parents

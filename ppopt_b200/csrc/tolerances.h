@@ -28,6 +28,19 @@
 // candidate whose radius lies within this band of the threshold, so that the discrepancy is never silent.
 #define PPG_RADIUS_BAND 1e-7
 
+// Infeasibility certificate of the vertex walk (csrc/k2w_walk.cu).  A drive of row b that stops with every free
+// coefficient of its row <= 0 proves that the feasibility LP of its candidate (K2: max s with every slack >= s and the
+// candidate's slacks = 0) has s* <= -beta_b / sum_free |D_bj|.  The walk decides "infeasible" only when
+//     beta_b - PPG_WALK_INF_REL * (1 + |beta_b|) > PPG_WALK_INF_MARGIN * sum_free |D_bj|
+// i.e. when that bound clears K2's threshold (-PPG_FEAS_TOL) ten times over, after an allowance for the rounding of the
+// walk's beta.  Measured drift of the walk's dictionary before it is reloaded (DESIGN.md section 3): 9e-14 absolute on D,
+// 1e-13 relative on beta after 2,400 pivots.  The allowance is relative to |beta_b| because the programs carry box rows of
+// 1e7 next to rows near 1 (an absolute error of 1e-6 on such a row is still 1e-13 relative); 1e-9 keeps four orders of
+// magnitude over the measured drift.  The factor ten on PPG_FEAS_TOL covers K2's own rounding.  Bounds inside the band are
+// left to K2a and K2.
+#define PPG_WALK_INF_MARGIN (10 * PPG_FEAS_TOL)
+#define PPG_WALK_INF_REL 1e-9
+
 #define PPG_PIV_TOL 1e-9
 #define PPG_OPT_TOL 1e-12  // reduced-cost threshold: the objective error is tol x distance travelled (theta ranges of 1e2), so 1e-9 was too loose
 #define PPG_HARRIS 1e-9
@@ -48,7 +61,9 @@
 #define PPG_ST_BORDER 16u   // a decision fell inside a borderline band (reported, never silently ignored)
 #define PPG_ST_NUMERIC 32u  // iteration limit / singular KKT / non-finite value
 #define PPG_ST_THIN 64u     // full-dimension decision taken inside PPG_RADIUS_BAND of the 1e-8 threshold (reported)
-#define PPG_ST_PRE 128u       // transient: passed the K3 thread-per-candidate prefilter (cleared by k34_kernel)
+#define PPG_ST_PRE 128u       // transient: passed the K3 thread-per-candidate prefilter (cleared by k34_kernel); before
+                              // that, in the feasibility stage: handed over by K2a, or proved infeasible by the vertex walk
+                              // (cleared after K2)
 
 // witness slots per candidate (ppgpu_level_eval_w): [0] the vertex that certified it (walk or inheritance), [1..] later
 // vertices of the walk that hold it as well, written in turn.  Measured on the bench program (share of level 5 that inherits /
