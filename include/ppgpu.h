@@ -202,6 +202,52 @@ int ppgpu_solve_theta_batch(ppgpu_program* prog, const double* d_theta, int64_t 
 int ppgpu_solve_theta_lp_batch(ppgpu_program* prog, const double* d_theta, int64_t n_points, uint8_t* d_status, double* d_x,
                                double* d_dual, uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream);
 
+/* ---- Mixed-integer programs at fixed theta, by binary assignment y (MixedIntegerThetaSolver of ppopt_b200/mi_theta.py).
+ * The handle is the continuous program: the rows that contain a continuous variable, at y = 0.  y enters it the way theta
+ * does (right-hand side b + F theta + Fy y with Fy = -A_y; linear term c + H theta + Hy y with Hy the symmetrised Q_xy, zero
+ * for an mpMILP).
+ *
+ * The y columns of the maps the kernels read, reduced with reduce_program's theta-column formulas (host):
+ *   h_Fy  m x ny, h_Hy  n x ny or NULL (zero), row major
+ *   h_maps  rows x ny, rows = mi + 2 n (mpQP: [V_y | Xp_y | Hy]) or 2 mi + n (mpLP: [Dth_y | Ft_y | X0t_y]); NULL: only
+ *           *h_rows is set.
+ * Returns -2 when the handle is outside K8 / K9 (see ppgpu_solve_theta_batch / ppgpu_solve_theta_lp_batch). */
+int ppgpu_program_param_maps(ppgpu_program* prog, int32_t ny, const double* h_Fy, const double* h_Hy, double* h_maps,
+                             int32_t* h_rows);
+
+/* Per assignment a (bit k of d_assign[a] is y_k, nb <= 63): d_off[a][r] = d_base[r] + sum_k d_maps[r][k] y_k (d_base may be
+ * NULL), plus 1/2 y' Qyy y on row quad_row when d_qyy (nb x nb) is given.  d_off: n_assign x rows.  Stateless. */
+int ppgpu_mi_offsets(const double* d_maps, const double* d_base, int32_t rows, int32_t nb, const uint64_t* d_assign,
+                     int64_t n_assign, const double* d_qyy, int32_t quad_row, double* d_off, ppgpu_stream stream);
+
+/* K8 / K9 pair mode: one warp per (point, assignment) pair p = (d_pairs[2p], d_pairs[2p + 1]), the assignment's terms at
+ * d_off + d_pairs[2p + 1] * off_ld (the first rows of ppgpu_mi_offsets' output, in the order of ppgpu_program_param_maps).
+ * Outputs are per pair and have the meaning of ppgpu_solve_theta_batch / ppgpu_solve_theta_lp_batch's (x the continuous
+ * variables of the handle); every one but d_status may be NULL.  d_obj: the continuous part of the objective,
+ * 1/2 x'Qx + (c + H theta + Hy y)' x, computed in the warp (NaN unless optimal).  Pass 1 of a batch asks for status and
+ * objective only; pass 2 re-solves the winning pair of each point with the full outputs (the same pair gives the same
+ * result).  ppgpu_solve_pairs_qp needs an mpQP handle with use_gram, ppgpu_solve_pairs_lp an mpLP handle with a vertex
+ * (-2 otherwise). */
+int ppgpu_solve_pairs_qp(ppgpu_program* prog, const double* d_theta, const int32_t* d_pairs, int64_t n_pairs, const double* d_off,
+                         int64_t off_ld, uint8_t* d_status, double* d_obj, double* d_x, double* d_dual, uint64_t* d_active,
+                         int32_t* d_iters, ppgpu_stream stream);
+int ppgpu_solve_pairs_lp(ppgpu_program* prog, const double* d_theta, const int32_t* d_pairs, int64_t n_pairs, const double* d_off,
+                         int64_t off_ld, uint8_t* d_status, double* d_obj, double* d_x, double* d_dual, uint64_t* d_active,
+                         int32_t* d_iters, ppgpu_stream stream);
+
+/* The winner over one chunk of assignments a0 .. a0 + na - 1 (pass-1 outputs d_pair_status / d_pair_obj, n_points x na),
+ * folded into a running state per point (d_best = +inf, d_second = +inf, d_best_idx = -1, d_flags = 0 before the first
+ * chunk).  A pair counts when its binary-only rows hold at theta (rows of d_off[a] from seg: mb right-hand sides
+ * b_i - A_{i,y} y, then H_y' y (t), then the constant c_y'y + 1/2 y'Qyy y; d_Fb mb x t, d_beq mb equality flags) and it is
+ * optimal; its objective is d_pair_obj + the constant + theta' H_y' y.  Strict minimum in assignment order (exact ties: the
+ * lowest index), d_second the runner-up.  d_status (PPG_MI_* of csrc/tolerances.h) is the status after the chunks so far:
+ * unbounded if any counted pair is unbounded, else failed if any hit the iteration cap or broke down, else optimal if any is
+ * optimal, else infeasible.  Stateless. */
+int ppgpu_mi_select(const double* d_theta, int64_t n_points, int32_t t, const uint8_t* d_pair_status, const double* d_pair_obj,
+                    int64_t a0, int32_t na, const double* d_off, int64_t off_ld, int32_t seg, int32_t mb, const double* d_Fb,
+                    const uint8_t* d_beq, double* d_best, double* d_second, int32_t* d_best_idx, uint8_t* d_flags,
+                    uint8_t* d_status, ppgpu_stream stream);
+
 /* Batched Chebyshev balls of polytopes {theta : E theta <= f} (chebyshev_ball, utils/chebyshev_ball.py:10-63: max r subject to
  * E_i theta + |E_i| r <= f_i): CriticalRegion.is_full_dimension (critical_region.py:89-105, radius > 1e-8) and the Chebyshev /
  * feasibility checks of the program constructor's warnings() (mplp_program.py:162-215).  Stateless - no program handle.

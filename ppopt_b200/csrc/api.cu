@@ -621,6 +621,85 @@ int ppgpu_solve_theta_lp_batch(ppgpu_program* p, const double* d_theta, int64_t 
     return 0;
 }
 
+int ppgpu_program_param_maps(ppgpu_program* p, int32_t ny, const double* h_Fy, const double* h_Hy, double* h_maps,
+                             int32_t* h_rows) {
+    if (!p || !h_rows || (ny > 0 && !h_Fy)) return fail_msg("null argument");
+    if (ny < 1 || ny > 63) return fail_msg("1 <= ny <= 63 extra parameter columns are supported");
+    const ReducedProgram& R = p->host;
+    if (R.is_qp ? !R.use_gram : !R.lp_ok)
+        return fail_msg(R.is_qp ? "the continuous Hessian is not positive definite on the reduced space (use_gram = 0)"
+                                : "the reduced inequality rows have rank below n - n_eq, the LP has no vertex");
+    *h_rows = parameter_map_rows(R);
+    if (!h_maps) return 0;
+    vec maps;
+    std::string err;
+    if (!parameter_column_maps(R, ny, h_Fy, h_Hy, maps, err)) return fail_msg("parameter maps: " + err);
+    std::memcpy(h_maps, maps.data(), maps.size() * sizeof(double));
+    return 0;
+}
+
+int ppgpu_mi_offsets(const double* d_maps, const double* d_base, int32_t rows, int32_t nb, const uint64_t* d_assign,
+                     int64_t n_assign, const double* d_qyy, int32_t quad_row, double* d_off, ppgpu_stream stream) {
+    if (rows < 0 || nb < 0 || nb > 63 || n_assign < 0) return fail_msg("bad size (0 <= nb <= 63)");
+    if (rows == 0 || n_assign == 0) return 0;
+    if ((nb > 0 && !d_maps) || !d_assign || !d_off) return fail_msg("null argument");
+    if (d_qyy && (quad_row < 0 || quad_row >= rows)) return fail_msg("quad_row out of range");
+    cudaError_t e = launch_mi_offsets(d_maps, d_base, rows, nb, d_assign, n_assign, d_qyy, quad_row, d_off, (cudaStream_t)stream);
+    if (e != cudaSuccess) return fail("mixed-integer offsets", e);
+    return 0;
+}
+
+static int solve_pairs(ppgpu_program* p, bool qp, const double* d_theta, const int32_t* d_pairs, int64_t n_pairs,
+                       const double* d_off, int64_t off_ld, uint8_t* d_status, double* d_obj, double* d_x, double* d_dual,
+                       uint64_t* d_active, int32_t* d_iters, ppgpu_stream stream) {
+    if (!p) return fail_msg("null argument");
+    if (qp && (!p->dev.is_qp || !p->dev.use_gram))
+        return fail_msg("solve_pairs_qp needs an mpQP handle whose Hessian is positive definite on the reduced space");
+    if (!qp && (p->dev.is_qp || !p->dev.lp_ok))
+        return fail_msg("solve_pairs_lp needs an mpLP handle whose reduced inequality rows have a vertex");
+    if (n_pairs < 0) return fail_msg("negative size");
+    if (off_ld < parameter_map_rows(p->host)) return fail_msg("off_ld is below the rows of the parameter maps");
+    if (n_pairs == 0) return 0;
+    if (!d_theta || !d_pairs || !d_off || !d_status) return fail_msg("null argument");
+    cudaError_t e = cudaSetDevice(p->device);
+    const PairArgs pa{d_pairs, d_off, off_ld, d_obj};
+    if (e == cudaSuccess)
+        e = (qp ? launch_theta_qp_pairs : launch_theta_lp_pairs)(p->dev, d_theta, pa, n_pairs, d_status, d_x, d_dual, d_active,
+                                                                 d_iters, p->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return fail(qp ? "K8 pair mode" : "K9 pair mode", e);
+    p->launches++;
+    return 0;
+}
+
+int ppgpu_solve_pairs_qp(ppgpu_program* p, const double* d_theta, const int32_t* d_pairs, int64_t n_pairs, const double* d_off,
+                         int64_t off_ld, uint8_t* d_status, double* d_obj, double* d_x, double* d_dual, uint64_t* d_active,
+                         int32_t* d_iters, ppgpu_stream stream) {
+    return solve_pairs(p, true, d_theta, d_pairs, n_pairs, d_off, off_ld, d_status, d_obj, d_x, d_dual, d_active, d_iters, stream);
+}
+
+int ppgpu_solve_pairs_lp(ppgpu_program* p, const double* d_theta, const int32_t* d_pairs, int64_t n_pairs, const double* d_off,
+                         int64_t off_ld, uint8_t* d_status, double* d_obj, double* d_x, double* d_dual, uint64_t* d_active,
+                         int32_t* d_iters, ppgpu_stream stream) {
+    return solve_pairs(p, false, d_theta, d_pairs, n_pairs, d_off, off_ld, d_status, d_obj, d_x, d_dual, d_active, d_iters, stream);
+}
+
+int ppgpu_mi_select(const double* d_theta, int64_t n_points, int32_t t, const uint8_t* d_pair_status, const double* d_pair_obj,
+                    int64_t a0, int32_t na, const double* d_off, int64_t off_ld, int32_t seg, int32_t mb, const double* d_Fb,
+                    const uint8_t* d_beq, double* d_best, double* d_second, int32_t* d_best_idx, uint8_t* d_flags,
+                    uint8_t* d_status, ppgpu_stream stream) {
+    if (n_points < 0 || na < 0 || a0 < 0 || t < 1 || mb < 0 || seg < 0) return fail_msg("bad size");
+    if (off_ld < (int64_t)seg + mb + t + 1) return fail_msg("off_ld is below seg + mb + t + 1");
+    if (n_points == 0 || na == 0) return 0;
+    if (!d_theta || !d_pair_status || !d_pair_obj || !d_off || (mb > 0 && (!d_Fb || !d_beq)) || !d_best || !d_second ||
+        !d_best_idx || !d_flags || !d_status)
+        return fail_msg("null argument");
+    const MiSelectArgs a{d_theta, n_points, t, d_pair_status, d_pair_obj, a0, na, d_off, off_ld, seg, mb, d_Fb, d_beq,
+                         d_best, d_second, d_best_idx, d_flags, d_status};
+    cudaError_t e = launch_mi_select(a, (cudaStream_t)stream);
+    if (e != cudaSuccess) return fail("mixed-integer winner", e);
+    return 0;
+}
+
 int ppgpu_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_t n_polytopes, int32_t t, int32_t max_rows,
                           double* d_radius, int32_t* d_code, ppgpu_stream stream) {
     if (n_polytopes < 0) return fail_msg("negative size");

@@ -48,6 +48,17 @@ struct DevProgram {
     const double* Q2;      // n x np
 };
 
+// Pair mode of K8 / K9 (a mixed-integer program at fixed binary assignments): work item p is the point pairs[2p] at the
+// assignment pairs[2p + 1], whose additive terms are off + pairs[2p + 1] * off_ld (host_math.hpp::parameter_column_maps:
+// K8 [v_y (mi) | x_y (n) | h_y (n)], K9 [d_y (mi) | f_y (mi) | x_y (n)]).  obj (may be null) receives per pair the
+// continuous part of the objective, 1/2 x'Qx + (c + H theta + h_y)' x; every other output is indexed by the pair.
+struct PairArgs {
+    const int* pairs;
+    const double* off;
+    long long off_ld;
+    double* obj;
+};
+
 // indices into the device counter array (uint64 each)
 enum Counter {
     CNT_K1_CAND = 0,

@@ -8,6 +8,7 @@
 //     complement  S = A_act Q^-1 A_act'  so a candidate only gathers a k'xk' block of a precomputed Gram.
 // Pure C++ (no CUDA) so that the CPU checker in oracle/ can reuse exactly the same program reduction.
 #pragma once
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <string>
@@ -485,6 +486,60 @@ inline bool reduce_program(int n, int t, int m, int q, int ne, int is_qp, const 
         P.Pm = Pm;
         build_lp_dictionary(P);
     }
+    return true;
+}
+
+// Mixed-integer programs at a fixed binary assignment y (K8 / K9 pair mode).  y enters the continuous program exactly the way
+// theta does: right-hand side b + F theta + Fy y (Fy = -A_y), linear term c + H theta + Hy y (Hy = the symmetrised Q_xy, zero
+// for an mpMILP).  So the y columns reduce with the theta-column formulas of reduce_program: P's program is reduced once more
+// with the parameters (theta, y), and the y columns of the maps the kernels read are returned (row major, rows x ny):
+//   mpQP (use_gram):  [V_y (mi) | Xp_y (n) | Hy (n)]         w(0) += V_y y,  x += Xp_y y,  the mu term's linear part += Hy y
+//   mpLP (lp_ok):     [Dth_y (mi) | Ft_y (mi) | X0t_y (n)]   beta -= Dth_y y,  bti + Ft theta += Ft_y y,  x += X0t_y y
+// The reduction of the theta part (pivots, Cholesky factor, elimination) is the same arithmetic on the same data, so the maps
+// belong to P's dictionary; the pivot choice is checked all the same.  Returns false (err set) when P is outside K8 / K9.
+inline int parameter_map_rows(const ReducedProgram& P) { return P.is_qp ? P.mi + 2 * P.n : 2 * P.mi + P.n; }
+
+inline bool parameter_column_maps(const ReducedProgram& P, int ny, const double* Fy, const double* Hy, vec& maps,
+                                  std::string& err) {
+    const int n = P.n, t = P.t, m = P.m, q = P.q, t2 = t + ny, mi = P.mi;
+    if (ny < 1) { err = "no extra parameter columns"; return false; }
+    if (P.is_qp ? !P.use_gram : !P.lp_ok) { err = "the program is outside the fixed-theta solves (K8 / K9)"; return false; }
+    vec F2((size_t)m * t2, 0.0), H2((size_t)n * t2, 0.0), At2((size_t)q * t2, 0.0);
+    for (int i = 0; i < m; ++i)
+        for (int j = 0; j < t2; ++j) F2[(size_t)i * t2 + j] = j < t ? P.F[(size_t)i * t + j] : Fy[(size_t)i * ny + j - t];
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < t2; ++j) H2[(size_t)i * t2 + j] = j < t ? P.H[(size_t)i * t + j] : (Hy ? Hy[(size_t)i * ny + j - t] : 0.0);
+    for (int i = 0; i < q; ++i)
+        for (int j = 0; j < t; ++j) At2[(size_t)i * t2 + j] = P.At_theta[(size_t)i * t + j];
+    ReducedProgram R;
+    if (!reduce_program(n, t2, m, q, P.ne, P.is_qp, P.A.data(), P.b.data(), F2.data(), At2.data(), P.bt.data(),
+                        P.is_qp ? P.Q.data() : nullptr, P.c.data(), H2.data(), R)) {
+        err = R.error;
+        return false;
+    }
+    const int rows = parameter_map_rows(P);
+    maps.assign((size_t)rows * ny, 0.0);
+    auto col = [&](const vec& M, int ld, int i, int c0) { return &M[(size_t)i * ld + c0]; };
+    if (P.is_qp) {
+        if (!R.use_gram) { err = "the reduction with the binary columns lost the Gram data"; return false; }
+        for (int r = 0; r < mi; ++r) std::copy_n(col(R.V, t2 + 1, r, 1 + t), ny, &maps[(size_t)r * ny]);
+        for (int i = 0; i < n; ++i) {
+            std::copy_n(col(R.Xp, t2 + 1, i, 1 + t), ny, &maps[(size_t)(mi + i) * ny]);
+            for (int k = 0; k < ny; ++k) maps[(size_t)(mi + n + i) * ny + k] = Hy ? Hy[(size_t)i * ny + k] : 0.0;
+        }
+    } else {
+        if (!R.lp_ok || R.lp_bvar != P.lp_bvar || R.lp_nvar != P.lp_nvar) {
+            err = "the reduction with the binary columns pivoted differently";
+            return false;
+        }
+        const int dc = R.nfree + 2;
+        for (int r = 0; r < mi; ++r) {
+            std::copy_n(col(R.lp_D0, R.lp_ld, r, 1 + P.np + t), ny, &maps[(size_t)r * ny]);
+            for (int k = 0; k < ny; ++k) maps[(size_t)(mi + r) * ny + k] = -R.T0[(size_t)r * dc + 1 + P.np + t + k];   // T0 holds -Ft
+        }
+        for (int i = 0; i < n; ++i) std::copy_n(col(R.X0t, t2 + 1, i, 1 + t), ny, &maps[(size_t)(2 * mi + i) * ny]);
+    }
+    for (double v : maps) if (!std::isfinite(v)) { err = "non-finite parameter map"; return false; }
     return true;
 }
 

@@ -18,6 +18,11 @@
 // W, L (packed lower triangle), three vectors of np and the output staging.  Lanes split the update
 // w += s (G[:,j] + G[:,W] d) (mi x (|W| + 1) FMA per step, rows of G read contiguously: G is symmetric) and the columns of
 // the triangular solves; every decision is taken on values broadcast from lane 0, so the lanes never diverge.
+//
+// Pair mode (PairArgs, a mixed-integer program at fixed binary assignments; a separate instantiation): a warp solves the
+// point pairs[2p] at the assignment pairs[2p + 1], whose terms [v_y | x_y | h_y] enter as w(0) = V [1; theta] + v_y,
+// x = Xp [1; theta] + x_y - K lambda and the linear part c + H theta + h_y of the mu term; obj receives
+// 1/2 x'Qx + (c + H theta + h_y)' x per pair.
 #include <cmath>
 
 #include "common.cuh"
@@ -52,10 +57,12 @@ __host__ __device__ inline K8Layout k8_layout(int mi, int np, int t, int n, int 
     return o;
 }
 
+// PAIRS: the pair mode of PairArgs (a separate instantiation: the point mode's code is the one without it)
+template <bool PAIRS>
 __global__ void __launch_bounds__(K8_MAX_WARPS * 32)
 k8_theta_qp_kernel(DevProgram P, const double* __restrict__ theta, long long n_points, int stage_g, uint8_t* __restrict__ status_out,
                    double* __restrict__ x_out, double* __restrict__ dual_out, uint64_t* __restrict__ mask_out,
-                   int* __restrict__ iters_out) {
+                   int* __restrict__ iters_out, PairArgs pa) {
     extern __shared__ double k8_smem[];
     const int mi = P.mi, np = P.np, t = P.t, t1 = t + 1, n = P.n, ne = P.ne, Wd = P.W;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
@@ -86,13 +93,21 @@ k8_theta_qp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
 
     for (long long pt = (long long)blockIdx.x * wpb + warp; pt < n_points; pt += (long long)gridDim.x * wpb) {
         __syncwarp();
-        for (int k = lane; k < t; k += 32) th[k] = theta[pt * t + k];
+        const double* oy = nullptr;   // the pair's assignment terms [v_y | x_y | h_y]
+        if (PAIRS) {
+            const long long tp = pa.pairs[2 * pt];
+            oy = pa.off + (long long)pa.pairs[2 * pt + 1] * pa.off_ld;
+            for (int k = lane; k < t; k += 32) th[k] = theta[tp * t + k];
+        } else {
+            for (int k = lane; k < t; k += 32) th[k] = theta[pt * t + k];
+        }
         for (int k = lane; k < Wd; k += 32) wmask[k] = 0ull;
         __syncwarp();
         for (int r = lane; r < mi; r += 32) {
             const double* vr = P.V + (size_t)r * t1;
             double v = __ldg(vr);
             for (int k = 0; k < t; ++k) v = fma(__ldg(vr + 1 + k), th[k], v);
+            if (PAIRS) v += oy[r];
             w[r] = v;
             tolv[r] = PPG_QP_TOL * (1.0 + fabs(v));
         }
@@ -240,25 +255,45 @@ k8_theta_qp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
         if (lane == 0) status_out[pt] = (uint8_t)status;
         if (iters_out && lane == 0) iters_out[pt] = it;
         if (mask_out) for (int k = lane; k < Wd; k += 32) mask_out[pt * Wd + k] = wmask[k];
-        if (!x_out && !dual_out) continue;
+        const bool want_obj = PAIRS && pa.obj;
+        if (!x_out && !dual_out && !want_obj) continue;
         if (status != PPG_QP_OPTIMAL) {
             if (x_out) for (int i = lane; i < n; i += 32) x_out[pt * n + i] = QNAN;
             if (dual_out) for (int i = lane; i < P.m; i += 32) dual_out[pt * P.m + i] = QNAN;
+            if (want_obj && lane == 0) pa.obj[pt] = QNAN;
             continue;
         }
         for (int i = lane; i < n; i += 32) {
             const double* xr = P.Xp + (size_t)i * t1;
             double v = __ldg(xr);
             for (int k = 0; k < t; ++k) v = fma(__ldg(xr + 1 + k), th[k], v);
+            if (PAIRS) v += oy[mi + i];
             for (int k = 0; k < nW; ++k) v = fma(-__ldg(P.K + (size_t)i * mi + widx[k]), lam[k], v);
             xo[i] = v;
             if (x_out) x_out[pt * n + i] = v;
+        }
+        if (want_obj) {
+            // 1/2 x'Qx + (c + H theta + h_y)' x, lanes over the rows, a fixed butterfly: the same value for the same pair
+            __syncwarp();
+            double acc = 0.0;
+            for (int i = lane; i < n; i += 32) {
+                double g = 0.0;
+                for (int k = 0; k < n; ++k) g = fma(__ldg(P.Q + (size_t)i * n + k), xo[k], g);
+                double v = __ldg(P.c + i);
+                for (int k = 0; k < t; ++k) v = fma(__ldg(P.H + (size_t)i * t + k), th[k], v);
+                v += oy[mi + n + i];
+                acc = fma(fma(0.5, g, v), xo[i], acc);
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+            if (lane == 0) pa.obj[pt] = acc;
         }
         if (!dual_out) continue;
         __syncwarp();
         for (int i = lane; i < n; i += 32) {
             double v = __ldg(P.c + i);
             for (int k = 0; k < t; ++k) v = fma(__ldg(P.H + (size_t)i * t + k), th[k], v);
+            if (PAIRS) v += oy[mi + n + i];
             for (int k = 0; k < n; ++k) v = fma(__ldg(P.Q + (size_t)i * n + k), xo[k], v);
             for (int k = 0; k < nW; ++k) v = fma(__ldg(P.A + (size_t)(ne + widx[k]) * n + i), lam[k], v);
             ro[i] = v;
@@ -276,8 +311,9 @@ k8_theta_qp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
     }
 }
 
-cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
-                            double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
+template <bool PAIRS>
+static cudaError_t launch_k8(const DevProgram& P, const double* theta, const PairArgs& pa, long long n_points, uint8_t* status,
+                             double* x, double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
     if (n_points <= 0) return cudaSuccess;
     if (!P.use_gram || P.np < 1 || P.np > 64) return cudaErrorInvalidValue;
     int dev = 0, lim = 0;
@@ -288,10 +324,21 @@ cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long 
     const size_t g_bytes = (((size_t)P.mi * P.mi + 1) & ~(size_t)1) * sizeof(double);
     const int stage_g = g_bytes + 4 * warp_bytes <= (size_t)lim;
     WarpGrid g;
-    if ((e = warp_grid(k8_theta_qp_kernel, warp_bytes, stage_g ? g_bytes : 0, K8_MAX_WARPS, n_points, sm_count, &g)) != cudaSuccess)
+    if ((e = warp_grid(k8_theta_qp_kernel<PAIRS>, warp_bytes, stage_g ? g_bytes : 0, K8_MAX_WARPS, n_points, sm_count, &g)) != cudaSuccess)
         return e;
-    k8_theta_qp_kernel<<<g.grid, g.warps * 32, g.smem, st>>>(P, theta, n_points, stage_g, status, x, dual, mask, iters);
+    k8_theta_qp_kernel<PAIRS><<<g.grid, g.warps * 32, g.smem, st>>>(P, theta, n_points, stage_g, status, x, dual, mask, iters, pa);
     return cudaGetLastError();
+}
+
+cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
+                            double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
+    return launch_k8<false>(P, theta, PairArgs{nullptr, nullptr, 0, nullptr}, n_points, status, x, dual, mask, iters, sm_count, st);
+}
+
+cudaError_t launch_theta_qp_pairs(const DevProgram& P, const double* theta, const PairArgs& pa, long long n_pairs, uint8_t* status,
+                                  double* x, double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
+    if (!pa.pairs || !pa.off) return cudaErrorInvalidValue;
+    return launch_k8<true>(P, theta, pa, n_pairs, status, x, dual, mask, iters, sm_count, st);
 }
 
 }  // namespace ppgpu

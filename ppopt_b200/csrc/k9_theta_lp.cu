@@ -20,6 +20,11 @@
 //
 // One warp per point, the grid strides over points.  Per warp in shared memory: the dictionary of warp_dict.cuh (mi + 1
 // rows incl. the objective row), then theta, a row of n doubles for the refinement and the output staging, and the mask.
+//
+// Pair mode (PairArgs, an mpMILP at fixed binary assignments; a separate instantiation): the assignment's terms
+// [d_y | f_y | x_y] enter as beta = beta0 - Dth theta - d_y, the slack scale and refinement right-hand side
+// bti + Ft theta + f_y, and x = X0t [1; theta] + x_y + Q2 v; the objective row does not depend on y; obj receives
+// (c + H theta)' x per pair.
 #include <cmath>
 
 #include "common.cuh"
@@ -36,10 +41,12 @@ __host__ __device__ inline WarpDictLayout k9_layout(int mi, int np, int t, int n
     return warp_dict_layout(mi, mi + 1, np, t + n + W);
 }
 
+// PAIRS: the pair mode of PairArgs (a separate instantiation: the point mode's code is the one without it)
+template <bool PAIRS>
 __global__ void __launch_bounds__(K9_MAX_WARPS * 32)
 k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_points, uint8_t* __restrict__ status_out,
                    double* __restrict__ x_out, double* __restrict__ dual_out, uint64_t* __restrict__ mask_out,
-                   int* __restrict__ iters_out) {
+                   int* __restrict__ iters_out, PairArgs pa) {
     extern __shared__ double k9_smem[];
     const int mi = P.mi, np = P.np, t = P.t, t1 = t + 1, n = P.n, ne = P.ne, Wd = P.W, ld0 = P.lp_ld;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
@@ -59,7 +66,14 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
 
     for (long long pt = (long long)blockIdx.x * wpb + warp; pt < n_points; pt += (long long)gridDim.x * wpb) {
         __syncwarp();
-        for (int k = lane; k < t; k += 32) th[k] = theta[pt * t + k];
+        const double* oy = nullptr;   // the pair's assignment terms [d_y | f_y | x_y]
+        if (PAIRS) {
+            const long long tp = pa.pairs[2 * pt];
+            oy = pa.off + (long long)pa.pairs[2 * pt + 1] * pa.off_ld;
+            for (int k = lane; k < t; k += 32) th[k] = theta[tp * t + k];
+        } else {
+            for (int k = lane; k < t; k += 32) th[k] = theta[pt * t + k];
+        }
         for (int k = lane; k < Wd; k += 32) wmask[k] = 0ull;
         // constant entries: row by row, lanes over the columns (coalesced reads of the start dictionary)
         for (int r = 0; r < mi; ++r)
@@ -69,6 +83,7 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
             const double* src = P.lp_D0 + (size_t)r * ld0;
             double b = __ldg(src);
             for (int k = 0; k < t; ++k) b = fma(-__ldg(src + 1 + np + k), th[k], b);
+            if (PAIRS) b -= oy[r];
             const int bv = __ldg(P.lp_bvar + r);
             T[(size_t)r * LD] = b;
             T[(size_t)r * LD + 1 + np] = bv >= 0 ? -1.0 : 0.0;
@@ -77,6 +92,7 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
             const double* t0 = P.T0 + (size_t)r * P.dc0;
             double h = __ldg(t0);
             for (int k = 0; k < t; ++k) h = fma(-__ldg(t0 + 1 + np + k), th[k], h);
+            if (PAIRS) h += oy[mi + r];
             tolv[r] = PPG_TLP_TOL * (1.0 + fabs(h));
         }
         for (int c = lane; c < np; c += 32) {
@@ -152,10 +168,12 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
         if (lane == 0) status_out[pt] = (uint8_t)status;
         if (iters_out && lane == 0) { iters_out[2 * pt] = wd.it; iters_out[2 * pt + 1] = it1; }
         if (mask_out) for (int k = lane; k < Wd; k += 32) mask_out[pt * Wd + k] = wmask[k];
-        if (!x_out && !dual_out) continue;
+        const bool want_obj = PAIRS && pa.obj;
+        if (!x_out && !dual_out && !want_obj) continue;
         if (status != PPG_TLP_OPTIMAL) {
             if (x_out) for (int i = lane; i < n; i += 32) x_out[pt * n + i] = QNAN;
             if (dual_out) for (int i = lane; i < P.m; i += 32) dual_out[pt * P.m + i] = QNAN;
+            if (want_obj && lane == 0) pa.obj[pt] = QNAN;
             continue;
         }
         // v (staged in the pivot row) and x
@@ -169,6 +187,7 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
                 const double* t0 = P.T0 + (size_t)s * P.dc0;
                 double h = __ldg(t0);
                 for (int k = 0; k < t; ++k) h = fma(-__ldg(t0 + 1 + np + k), th[k], h);
+                if (PAIRS) h += oy[mi + s];
                 for (int j = 0; j < np; ++j) h = fma(-__ldg(t0 + 1 + j), Pr[j], h);
                 tolv[s] = h;   // residual slack of the nonbasic row s (tolv is free now)
             }
@@ -185,14 +204,27 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
             for (int j = lane; j < np; j += 32) Pr[j] += ro[j];
             __syncwarp();
         }
-        if (x_out)
+        if (x_out || want_obj) {
+            double acc = 0.0;   // (c + H theta)' x of the pair (an mpMILP's objective row does not depend on y)
             for (int i = lane; i < n; i += 32) {
                 const double* xr = P.X0t + (size_t)i * t1;
                 double v = __ldg(xr);
                 for (int k = 0; k < t; ++k) v = fma(__ldg(xr + 1 + k), th[k], v);
+                if (PAIRS) v += oy[2 * mi + i];
                 for (int c = 0; c < np; ++c) v = fma(__ldg(P.Q2 + (size_t)i * np + c), Pr[c], v);
-                x_out[pt * n + i] = v;
+                if (x_out) x_out[pt * n + i] = v;
+                if (want_obj) {
+                    double g = __ldg(P.c + i);
+                    for (int k = 0; k < t; ++k) g = fma(__ldg(P.H + (size_t)i * t + k), th[k], g);
+                    acc = fma(g, v, acc);
+                }
             }
+            if (want_obj) {
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+                if (lane == 0) pa.obj[pt] = acc;
+            }
+        }
         if (!dual_out) continue;
         __syncwarp();
         // lambda of the nonbasic slacks, scattered over the rows (tolv is free now)
@@ -259,16 +291,28 @@ k9_theta_lp_kernel(DevProgram P, const double* __restrict__ theta, long long n_p
     }
 }
 
-cudaError_t launch_theta_lp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
-                            double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
+template <bool PAIRS>
+static cudaError_t launch_k9(const DevProgram& P, const double* theta, const PairArgs& pa, long long n_points, uint8_t* status,
+                             double* x, double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
     if (n_points <= 0) return cudaSuccess;
     if (P.is_qp || !P.lp_ok || P.np > 64) return cudaErrorInvalidValue;
     const size_t warp_bytes = (size_t)k9_layout(P.mi, P.np, P.t, P.n, P.W).stride * sizeof(double);
     WarpGrid g;
-    const cudaError_t e = warp_grid(k9_theta_lp_kernel, warp_bytes, 0, K9_MAX_WARPS, n_points, sm_count, &g);
+    const cudaError_t e = warp_grid(k9_theta_lp_kernel<PAIRS>, warp_bytes, 0, K9_MAX_WARPS, n_points, sm_count, &g);
     if (e != cudaSuccess) return e;
-    k9_theta_lp_kernel<<<g.grid, g.warps * 32, g.smem, st>>>(P, theta, n_points, status, x, dual, mask, iters);
+    k9_theta_lp_kernel<PAIRS><<<g.grid, g.warps * 32, g.smem, st>>>(P, theta, n_points, status, x, dual, mask, iters, pa);
     return cudaGetLastError();
+}
+
+cudaError_t launch_theta_lp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
+                            double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
+    return launch_k9<false>(P, theta, PairArgs{nullptr, nullptr, 0, nullptr}, n_points, status, x, dual, mask, iters, sm_count, st);
+}
+
+cudaError_t launch_theta_lp_pairs(const DevProgram& P, const double* theta, const PairArgs& pa, long long n_pairs, uint8_t* status,
+                                  double* x, double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st) {
+    if (!pa.pairs || !pa.off) return cudaErrorInvalidValue;
+    return launch_k9<true>(P, theta, pa, n_pairs, status, x, dual, mask, iters, sm_count, st);
 }
 
 }  // namespace ppgpu

@@ -138,6 +138,24 @@ cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long 
 // iters (n x 2: pivots, Phase 1 pivots), x / dual / mask / iters may be null
 cudaError_t launch_theta_lp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
                             double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);
+// K8 / K9 pair mode (PairArgs of common.cuh): one warp per (point, assignment) pair, outputs per pair; all but status may be null
+cudaError_t launch_theta_qp_pairs(const DevProgram& P, const double* theta, const PairArgs& pa, long long n_pairs, uint8_t* status,
+                                  double* x, double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);
+cudaError_t launch_theta_lp_pairs(const DevProgram& P, const double* theta, const PairArgs& pa, long long n_pairs, uint8_t* status,
+                                  double* x, double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);
+// per assignment a (bit k of assign[a] = y_k): off[a][r] = base[r] + sum_k maps[r][k] y_k, plus 1/2 y'Qyy y on row quad_row
+cudaError_t launch_mi_offsets(const double* maps, const double* base, int rows, int nb, const uint64_t* assign, long long n_assign,
+                              const double* qyy, int quad_row, double* off, cudaStream_t st);
+// the running minimum over assignments a0 .. a0 + na - 1 per point (csrc/mi_theta.cu)
+struct MiSelectArgs {
+    const double* theta; long long n_points; int t;
+    const uint8_t* pair_status; const double* pair_obj;   // n_points x na
+    long long a0; int na;
+    const double* off; long long off_ld; int seg;         // off[a][seg ..]: binary-row rhs (mb), H_y' y (t), constant (1)
+    int mb; const double* Fb; const uint8_t* beq;          // binary-only rows: F (mb x t), equality flags
+    double* best; double* second; int* best_idx; uint8_t* flags; uint8_t* status;
+};
+cudaError_t launch_mi_select(const MiSelectArgs& a, cudaStream_t st);
 // K11: the relaxation tree of a mixed-integer program (csrc/k11_mitree.cu, lifted system of host_math.hpp::TreeProgram).
 // Nodes are uint64 with bit k = y_k for k < depth.
 struct DevTree {

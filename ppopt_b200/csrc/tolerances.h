@@ -135,3 +135,18 @@
 #define PPG_TREE_FEASIBLE 0
 #define PPG_TREE_INFEASIBLE 1
 #define PPG_TREE_UNDECIDED 255   // transient: the inheritance check did not certify the node, the LP decides it
+
+// ---- fixed-theta solves of a mixed-integer program by assignment (K8 / K9 pair mode, csrc/mi_theta.cu)
+//   PPG_MI_ROW_TOL   a binary-only row (no continuous variable) holds at (theta, y) when b_i + F_i theta - A_{i,y} y >=
+//                    -PPG_MI_ROW_TOL * (1 + |.|) (an equality row: |.| <= that), the tolerance of the relaxation tree
+#define PPG_MI_ROW_TOL 1e-7
+// status per point: the winner is optimal; no pair is feasible; some pair hit the iteration cap or broke down (the minimum
+// is not certified); some feasible pair is unbounded (mpMILP)
+#define PPG_MI_OPTIMAL 0
+#define PPG_MI_INFEASIBLE 1
+#define PPG_MI_FAILED 2
+#define PPG_MI_UNBOUNDED 4
+// running flags of mi_select
+#define PPG_MI_ANY_OPTIMAL 1
+#define PPG_MI_ANY_FAILED 2
+#define PPG_MI_ANY_UNBOUNDED 4

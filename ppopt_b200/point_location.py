@@ -11,7 +11,10 @@ critical_region.py:81-84).  Overlapping solutions (the flag `solve_mpqp` leaves 
 use the reference's rule as well: among the containing regions the one with the lowest objective, ties to the later
 region (solution.py:90-112, upop/point_location.py:68-84).  On a facet shared by two regions the two objectives agree to
 rounding, so which of the two is reported is noise in the reference too; the objective of the reported region is what
-is comparable.  No CPU fallback.
+is comparable.  Regions with fixed binaries (``y_fixation``, from solve_mpmiqp) are located the same way: their laws are
+stacked over the full variable vector (``x_indices`` rows from A / b, ``y_indices`` rows the constant assignment), and the
+overlap rule compares the full program's objective (Q, H, c), as Solution.get_region does; at most 128 variables.  No CPU
+fallback.
 """
 import ctypes
 from typing import Optional, Tuple
@@ -31,10 +34,18 @@ class PointLocation:
         regions = solution.critical_regions
         self.num_regions = len(regions)
         self.t = int(regions[0].E.shape[1]) if regions else int(solution.program.num_t())
-        self.n_x = int(regions[0].A.shape[0]) if regions else int(solution.program.num_x())
-        for r in regions:
-            if r.y_fixation is not None:
-                raise NotImplementedError('regions with fixed binaries are outside this engine')
+        # regions with fixed binaries (solve_mpmiqp): laws over the full variable vector, binary rows constant y
+        fixed = [getattr(r, 'y_fixation', None) is not None for r in regions]
+        if any(fixed) and not all(fixed):
+            raise ValueError('either every region or none fixes binaries')
+        self.mixed_integer = bool(fixed) and all(fixed)
+        if self.mixed_integer:
+            self.n_x = len(regions[0].x_indices) + len(regions[0].y_indices)
+            if self.n_x > 128:
+                raise NotImplementedError(f'point location of regions with fixed binaries supports at most 128 variables '
+                                          f'(continuous + binary), not {self.n_x}')
+        else:
+            self.n_x = int(regions[0].A.shape[0]) if regions else int(solution.program.num_x())
         off = numpy.zeros(self.num_regions + 1, dtype=numpy.int64)
         for i, r in enumerate(regions):
             off[i + 1] = off[i] + r.E.shape[0]
@@ -44,8 +55,14 @@ class PointLocation:
         for i, r in enumerate(regions):
             rows[off[i]:off[i + 1], 0] = numpy.asarray(r.f, dtype=float).ravel()
             rows[off[i]:off[i + 1], 1:] = numpy.asarray(r.E, dtype=float)
-            laws[i, :, 0] = numpy.asarray(r.b, dtype=float).ravel()
-            laws[i, :, 1:] = numpy.asarray(r.A, dtype=float)
+            if self.mixed_integer:
+                xi, yi = list(r.x_indices), list(r.y_indices)
+                laws[i, xi, 0] = numpy.asarray(r.b, dtype=float).ravel()
+                laws[i, xi, 1:] = numpy.asarray(r.A, dtype=float)
+                laws[i, yi, 0] = numpy.asarray(r.y_fixation, dtype=float).ravel()
+            else:
+                laws[i, :, 0] = numpy.asarray(r.b, dtype=float).ravel()
+                laws[i, :, 1:] = numpy.asarray(r.A, dtype=float)
         self.tdev = torch.device('cuda', device)
         self._rows = torch.from_numpy(rows).to(self.tdev)
         self._laws = torch.from_numpy(laws).to(self.tdev)

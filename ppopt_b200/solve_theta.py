@@ -258,7 +258,13 @@ def verify_solution(solution, thetas=None, num_samples: int = 100000, seed: int 
                                   (the optimal value is unique even where x is not)
         n_unbounded               points where the LP is unbounded
         n_dual_degenerate         points of max_dx where a multiplier of the basis is <= 1e-9 (1 + max |dual|): x need not be
-                                  unique there, so max_dx and n_dx_over_tol are taken over the other points only"""
+                                  unique there, so max_dx and n_dx_over_tol are taken over the other points only
+    A solution whose regions carry y_fixation (solve_mpmiqp) is checked against MixedIntegerThetaSolver instead
+    (mi_theta.verify_mixed_integer_solution: max_dobj, n_unbounded, n_ties and n_assignment_mismatch besides)."""
+    if getattr(solution.program, 'binary_indices', None) or \
+            any(getattr(r, 'y_fixation', None) is not None for r in solution.critical_regions):
+        from .mi_theta import verify_mixed_integer_solution
+        return verify_mixed_integer_solution(solution, thetas, num_samples, seed, tol, solver)
     from .point_location import PointLocation
     own = solver is None
     solver = solver_for(solution.program) if own else solver
