@@ -258,6 +258,21 @@ int ppgpu_mi_select(const double* d_theta, int64_t n_points, int32_t t, const ui
 int ppgpu_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_t n_polytopes, int32_t t, int32_t max_rows,
                           double* d_radius, int32_t* d_code, ppgpu_stream stream);
 
+/* K10: Chebyshev balls of facets.  For facet p = (d_facets[2p], d_facets[2p+1]) = (polytope, row i of that polytope):
+ *   max r  s.t.  a_j theta + |P a_j| r <= f_j  (every other row j of the polytope),  a_i theta = f_i,   P = I - n n', n = a_i / |a_i|
+ * solved as the Chebyshev LP of the facet in t - 1 coordinates of its hyperplane (one warp per facet).  A row parallel to the
+ * facet is dropped when it holds on the hyperplane and makes the facet empty when it does not.  Stateless.
+ *   d_rows, d_row_off, n_poly, t, max_rows   as ppgpu_chebyshev_batch ([f | E], rows need not be normalised), but
+ *             1 <= t <= 14 and max_rows <= 256 (a program handle's envelope)
+ *   d_center  n_facets x t    a centre of the largest ball inside the facet (NaN unless optimal; for t = 1 the facet's point
+ *                             f_i / a_i whenever it is not empty)
+ *   d_radius  n_facets        its radius (+inf unbounded, negative / -inf empty)
+ *   d_code    n_facets int32  PPG_LP_* of csrc/tolerances.h (0 optimal, 2 unbounded, 3 empty because of a parallel row,
+ *                             4 iteration limit), -1 when (polytope, row) is not in the batch.  t = 1: 2 or 3, no LP. */
+int ppgpu_facet_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_t n_poly, int32_t t, int32_t max_rows,
+                                const int64_t* d_facets, int64_t n_facets, double* d_center, double* d_radius,
+                                int32_t* d_code, ppgpu_stream stream);
+
 /* The relaxation tree of a mixed-integer program (mpMILP / mpMIQP): which assignments of the binaries have a feasible
  * relaxation.  Replaces the reference's MITree.__init__ / get_full_leafs (mitree.py) and, at the leaves, its
  * check_bin_feasibility (mpmilp_program.py); the reference runs a MILP per node with Gurobi, here an inner node answers

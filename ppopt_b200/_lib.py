@@ -62,6 +62,7 @@ SYMBOLS = {
     'ppgpu_solve_theta_batch': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'ppgpu_solve_theta_lp_batch': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'ppgpu_chebyshev_batch': (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp]),
+    'ppgpu_facet_chebyshev_batch': (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp]),
     'ppgpu_program_param_maps': (ctypes.c_int, [_vp, _i32, _vp, _vp, _vp, ctypes.POINTER(_i32)]),
     'ppgpu_mi_offsets': (ctypes.c_int, [_vp, _vp, _i32, _i32, _vp, _i64, _vp, _i32, _vp, _vp]),
     'ppgpu_solve_pairs_qp': (ctypes.c_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

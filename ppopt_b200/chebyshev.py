@@ -44,6 +44,31 @@ def chebyshev_radii(polytopes: Sequence[Tuple[numpy.ndarray, numpy.ndarray]], de
     return d_rad.cpu().numpy()
 
 
+def facet_balls(rows: torch.Tensor, row_off: torch.Tensor, facets: torch.Tensor, t: int):
+    """Chebyshev balls of facets (K10, ppgpu_facet_chebyshev_batch) on device tensors: rows (total x (t + 1), [f | E] of the
+    stacked polytopes), row_off (n_polytopes + 1, int64), facets (n_facets x 2 int64: polytope, row of that polytope).
+    Returns device tensors (centre n_facets x t, radius n_facets, code n_facets int32); the ball lies in the facet's hyperplane
+    E_i theta = f_i.  radius +inf unbounded, negative / -inf empty; centre NaN unless code is 0 (optimal), except for t = 1
+    where it is the facet's point whenever the facet is not empty."""
+    lib = _lib.load()
+    dev = rows.device
+    rows = rows.to(torch.float64).contiguous()
+    row_off = row_off.to(torch.int64).contiguous()
+    facets = facets.to(torch.int64).reshape(-1, 2).contiguous()
+    nf, n_poly = facets.shape[0], row_off.shape[0] - 1
+    center = torch.empty((nf, t), dtype=torch.float64, device=dev)
+    radius = torch.empty((nf,), dtype=torch.float64, device=dev)
+    code = torch.empty((nf,), dtype=torch.int32, device=dev)
+    if nf:
+        max_rows = max(1, int((row_off[1:] - row_off[:-1]).max().item())) if n_poly > 0 else 1
+        with torch.cuda.device(dev):
+            rc = lib.ppgpu_facet_chebyshev_batch(rows.data_ptr(), row_off.data_ptr(), n_poly, t, max_rows, facets.data_ptr(), nf,
+                                                 center.data_ptr(), radius.data_ptr(), code.data_ptr(),
+                                                 ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+        _lib.check(rc, 'facet_chebyshev_batch')
+    return center, radius, code
+
+
 def full_dimensional(regions: List) -> List[bool]:
     """CriticalRegion.is_full_dimension() for a list of regions in one launch"""
     rad = chebyshev_radii([(r.E, r.f) for r in regions])

@@ -716,6 +716,25 @@ int ppgpu_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_
     return 0;
 }
 
+int ppgpu_facet_chebyshev_batch(const double* d_rows, const int64_t* d_row_off, int64_t n_poly, int32_t t, int32_t max_rows,
+                                const int64_t* d_facets, int64_t n_facets, double* d_center, double* d_radius, int32_t* d_code,
+                                ppgpu_stream stream) {
+    if (n_poly < 0 || n_facets < 0) return fail_msg("negative size");
+    if (n_facets == 0) return 0;
+    if (!d_rows || !d_row_off || !d_facets || !d_center || !d_radius || !d_code) return fail_msg("null argument");
+    // the envelope of a program handle; four warps' tableaux then fit the 200 KB launch_facet_cheb allows (137 KB at the corner)
+    if (t < 1 || t > 14) return fail_msg("the facet Chebyshev batch supports 1 <= t <= 14 parameters");
+    if (max_rows < 1 || max_rows > 256) return fail_msg("the facet Chebyshev batch supports 1..256 rows per polytope");
+    int dev = 0, sms = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return fail("device query", e);
+    e = launch_facet_cheb(d_rows, (const long long*)d_row_off, n_poly, t, max_rows, (const long long*)d_facets, n_facets, d_center,
+                          d_radius, d_code, sms, (cudaStream_t)stream);
+    if (e != cudaSuccess) return fail("facet Chebyshev batch", e);
+    return 0;
+}
+
 }  // extern "C"
 
 // ---- K11: the relaxation tree of a mixed-integer program (a handle of its own: none of the path's limits apply)

@@ -451,4 +451,221 @@ cudaError_t launch_cheb_batch(const double* rows, const long long* row_off, long
     return cudaGetLastError();
 }
 
+// ---- K10: batched Chebyshev balls of FACETS {theta : E theta <= f, a_i theta = f_i} (the geometric mpQP algorithm steps across
+// every facet of a region from its centre).  theta = theta0 + N z with theta0 = f_i a_i / |a_i|^2 and N the t - 1 columns other
+// than k of the Householder reflector H = I - 2 v v' / v'v, v = n + sign(n_k) e_k, n = a_i / |a_i|, k = argmax |n_k|: H is
+// symmetric and orthogonal and maps n to -sign(n_k) e_k, so its other columns are an orthonormal basis of the hyperplane and
+// |N' a_j| = |P a_j|.  The facet LP is then the Chebyshev LP of {z : (N' a_j) z <= f_j - a_j theta0} in t - 1 variables.
+
+// row j of the polytope in the facet's coordinates: dst = [f_j - a_j theta0 | N' a_j | |N' a_j|]; returns |a_j|
+__device__ __forceinline__ double k10_row(const double* __restrict__ src, const double* __restrict__ v, double c2,
+                                          const double* __restrict__ th0, int t, int k, double* __restrict__ dst) {
+    double s = 0.0, at = 0.0, an = 0.0;
+#pragma unroll 1
+    for (int c = 0; c < t; ++c) { const double a = src[1 + c]; s = fma(v[c], a, s); at = fma(a, th0[c], at); an = fma(a, a, an); }
+    s *= c2;
+    double nn = 0.0;
+    int o = 1;
+#pragma unroll 1
+    for (int c = 0; c < t; ++c) {
+        if (c == k) continue;
+        const double h = fma(-s, v[c], src[1 + c]);
+        dst[o++] = h;
+        nn = fma(h, h, nn);
+    }
+    dst[0] = src[0] - at;
+    dst[t] = sqrt(nn);
+    return sqrt(an);
+}
+
+// the per-warp shared-memory layout of K10 (launch_facet_cheb sizes it).  The callees below rebuild it from the warp's base
+// pointer instead of taking ten pointers: the kernel then keeps one pointer live across its calls and needs no stack.
+struct K10Smem { double *Tab, *alpha, *prow, *v, *th0, *M; int *bvar, *kind, *nbv; unsigned char* flag; };
+__device__ __forceinline__ K10Smem k10_smem(unsigned char* base, int max_rows, int lds, int t) {
+    K10Smem S;
+    S.Tab = reinterpret_cast<double*>(base); base += (size_t)max_rows * lds * 8;
+    S.alpha = reinterpret_cast<double*>(base); base += (size_t)lds * 8;
+    S.prow = reinterpret_cast<double*>(base); base += (size_t)lds * 8;
+    S.v = reinterpret_cast<double*>(base); base += (size_t)t * 8;
+    S.th0 = reinterpret_cast<double*>(base); base += (size_t)t * 8;
+    S.M = reinterpret_cast<double*>(base); base += (size_t)t * (t + 1) * 8;   // final basis, then its solution
+    S.bvar = reinterpret_cast<int*>(base); base += (size_t)((max_rows + 1) & ~1) * 4;
+    S.kind = reinterpret_cast<int*>(base); base += (size_t)((lds + 1) & ~1) * 4;
+    S.nbv = reinterpret_cast<int*>(base); base += (size_t)((lds + 1) & ~1) * 4;
+    S.flag = base;
+    return S;
+}
+
+__device__ __noinline__ K4cOut k10_lp(unsigned char* base, int max_rows, int lds, int m, int t, int lane) {
+    const K10Smem S = k10_smem(base, max_rows, lds, t);
+    return k4c_solve(S.Tab, S.flag, S.bvar, S.alpha, S.kind, S.nbv, S.prow, m, t - 1, lds, CUDART_INF, lane);
+}
+
+// K10's output for one facet (lane 0): radius and code of the LP, and the centre - the vertex of the final basis.  Every
+// nonbasic variable is 0 there: a free one (z_c or r) by itself, a slack because its row is tight.  k4c_solve keeps no row
+// for a free basic variable, so the tight rows are rebuilt from the input and the nc x nc system [rhs | z r] is solved by
+// Gaussian elimination with partial pivoting.
+__device__ __noinline__ void k10_centre(const double* __restrict__ rows, long long r0, int t, int k, double c2, unsigned char* base,
+                                        int max_rows, int lds, K4cOut res, double* center, double* radius, int* code) {
+    const int t1 = t + 1, nc = t;
+    const K10Smem S = k10_smem(base, max_rows, lds, t);
+    const double* v = S.v;
+    const double* th0 = S.th0;
+    const int* nbv = S.nbv;
+    double* M = S.M;
+    double* th = S.prow;   // k4c_solve's scratch row, free again (lds >= t + 1)
+    bool ok = res.code == PPG_LP_OPTIMAL;
+    if (ok) {
+        const int ldm = nc + 1;
+        for (int c = 1; c <= nc; ++c) {
+            double* R = M + (size_t)(c - 1) * ldm;
+            const int var = nbv[c];
+            if (var <= nc) {
+                for (int q = 0; q <= nc; ++q) R[q] = 0.0;
+                R[var] = 1.0;
+            } else {
+                k10_row(rows + (size_t)(r0 + var - (nc + 1)) * t1, v, c2, th0, t, k, R);
+            }
+        }
+        for (int c = 1; c <= nc && ok; ++c) {
+            int piv = c - 1;
+            for (int r = c; r < nc; ++r) if (fabs(M[r * ldm + c]) > fabs(M[piv * ldm + c])) piv = r;
+            const double d = M[piv * ldm + c];
+            if (!(fabs(d) > 0.0)) { ok = false; break; }
+            if (piv != c - 1)
+                for (int q = 0; q <= nc; ++q) { const double x = M[(c - 1) * ldm + q]; M[(c - 1) * ldm + q] = M[piv * ldm + q]; M[piv * ldm + q] = x; }
+            for (int r = c; r < nc; ++r) {
+                const double f = M[r * ldm + c] / d;
+                for (int q = 0; q <= nc; ++q) M[r * ldm + q] = fma(-f, M[(c - 1) * ldm + q], M[r * ldm + q]);
+            }
+        }
+        if (ok) {
+            // back substitution: the solution of variable c - 1 replaces the right-hand side of row c - 1
+            for (int c = nc; c >= 1; --c) {
+                double s = M[(c - 1) * ldm];
+                for (int q = c + 1; q <= nc; ++q) s = fma(-M[(c - 1) * ldm + q], M[(q - 1) * ldm], s);
+                M[(c - 1) * ldm] = s / M[(c - 1) * ldm + c];
+            }
+            // theta = theta0 + H w, w = z placed on the coordinates other than k
+            double s = 0.0;
+            for (int c = 0, o = 0; c < t; ++c) { th[c] = (c == k) ? 0.0 : M[(o++) * ldm]; s = fma(v[c], th[c], s); }
+            s *= c2;
+            for (int c = 0; c < t; ++c) th[c] = th0[c] + fma(-s, v[c], th[c]);
+        }
+    }
+    for (int c = 0; c < t; ++c) center[c] = ok ? th[c] : CUDART_NAN;
+    *radius = res.beta;
+    *code = res.code;
+}
+
+__global__ void __launch_bounds__(128)
+facet_cheb_kernel(const double* __restrict__ rows, const long long* __restrict__ row_off, long long n_poly, int t,
+                  const long long* __restrict__ facets, long long n_facets, double* __restrict__ center,
+                  double* __restrict__ radius, int* __restrict__ code, int warp_bytes, int lds, int max_rows) {
+    extern __shared__ unsigned char facet_smem[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, t1 = t + 1;
+    unsigned char* const wbase = facet_smem + (size_t)warp * warp_bytes;
+    const K10Smem S = k10_smem(wbase, max_rows, lds, t);
+    double* Tab = S.Tab;
+    double* v = S.v;
+    double* th0 = S.th0;
+    unsigned char* flag = S.flag;
+    for (long long p = (long long)blockIdx.x * (blockDim.x >> 5) + warp; p < n_facets; p += (long long)gridDim.x * (blockDim.x >> 5)) {
+        const long long poly = facets[2 * p], fi = facets[2 * p + 1];
+        long long r0 = 0;
+        int m = 0;
+        if (poly >= 0 && poly < n_poly) { r0 = row_off[poly]; m = (int)(row_off[poly + 1] - r0); }
+        if (fi < 0 || fi >= m) {   // not a row of a polytope of the batch
+            if (lane < t) center[p * t + lane] = CUDART_NAN;
+            if (lane == 0) { radius[p] = CUDART_NAN; code[p] = -1; }
+            continue;
+        }
+        const double* src_i = rows + (size_t)(r0 + fi) * t1;
+        int k = 0;
+        double c2 = 0.0, ai2 = 0.0;
+        __syncwarp();
+        if (lane == 0) {
+            double big = -1.0;
+            for (int c = 0; c < t; ++c) { const double a = src_i[1 + c]; ai2 = fma(a, a, ai2); if (fabs(a) > big) { big = fabs(a); k = c; } }
+            if (ai2 > 0.0) {
+                const double inv = 1.0 / sqrt(ai2), q = src_i[0] / ai2;
+                double vv = 0.0;
+                for (int c = 0; c < t; ++c) {
+                    const double nc_ = src_i[1 + c] * inv;
+                    v[c] = nc_ + (c == k ? (nc_ >= 0.0 ? 1.0 : -1.0) : 0.0);
+                    vv = fma(v[c], v[c], vv);
+                    th0[c] = src_i[1 + c] * q;
+                }
+                c2 = 2.0 / vv;
+            }
+        }
+        k = __shfl_sync(PPG_FULL, k, 0);
+        c2 = shfl_d(c2, 0);
+        ai2 = shfl_d(ai2, 0);
+        __syncwarp();
+        K4cOut res; res.code = PPG_LP_INFEAS_EQ; res.beta = -CUDART_INF;
+        bool bad = !(ai2 > 0.0);   // a zero row has no facet
+        if (!bad && t == 1) {
+            // the facet is the point f_i / a_i: unbounded when every other row holds there, empty otherwise
+#pragma unroll 1
+            for (int j = lane; j < m; j += 32) {
+                const double* src = rows + (size_t)(r0 + j) * t1;
+                if (j != fi && src[0] - src[1] * th0[0] < -PPG_HARRIS * fmax(1.0, fabs(src[0]))) bad = true;
+            }
+            bad = __any_sync(PPG_FULL, bad);
+            if (!bad) { res.code = PPG_LP_UNBOUNDED; res.beta = CUDART_INF; }
+            if (lane == 0) center[p] = bad ? CUDART_NAN : th0[0];
+            if (lane == 0) { radius[p] = res.beta; code[p] = res.code; }
+            continue;
+        }
+        if (!bad) {
+#pragma unroll 1
+            for (int j = lane; j < m; j += 32) {
+                double* T = Tab + (size_t)j * lds;
+                const double* src = rows + (size_t)(r0 + j) * t1;
+                const double an = k10_row(src, v, c2, th0, t, k, T);
+                // a row parallel to the facet is constant on its hyperplane: dropped when it holds there, else the facet is
+                // empty.  "Parallel" up to 1e-9 |a_j|: below that the rounding of f_j - a_j theta0 (|f_j| 1e-16), divided by
+                // |N' a_j| when the row is scaled, would decide the radius (a facet of radius 3e-6 came out empty)
+                const bool live = j != fi && T[t] > PPG_HARRIS * an;
+                if (live) {
+                    // unit rows: k4c_solve's first pivot (r enters on the row of smallest right-hand side) leaves every
+                    // slack >= 0 only when every row's r coefficient is the same
+                    const double inv = 1.0 / T[t];
+#pragma unroll 1
+                    for (int c = 0; c < t; ++c) T[c] *= inv;
+                    T[t] = 1.0;
+                }
+                flag[j] = live ? 1 : 0;
+                if (!live && j != fi && T[0] < -PPG_HARRIS * fmax(1.0, fabs(src[0]))) bad = true;
+            }
+            __syncwarp();
+            bad = __any_sync(PPG_FULL, bad);
+            if (!bad) res = k10_lp(wbase, max_rows, lds, m, t, lane);
+        }
+        __syncwarp();
+        if (lane == 0) k10_centre(rows, r0, t, k, c2, wbase, max_rows, lds, res, center + p * t, radius + p, code + p);
+    }
+}
+
+cudaError_t launch_facet_cheb(const double* rows, const long long* row_off, long long n_poly, int t, int max_rows,
+                              const long long* facets, long long n_facets, double* center, double* radius, int* code,
+                              int sm_count, cudaStream_t st) {
+    constexpr int WPC = 4;
+    const int ld = t + 1, lds = ld | 1;   // t - 1 variables z, then r
+    size_t wb = (size_t)max_rows * lds * 8 + (size_t)2 * lds * 8 + (size_t)2 * t * 8 + (size_t)t * (t + 1) * 8 +
+                (size_t)(((max_rows + 1) & ~1) + 2 * ((lds + 1) & ~1)) * 4 + (size_t)max_rows;
+    wb = (wb + 15) & ~(size_t)15;
+    const size_t smem = wb * WPC;
+    if (smem > 200 * 1024) return cudaErrorInvalidValue;
+    cudaError_t e = allow_max_smem(facet_cheb_kernel);
+    if (e != cudaSuccess) return e;
+    long long grid = (n_facets + WPC - 1) / WPC;
+    if (grid > (long long)sm_count * 4) grid = (long long)sm_count * 4;
+    if (grid < 1) return cudaSuccess;
+    facet_cheb_kernel<<<(unsigned)grid, 32 * WPC, smem, st>>>(rows, row_off, n_poly, t, facets, n_facets, center, radius, code,
+                                                              (int)wb, lds, max_rows);
+    return cudaGetLastError();
+}
+
 }  // namespace ppgpu

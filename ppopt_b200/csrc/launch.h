@@ -131,6 +131,10 @@ cudaError_t launch_locate(const double* theta, long long n_points, int t, const 
 
 cudaError_t launch_cheb_batch(const double* rows, const long long* row_off, long long n_poly, int t, int max_rows,
                               double* radius, int* code, int sm_count, cudaStream_t st);
+// K10: Chebyshev balls of facets (polytope, row) of stacked polytopes (csrc/k34c_compact.cu)
+cudaError_t launch_facet_cheb(const double* rows, const long long* row_off, long long n_poly, int t, int max_rows,
+                              const long long* facets, long long n_facets, double* center, double* radius, int* code,
+                              int sm_count, cudaStream_t st);
 // K8: one fixed-theta QP per point (dual active set on the Gram data, csrc/k8_theta_qp.cu); x / dual / mask / iters may be null
 cudaError_t launch_theta_qp(const DevProgram& P, const double* theta, long long n_points, uint8_t* status, double* x,
                             double* dual, uint64_t* mask, int* iters, int sm_count, cudaStream_t st);

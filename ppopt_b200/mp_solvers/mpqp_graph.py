@@ -29,8 +29,10 @@ from .mpqp_combi_graph import _seed
 from .solver_utils import CombinationTester
 
 
-def _evaluate(eng, cr_cls, sets: List[Tuple[int, ...]], cache: Dict):
-    """cache[a] = (full_rank, feasible, optimal, region or None) for every active set in ``sets``"""
+def _evaluate(eng, cr_cls, sets: List[Tuple[int, ...]], cache: Dict, keep: Optional[list] = None):
+    """cache[a] = (full_rank, feasible, optimal, region or None) for every active set in ``sets``.  ``keep`` (list): receives,
+    per cardinality group that emitted regions, (active sets, regions or None, K5's device buffers laws / rows / flags / info)
+    in the order of the sets handed to K5"""
     n_eq = eng.n_eq
     by_k: Dict[int, List[Tuple[int, ...]]] = {}
     for a in sets:
@@ -45,13 +47,17 @@ def _evaluate(eng, cr_cls, sets: List[Tuple[int, ...]], cache: Dict):
         opt = eng.select(status, ST_OPT, ST_OPT)
         built = {}
         if opt.shape[0]:
-            laws, rows, flags, info = [x.cpu().numpy() for x in eng.emit(masks, opt, k_act, status)]
+            bufs = eng.emit(masks, opt, k_act, status)
+            laws, rows, flags, info = [x.cpu().numpy() for x in bufs]
             if numpy.any(info[:, 0] < 0):
                 raise numpy.linalg.LinAlgError('Singular matrix')
             asets = [list(group[i]) for i in opt.cpu().tolist()]
-            for a_, r in zip(asets, _engine.build_regions(eng, cr_cls, asets, k_act, laws, rows, flags, info)):
+            regs = _engine.build_regions(eng, cr_cls, asets, k_act, laws, rows, flags, info)
+            for a_, r in zip(asets, regs):
                 if r is not None:
                     built[tuple(a_)] = r
+            if keep is not None:
+                keep.append(([tuple(a_) for a_ in asets], regs, bufs))
         for a, s_ in zip(group, status.cpu().numpy()):
             rank_ok = bool(s_ & ST_RANK)
             feas = rank_ok and bool(s_ & ST_FEAS)

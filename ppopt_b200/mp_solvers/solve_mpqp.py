@@ -1,14 +1,14 @@
 """Dispatch with the reference's surface (/root/reference/src/ppopt/mp_solvers/solve_mpqp.py:23-114).
 
 The combinatorial algorithm is the scope (BASELINE.json north_star), the two connected-graph algorithms ride on the same
-kernels (SURVEY.md 8f row 2); the enum keeps the reference's member names so
+kernels (SURVEY.md 8f row 2), and the geometric algorithm steps across facets with K10 and K8 (mpqp_geometric); the enum keeps the reference's member names so
 that calling code type-checks, and every other member raises NotImplementedError instead of silently returning an
 empty solution."""
 from enum import Enum
 
 import numpy
 
-from . import mpqp_combi_graph, mpqp_combinatorial, mpqp_graph
+from . import mpqp_combi_graph, mpqp_combinatorial, mpqp_geometric, mpqp_graph
 
 
 class mpqp_algorithm(Enum):
@@ -49,8 +49,12 @@ def solve_mpqp(problem, algorithm: mpqp_algorithm = mpqp_algorithm.combinatorial
         solution = mpqp_graph.solve(problem)                # solve_mpqp.py:79-80
     elif algorithm is mpqp_algorithm.graph_exp:
         solution = mpqp_graph.solve(problem, use_pruning=False)   # solve_mpqp.py:82-83
+    elif algorithm in (mpqp_algorithm.geometric, mpqp_algorithm.geometric_parallel, mpqp_algorithm.geometric_parallel_exp):
+        # the reference's pool variants do the same work per facet; here every wave of facets is one GPU batch anyway
+        solution = mpqp_geometric.solve(problem)
     else:
-        raise NotImplementedError(f'{algorithm} is outside the scope of the B200 engine (combinatorial*, combinatorial_graph, graph, graph_exp)')
+        raise NotImplementedError(f'{algorithm} is outside the scope of the B200 engine (combinatorial*, combinatorial_graph, '
+                                  'graph, graph_exp, geometric*)')
     # overlap flags exactly as the reference sets them (solve_mpqp.py:105-112)
     if hasattr(problem, 'Q') and problem.Q is not None:
         if min(numpy.linalg.eigvalsh(problem.Q)) <= 0:
